@@ -44,6 +44,14 @@ its own trajectory (weak scaling).
 
 Multi-GPU: frames shard over ranks, no data-path collective; one NCCL all-reduce of the
 accumulators at the end, inside the timed region.
+
+``--dump-outputs DIR`` writes, after the timed steps, what the last timed step of each
+measured path returned to its caller as ``DIR/<name>.npy`` (float64, a few kB in all):
+``rdf_counts`` (headline), ``rdf_e2e_counts`` / ``rdf_e2e_rdf`` (``run()``), ``sq_sums``
+(secondary; the raw accumulator of the K identical timed steps over K),
+``sq_e2e_ssf`` / ``sq_e2e_wavenumbers`` and ``strong_<cfg>_{counts,rdf,ssf}``.  Every input
+is generated from a fixed seed, so two builds run with the same arguments can be compared
+output for output.
 """
 
 import argparse
@@ -93,7 +101,39 @@ def parse():
     ap.add_argument("--arith", default="auto", choices=["auto", "off"],
                     help="auto: fp32 filter + exact fp64 re-evaluation; off: fp64 for "
                          "every pair")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step of every "
+                         "measured path computed as DIR/<name>.npy (float64)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.warmup < 0:
+        ap.error("--warmup must not be negative")
+    return a
+
+
+# ---------------------------------------------------------------------------------
+# outputs of the timed paths (--dump-outputs)
+# ---------------------------------------------------------------------------------
+
+_OUTPUTS = {}
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def keep_output(name, array):
+    """Records what a timed path returned to its caller in its last step; rank 0 writes."""
+    _OUTPUTS[name] = np.array(array, dtype=np.float64)
+
+
+def dump_outputs(directory):
+    """Writes every recorded output as ``directory/<name>.npy``.  The inputs are seeded, so
+    two builds run with the same arguments can be compared output for output."""
+    total = sum(a.nbytes for a in _OUTPUTS.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed {DUMP_LIMIT_BYTES}")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in _OUTPUTS.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
 
 
 # ---------------------------------------------------------------------------------
@@ -321,6 +361,7 @@ def run_reference(args):
         _, _, c = cpu_rdf([(s * fps + i) % n_have for i in range(fps)], cores)
         binned += int(c.sum())
     dt = time.perf_counter() - t0
+    keep_output("rdf_counts", c)
     value = binned / dt
     sample = (f"each step = {fps} frames of the workload's 2,000 ({fps * args.steps} in "
               f"all), multiprocessing fork pool of {cores} processes over frames "
@@ -354,6 +395,8 @@ def run_reference(args):
                 "capped_distance is the C restatement in oracle/ feeding the real "
                 "numpy.histogram",
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs)
     emit(line)
 
 
@@ -442,6 +485,8 @@ def run_ours(args):
             line = dict({"metric": "strong_scaling_passes", "n_gpus": world}, **line)
         if bound is not None:
             line["affinity"] = bound
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs)
         emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -520,6 +565,11 @@ def bench_rdf(args, rank, world, local, cpu, dist, torch):
     ms = float(ms.item())
     launches = ctx.launch_count() - launches0
     binned_total = int(counts.sum().item())
+    # every timed step bins the same frames, so the integer counts of the timed region are
+    # exactly K times those of its last step
+    total = counts.cpu().numpy()
+    assert not (total % K).any(), "timed steps binned different counts"
+    keep_output("rdf_counts", total // K)
     evals_local = ctx.rdf_pair_evaluations()
     fstats = ctx.rdf_filter_stats()
     filtered = bool(fstats["eligible"]) and args.arith != "off" and args.hist in ("auto", "warp_atomic")
@@ -557,6 +607,8 @@ def bench_rdf(args, rank, world, local, cpu, dist, torch):
     if world > 1:
         dist.all_reduce(e2e_s, op=dist.ReduceOp.MAX)
     e2e_value = e2e_binned / float(e2e_s.item())
+    keep_output("rdf_e2e_counts", rdf.results.counts)
+    keep_output("rdf_e2e_rdf", rdf.results.rdf)
     if rank != 0:
         return None
 
@@ -710,6 +762,9 @@ def bench_sq(args, rank, world, local, cores, dist, torch):
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms = float(ms.item())
     launches = ctx.launch_count() - l0
+    # raw fp64 sums of the K identical timed steps: their mean is the last step's sums to
+    # rounding
+    keep_output("sq_sums", acc.cpu().numpy() / K)
     _, _, kern_total_ms, kern_calls = ctx.kernel_time(reset=True)
     kern_ms = kern_total_ms / max(kern_calls, 1)
     del dev
@@ -730,6 +785,8 @@ def bench_sq(args, rank, world, local, cores, dist, torch):
     e2e_s = torch.tensor([time.perf_counter() - t0], device="cuda")
     if world > 1:
         dist.all_reduce(e2e_s, op=dist.ReduceOp.MAX)
+    keep_output("sq_e2e_ssf", sf.results.ssf)
+    keep_output("sq_e2e_wavenumbers", sf.results.wavenumbers)
     if rank != 0:
         return None
 
@@ -884,8 +941,11 @@ def bench_strong(which, args, rank, world, local, dist, torch):
         counts = rdf.results.counts.copy()
         out["pairs_binned_per_s"] = float(counts.sum()) / mean
         out["counts_sum"] = int(counts.sum())
+        keep_output(f"strong_{which}_counts", counts)
+        keep_output(f"strong_{which}_rdf", rdf.results.rdf)
     if sf is not None:
         ssf = sf.results.ssf.copy()
+        keep_output(f"strong_{which}_ssf", ssf)
     # ---- multi-GPU parity: rank 0 alone over the whole frame list ----
     if world > 1:
         ok = torch.ones(1, device="cuda")

@@ -95,7 +95,6 @@ def test_sq_port_noncubic(golden):
     np.testing.assert_allclose(out["wavenumbers"], g["wavenumbers"], rtol=1e-13)
 
 
-@pytest.mark.skipif(not ref_harness.available(), reason="/root/reference not present")
 @pytest.mark.parametrize("mode", [None, "pair", "partial"])
 def test_isf_port_matches_golden(golden, mode):
     """oracle isf_run vs fixtures produced by the reference's real
@@ -121,6 +120,13 @@ def test_isf_port_matches_golden(golden, mode):
         np.testing.assert_allclose(o["times"], g["times_strided"])
         # F_s(q, 0) = 1 and F(q, 0) = S(q)
         np.testing.assert_allclose(o["iisf"][0], 1.0, rtol=1e-12)
+    if mode == "partial":
+        # user wavevectors off the lattice, in the order given
+        o = rp.isf_run(u, [cat, an], mode=mode, wavevectors=g["wavevectors_user"],
+                       n_lags=4, incoherent=True, sort=False, unique=False,
+                       dt=float(g["dt"]))
+        np.testing.assert_allclose(o["cisf"], g["cisf_user"], rtol=1e-9, atol=1e-10)
+        np.testing.assert_allclose(o["iisf"], g["iisf_user"], rtol=1e-9, atol=1e-10)
 
 
 def test_scsf_port_matches_golden(golden):
@@ -136,22 +142,6 @@ def test_scsf_port_matches_golden(golden):
     o = rp.scsf_run(u, u.atoms, start=1, stop=6, step=2, **kw)
     np.testing.assert_allclose(o["scsf"], g["scsf_strided"], rtol=1e-12)
     assert abs(o["scsf"][0] - 20.0) < 1e-12          # S_sc(0) = chain length
-
-
-def test_port_matches_live_reference():
-    """Where the reference tree exists, the port is checked against the real classes."""
-    from mdhelper_b200 import synthetic
-    S = ref_harness.load()
-    u, cat, an = synthetic.electrolyte(250, 2, seed=7)
-    L = float(u.dimensions[0])
-    r = S.RadialDistributionFunction(cat, an, n_bins=31, range=(0.2, L / 2),
-                                     exclusion=(2, 3), verbose=False).run()
-    p = rp.rdf_run(u, cat, an, n_bins=31, range=(0.2, L / 2), exclusion=(2, 3))
-    assert np.array_equal(p["counts"], r.results.counts)
-    np.testing.assert_allclose(p["rdf"], r.results.rdf, rtol=1e-12)
-    s = S.StructureFactor([cat, an], mode="partial", n_points=5, verbose=False).run()
-    p = rp.ssf_run(u, [cat, an], mode="partial", n_points=5)
-    np.testing.assert_allclose(p["ssf"], s.results.ssf, rtol=1e-10, atol=1e-12)
 
 
 @pytest.mark.parametrize("tag", ["equal", "unequal"])
