@@ -170,13 +170,28 @@ int mdh_rdf_accumulate(mdh_ctx *ctx, const float *pos1, int64_t frame_stride1,
  * lower-triangular cell matrix (a_x 0 0 / b_x b_y 0 / c_x c_y c_z) as float32 -- what
  * MDAnalysis' triclinic_vectors(ts.dimensions) gives; the reference passes ts.dimensions
  * with its angles to capped_distance (structure.py:93-96).  Coordinates are wrapped into
- * the cell, then every pair takes the shortest of its 27 images (fp64).  All-pairs only;
- * drop_axis is not available.  Restated from MDAnalysis' published algorithm and NOT
- * pinned against MDAnalysis (see DESIGN.md).
+ * the cell, then every pair takes the shortest of its 27 images (fp64).  The configured
+ * mode selects the pair kernel: MDH_RDF_ALLPAIRS evaluates all 27 images of every pair;
+ * MDH_RDF_CELLS uses a cell list in fractional coordinates and evaluates, per candidate,
+ * the one image that can be in range (same counts; MDH_EINVAL if some frame fits fewer
+ * than 3 cells on an axis, see mdh_rdf_triclinic_grid); MDH_RDF_AUTO takes the cell list
+ * when every frame fits at least 4 cells per axis and n1*n2 >= 4e6.  drop_axis is not
+ * available.  Restated from MDAnalysis' published algorithm and NOT pinned against
+ * MDAnalysis (see DESIGN.md).
  */
 int mdh_rdf_accumulate_triclinic(mdh_ctx *ctx, const float *pos1, int64_t frame_stride1,
                                  const float *pos2, int64_t frame_stride2, int location,
                                  const float *cell, int n_frames);
+
+/*
+ * Cell-list grid of one triclinic frame, as mdh_rdf_accumulate_triclinic would use it;
+ * device-free.  cell: the [9] matrix as above; r_hi: sqrt of the last squared threshold;
+ * n_max: the larger group size (about 2 particles per cell are kept).  Writes the cells
+ * per axis (a, b, c; all 0 when fewer than 3 fit on some axis) and the margin M: every
+ * cell's perpendicular width is at least r_hi + M (derivation: DESIGN.md 4.8).
+ */
+int mdh_rdf_triclinic_grid(const float *cell /* [9] */, double r_hi, int64_t n_max,
+                           int32_t *nc /* [3] */, double *margin);
 
 int mdh_rdf_fetch(mdh_ctx *ctx, int64_t *counts /* [n_bins] host */);
 int mdh_rdf_reset(mdh_ctx *ctx);

@@ -47,6 +47,7 @@ SIGNATURES = {
                                  _i64, _i32, _i32, _i32]),
     "mdh_rdf_accumulate": (_i32, [_p, _p, _i64, _p, _i64, _i32, _p, _i32]),
     "mdh_rdf_accumulate_triclinic": (_i32, [_p, _p, _i64, _p, _i64, _i32, _p, _i32]),
+    "mdh_rdf_triclinic_grid": (_i32, [_p, _f64, _i64, _p, ctypes.POINTER(_f64)]),
     "mdh_rdf_fetch": (_i32, [_p, _p]),
     "mdh_rdf_reset": (_i32, [_p]),
     "mdh_rdf_counts_device": (_i32, [_p, ctypes.POINTER(_p)]),
@@ -147,6 +148,19 @@ def stage_plan(n_frames: int, bytes_per_frame: float, copy_over_kernel: float = 
     check(lib().mdh_stage_plan(int(n_frames), float(bytes_per_frame), float(copy_over_kernel),
                                pieces, len(pieces), ctypes.byref(n)))
     return list(pieces[:n.value])
+
+
+def triclinic_grid(cell, r_hi: float, n_max: int):
+    """Cell-list grid of one triclinic frame (``mdh_rdf_triclinic_grid``; no device
+    needed): ``(cells per axis, margin M)`` for the lower-triangular ``cell`` (3x3, float32)
+    and cut-off ``r_hi``; the cells are ``(0, 0, 0)`` when fewer than 3 fit on some axis.
+    Every cell's perpendicular width is at least ``r_hi + M``."""
+    m = np.ascontiguousarray(cell, dtype=np.float32).reshape(9)
+    nc = np.zeros(3, dtype=np.int32)
+    margin = _f64(0.0)
+    check(lib().mdh_rdf_triclinic_grid(m.ctypes.data, float(r_hi), int(n_max), nc.ctypes.data,
+                                       ctypes.byref(margin)))
+    return tuple(int(v) for v in nc), margin.value
 
 
 class Context:

@@ -230,9 +230,13 @@ class RadialDistributionFunction(GpuAnalysisBase):
     * ``n_batches`` has no effect (the reference documents that its batched
       mode can be off by a few counts, ``structure.py:601-607``; the GPU result
       is the unbatched one).
-    * Triclinic cells run through a separate all-pairs kernel (coordinates wrapped into
-      the cell, shortest of the 27 images per pair); ``drop_axis`` needs an orthorhombic
-      cell.
+    * Triclinic cells run through separate kernels (coordinates wrapped into the cell,
+      shortest of the 27 images per pair): ``mode="allpairs"`` evaluates all 27 images of
+      every pair, ``mode="cells"`` a cell list in fractional coordinates that evaluates
+      the one image per candidate that can be in range (same counts; every perpendicular
+      width of the cell must hold 3 cells of ``range[1]`` plus a small margin), and
+      ``"auto"`` takes the cell list for cut-off runs on large systems.  ``drop_axis``
+      needs an orthorhombic cell.
     """
 
     def __init__(

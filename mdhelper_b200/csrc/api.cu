@@ -333,6 +333,12 @@ int mdh_rdf_accumulate_triclinic(mdh_ctx *c, const float *pos1, int64_t frame_st
                                          cell, n_frames);
 }
 
+int mdh_rdf_triclinic_grid(const float *cell, double r_hi, int64_t n_max, int32_t *nc,
+                           double *margin)
+{
+    return rdf_triclinic_grid_impl(cell, r_hi, n_max, nc, margin);
+}
+
 int mdh_rdf_fetch(mdh_ctx *c, int64_t *counts)
 {
     CTX_GUARD(c);

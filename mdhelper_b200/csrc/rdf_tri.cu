@@ -16,11 +16,15 @@
 //      and d^2 = (rx rx + ry ry) + rz rz.
 // Binning is the squared-threshold comparison of the orthorhombic kernels (rdf.cu).
 //
-// This is a correctness path (every pair evaluates 27 images in fp64); it exists so that
-// triclinic trajectories are analysed instead of rejected.
+// Two pair kernels give the same counts:
+//   rdf_triclinic_kernel   all pairs, every pair evaluates the 27 images (fp64);
+//   rdf_tri_cells_kernel   cut-off runs: a cell list in fractional coordinates, and for
+//                          every candidate only the ONE image that can be in range
+//                          (argument and margin: tri_grid_plan below, DESIGN.md 4.8).
 
 #include <algorithm>
 
+#include "rdf_cells.cuh"
 #include "rdf_device.cuh"
 
 using namespace rdfdev;
@@ -52,6 +56,20 @@ __global__ void tri_wrap_kernel(float4 *__restrict__ p, int64_t npad, int n,
     }
 }
 
+// d^2 of ONE image of dx = (double)(float)(r_j - r_i), in the reference's operation order;
+// s.. are the image's shift terms h_k * i (i in {-1, 0, 1}: exact products).  tri_d2 (all
+// 27 images) and the cell-list kernel (the one image that can be in range) both go
+// through it, so the two cannot drift apart.
+__device__ __forceinline__ double tri_image_d2(double dx0, double dx1, double dx2, double sax,
+                                               double sbx, double sby, double scx, double scy,
+                                               double scz)
+{
+    const double rx = __dadd_rn(__dadd_rn(__dadd_rn(dx0, sax), sbx), scx);
+    const double ry = __dadd_rn(__dadd_rn(dx1, sby), scy);
+    const double rz = __dadd_rn(dx2, scz);
+    return __dadd_rn(__dadd_rn(__dmul_rn(rx, rx), __dmul_rn(ry, ry)), __dmul_rn(rz, rz));
+}
+
 __device__ __forceinline__ double tri_d2(float xi, float yi, float zi, const float4 &pj,
                                          const TriBox &h)
 {
@@ -60,23 +78,15 @@ __device__ __forceinline__ double tri_d2(float xi, float yi, float zi, const flo
     const double dx2 = (double)__fsub_rn(pj.z, zi);
     double best = (double)FLT_MAX;
 #pragma unroll
-    for (int ix = -1; ix <= 1; ++ix) {
-        const double rx = __dadd_rn(dx0, h.ax * ix);            // products with -1, 0, 1: exact
+    for (int ix = -1; ix <= 1; ++ix)
 #pragma unroll
-        for (int iy = -1; iy <= 1; ++iy) {
-            const double ry0 = __dadd_rn(rx, h.bx * iy);
-            const double ry1 = __dadd_rn(dx1, h.by * iy);
+        for (int iy = -1; iy <= 1; ++iy)
 #pragma unroll
             for (int iz = -1; iz <= 1; ++iz) {
-                const double rz0 = __dadd_rn(ry0, h.cx * iz);
-                const double rz1 = __dadd_rn(ry1, h.cy * iz);
-                const double rz2 = __dadd_rn(dx2, h.cz * iz);
-                const double dsq = __dadd_rn(__dadd_rn(__dmul_rn(rz0, rz0), __dmul_rn(rz1, rz1)),
-                                             __dmul_rn(rz2, rz2));
+                const double dsq = tri_image_d2(dx0, dx1, dx2, h.ax * ix, h.bx * iy, h.by * iy,
+                                                h.cx * iz, h.cy * iz, h.cz * iz);
                 if (dsq < best) best = dsq;
             }
-        }
-    }
     return best;
 }
 
@@ -137,6 +147,496 @@ __global__ void __launch_bounds__(256) rdf_triclinic_kernel(const TriParams P)
     }
 }
 
+// ---- cell list in fractional coordinates ---------------------------------------------
+
+constexpr int kTriShiftMax = 60;   // |k| per axis: k_j - k_i + wrap stays inside a signed byte
+
+struct TriGrid {           // per frame
+    TriBox h;
+    int nc[3];
+    int ncell;
+};
+
+// Fractional coordinates of a wrapped particle, s = r H^-1 (H lower triangular; the
+// operation order is the one tri_grid_plan bounds), its cell in [0, n_k) per axis
+// (clamped) and its lattice shift k = -floor(s): p = r + k H lies in the cell.  k is
+// returned as packed signed bytes (axis a in byte 0).  A NaN coordinate lands in some
+// cell; its pairs are NaN and binned nowhere.
+__device__ __forceinline__ int tri_cell(const float4 &p, const TriGrid &g, unsigned &kcode)
+{
+    const TriBox &h = g.h;
+    const double sc = __ddiv_rn((double)p.z, h.cz);
+    const double sb = __ddiv_rn(__dsub_rn((double)p.y, __dmul_rn(sc, h.cy)), h.by);
+    const double sa = __ddiv_rn(
+        __dsub_rn(__dsub_rn((double)p.x, __dmul_rn(sb, h.bx)), __dmul_rn(sc, h.cx)), h.ax);
+    const double s[3] = {sa, sb, sc};
+    int c[3];
+    kcode = 0u;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const double f = floor(s[k]);
+        c[k] = min(max((int)__dmul_rn(__dsub_rn(s[k], f), (double)g.nc[k]), 0), g.nc[k] - 1);
+        const int kk = (int)fmin(fmax(-f, (double)-kTriShiftMax), (double)kTriShiftMax);
+        kcode |= ((unsigned)kk & 0xffu) << (8 * k);
+    }
+    return (c[2] * g.nc[1] + c[1]) * g.nc[0] + c[0];
+}
+
+// Coordinates outside the wrapped cell's brick widened by half its edges on either side:
+// there the margin of tri_grid_plan does not bound the float32 rounding of dx (only
+// finite coordinates a long way out of the cell, which tri_wrap_kernel cannot move in
+// exactly, get here).  NaN is not "far".
+__device__ __forceinline__ bool tri_far(const float4 &p, const TriBox &h)
+{
+    const double x = p.x, y = p.y, z = p.z;
+    return x < -0.5 * h.ax || x > 1.5 * h.ax || y < -0.5 * h.by || y > 1.5 * h.by ||
+           z < -0.5 * h.cz || z > 1.5 * h.cz;
+}
+
+// pass 1: cell and rank in the cell of every particle of the packed, wrapped array;
+// far[frame] = 1 if the frame has a far coordinate
+__global__ void __launch_bounds__(256)
+    tri_bin_kernel(const float4 *__restrict__ pk, int64_t npad, int n,
+                   const TriGrid *__restrict__ grids, int *__restrict__ cnt, int cstride,
+                   int2 *__restrict__ keyrank, int *__restrict__ far)
+{
+    const int frame = blockIdx.y, tid = threadIdx.x;
+    const TriGrid g = grids[frame];
+    const float4 *src = pk + (int64_t)frame * npad;
+    bool is_far = false;
+    for (int64_t i0 = (int64_t)blockIdx.x * 256; i0 < n; i0 += (int64_t)gridDim.x * 256) {
+        const int64_t i = i0 + tid;
+        const unsigned active = __ballot_sync(0xffffffffu, i < n);
+        if (i < n) {
+            const float4 p = src[i];
+            unsigned kc;
+            const int cell = tri_cell(p, g, kc);
+            is_far = is_far || tri_far(p, g.h);
+            // warp-aggregated counter update, as cells_bin_kernel (rdf_cells.cu)
+            const unsigned peers = __match_any_sync(active, cell);
+            const int leader = __ffs(peers) - 1, lane = tid & 31;
+            int base = 0;
+            if (lane == leader)
+                base = atomicAdd(&cnt[(int64_t)frame * cstride + cell], __popc(peers));
+            base = __shfl_sync(peers, base, leader);
+            keyrank[(int64_t)frame * n + i] =
+                make_int2(cell, base + __popc(peers & ((1u << lane) - 1u)));
+        }
+    }
+    if (__syncthreads_or(is_far) && tid == 0) far[frame] = 1;
+}
+
+// pass 3: packed -> cell-sorted float4 (x, y, z, exclusion block id) and shift codes
+__global__ void __launch_bounds__(256)
+    tri_scatter_kernel(const float4 *__restrict__ pk, int64_t npad, int n,
+                       const TriGrid *__restrict__ grids, const int *__restrict__ start,
+                       int cstride, const int2 *__restrict__ keyrank,
+                       float4 *__restrict__ sorted, int *__restrict__ kcode)
+{
+    const int frame = blockIdx.y;
+    const TriGrid g = grids[frame];
+    const float4 *src = pk + (int64_t)frame * npad;
+    const int *st = start + (int64_t)frame * cstride;
+    for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n;
+         i += (int64_t)gridDim.x * 256) {
+        const float4 p = src[i];
+        unsigned kc;
+        tri_cell(p, g, kc);
+        const int2 kr = keyrank[(int64_t)frame * n + i];
+        const int64_t o = (int64_t)frame * n + st[kr.x] + kr.y;
+        sorted[o] = p;
+        kcode[o] = (int)kc;
+    }
+}
+
+struct TriCellParams {
+    const float4 *s1, *s2;        // cell-sorted particles, [G][n1], [G][n2]
+    const int *k2;                // shift codes of s2 (tri_cell), [G][n2]
+    int n1, n2;
+    const int *start2;            // [G][cstride]
+    int cstride;
+    const TriGrid *grids;
+    const int *far;               // [G]
+    const double *thr;
+    int n_bins;
+    BinGuess guess;
+    unsigned long long *counts;
+    unsigned long long *evals;
+    int half;                     // same group: half stencil, weight 2
+};
+
+__host__ inline size_t tri_cells_smem_bytes(int n_bins)
+{
+    return align16(sizeof(double) * (n_bins + 1)) +
+           sizeof(unsigned) * kWarps * warp_hist_words(n_bins);
+}
+
+// One thread per particle i of the cell-sorted group 1, candidates from the 27 (same
+// group: 13 forward + own) cells around i's cell.  A candidate j of the run that starts
+// at neighbour cell index c_i + d (wrapped: c_i + d = c_j + w n, w in {-1, 0, 1}) is at
+// the image m' = k_j - k_i + w of the reference's dx; if m' is not one of the reference's
+// 27 images, the pair is out of range for both (tri_grid_plan).  The per-byte arithmetic
+// of the packed shift codes gives m' with one VADD4.
+template <bool EXCL, bool FAST>
+__global__ void __launch_bounds__(kThreads, 2) rdf_tri_cells_kernel(const TriCellParams P)
+{
+    extern __shared__ __align__(16) unsigned char smem[];
+    double *sT = reinterpret_cast<double *>(smem);
+    unsigned *sH =
+        reinterpret_cast<unsigned *>(smem + align16(sizeof(double) * (P.n_bins + 1)));
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int frame = blockIdx.y;
+    const int n_bins = P.n_bins;
+    for (int k = tid; k <= n_bins; k += kThreads) sT[k] = P.thr[k];
+    for (int k = tid; k < kWarps * warp_hist_words(n_bins); k += kThreads) sH[k] = 0;
+    __syncthreads();
+
+    unsigned *myhist = sH + warp * warp_hist_words(n_bins) + 1;
+    const unsigned hist32 = (unsigned)__cvta_generic_to_shared(myhist);
+    const unsigned trash32 = hist32 + 4u * (unsigned)(n_bins + lane);
+    const BinGuess guess = P.guess;
+
+    const TriGrid g = P.grids[frame];
+    const TriBox h = g.h;
+    const float4 *s1 = P.s1 + (int64_t)frame * P.n1;
+    const float4 *s2 = P.s2 + (int64_t)frame * P.n2;
+    const int *k2 = P.k2 + (int64_t)frame * P.n2;
+    const int *start = P.start2 + (int64_t)frame * P.cstride;
+
+    const int i = blockIdx.x * kThreads + tid;
+    const bool valid = i < P.n1;
+    const float4 pi = s1[min(i, P.n1 - 1)];
+    const int gi = __float_as_int(pi.w);
+    unsigned ki;
+    const int my_cell = tri_cell(pi, g, ki);
+    const int cx = my_cell % g.nc[0], cy = (my_cell / g.nc[0]) % g.nc[1],
+              cz = my_cell / (g.nc[0] * g.nc[1]);
+    const unsigned kneg = __vsub4(0u, ki);          // -k_i per byte
+    unsigned long long my_evals = 0;
+
+    auto bin = [&](double d2, bool keep, unsigned w) {
+        if (FAST) {
+            bool below;
+            const int j = slot_fast_parts(d2, sT, n_bins, guess, below);
+            unsigned a = (below ? hist32 - 4u : hist32) + 4u * (unsigned)j;
+            if ((!below && j == n_bins) || !keep) a = trash32;
+            red_shared(a, w);
+        } else {
+            const int slot = slot_search(d2, sT, n_bins);
+            if (keep && (unsigned)(slot - 1) < (unsigned)n_bins) atomicAdd(&myhist[slot - 1], w);
+        }
+    };
+
+    if (P.far[frame]) {
+        // the margin does not hold for this frame: every ordered pair, all 27 images
+        if (valid) {
+            for (int j = 0; j < P.n2; ++j) {
+                const float4 pj = s2[j];
+                bin(tri_d2(pi.x, pi.y, pi.z, pj, h), !(EXCL && gi == __float_as_int(pj.w)),
+                    1u);
+            }
+            my_evals += P.n2;
+        }
+    } else {
+        // candidates s2[b, b + len); base = (w - k_i) per byte: m' = k_j + base
+        auto sweep = [&](int b, int len, unsigned base, unsigned w_first, unsigned w_rest) {
+            if (!valid) return;
+            my_evals += len;
+            for (int t = 0; t < len; ++t) {
+                const float4 pj = __ldg(s2 + b + t);
+                const unsigned m = __vadd4((unsigned)__ldg(k2 + b + t), base);
+                // every byte in {-1, 0, 1} (byte 3 is 0)
+                const bool ref_image = __vcmpleu4(__vadd4(m, 0x00010101u), 0x00020202u) ==
+                                       0xffffffffu;
+                const int ix = (int)(signed char)(m & 0xffu);
+                const int iy = (int)(signed char)((m >> 8) & 0xffu);
+                const int iz = (int)(signed char)((m >> 16) & 0xffu);
+                auto sh = [](double v, int s) { return s == 0 ? 0.0 : (s > 0 ? v : -v); };
+                const double d2 = tri_image_d2(
+                    (double)__fsub_rn(pj.x, pi.x), (double)__fsub_rn(pj.y, pi.y),
+                    (double)__fsub_rn(pj.z, pi.z), sh(h.ax, ix), sh(h.bx, iy), sh(h.by, iy),
+                    sh(h.cx, iz), sh(h.cy, iz), sh(h.cz, iz));
+                bin(d2, ref_image && !(EXCL && gi == __float_as_int(pj.w)),
+                    t == 0 ? w_first : w_rest);
+            }
+        };
+        auto wrap = [](int v, int n, int &w) {
+            w = v < 0 ? -1 : (v >= n ? 1 : 0);
+            return v - w * n;
+        };
+        auto code = [](int wa, int wb, int wc) {
+            return ((unsigned)wa & 0xffu) | (((unsigned)wb & 0xffu) << 8) |
+                   (((unsigned)wc & 0xffu) << 16);
+        };
+        // the three x-adjacent cells of row (cy + dy, cz + dz) are one contiguous range of
+        // the sorted array, plus one more cell when the x stencil wraps around the cell
+        auto sweep_row = [&](int dy, int dz, unsigned w) {
+            int wb, wc;
+            const int y = wrap(cy + dy, g.nc[1], wb), z = wrap(cz + dz, g.nc[2], wc);
+            const int row = (z * g.nc[1] + y) * g.nc[0];
+            const int xa = max(cx - 1, 0), xb = min(cx + 1, g.nc[0] - 1);
+            const int b0 = start[row + xa];
+            sweep(b0, start[row + xb + 1] - b0, __vadd4(code(0, wb, wc), kneg), w, w);
+            if (cx == 0 || cx == g.nc[0] - 1) {
+                const int wa = cx == 0 ? -1 : 1, xw = cx == 0 ? g.nc[0] - 1 : 0;
+                const int bw = start[row + xw];
+                sweep(bw, start[row + xw + 1] - bw, __vadd4(code(wa, wb, wc), kneg), w, w);
+            }
+        };
+        if (!P.half) {
+            for (int dz = -1; dz <= 1; ++dz)
+                for (int dy = -1; dy <= 1; ++dy) sweep_row(dy, dz, 1u);
+        } else {
+            // forward offsets (dz, dy, dx) > 0 in lexicographic order, weight 2 for both
+            // orders ((i, j) and (j, i) have the same 27-image minimum: float rounding is
+            // odd-symmetric); the own cell from j = i: the self pair once
+            for (int dy = -1; dy <= 1; ++dy) sweep_row(dy, 1, 2u);
+            sweep_row(1, 0, 2u);
+            const int row = (cz * g.nc[1] + cy) * g.nc[0];
+            int wa;
+            const int xr = wrap(cx + 1, g.nc[0], wa);
+            const int br = start[row + xr];
+            sweep(br, start[row + xr + 1] - br, __vadd4(code(wa, 0, 0), kneg), 2u, 2u);
+            sweep(i, start[row + cx + 1] - i, kneg, 1u, 2u);
+        }
+    }
+    __syncthreads();
+    for (int k = tid; k < n_bins; k += kThreads) {
+        unsigned long long s = 0;
+#pragma unroll
+        for (int w = 0; w < kWarps; ++w) s += sH[w * warp_hist_words(n_bins) + 1 + k];
+        if (s) atomicAdd(&P.counts[k], s);
+    }
+    for (int o = 16; o; o >>= 1) my_evals += __shfl_xor_sync(0xffffffffu, my_evals, o);
+    if (lane == 0 && my_evals) atomicAdd(P.evals, my_evals);
+}
+
+template <bool EXCL, bool FAST>
+int launch_tri_cells(mdh_ctx *c, const TriCellParams &P, dim3 grid)
+{
+    const size_t smem = tri_cells_smem_bytes(P.n_bins);
+    auto kern = rdf_tri_cells_kernel<EXCL, FAST>;
+    MDH_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<grid, kThreads, smem, c->stream>>>(P);
+    MDH_CUDA(cudaGetLastError());
+    c->launches++;
+    return MDH_OK;
+}
+
+// ---- grid planner (host, no device) ------------------------------------------------------
+//
+// Why one image per candidate gives the reference's counts.  Cells are cut in fractional
+// coordinates, n_k >= 3 per axis, and every cell's perpendicular width w_k / n_k is at least
+// r + M (r = sqrt(U), U the last squared threshold).  Let p_i = r_i + k_i H be particle i's
+// position in the cell (tri_cell).  The 3x3x3 block of cells around p_i's cell spans less
+// than one period per axis (n_k >= 3), so exactly one lattice image of j lies in it,
+// p_j + w H = r_j + m' H, m' = k_j - k_i + w; every other image of j -- and every image of
+// a j whose cell is not in the block -- differs from p_i in some fractional coordinate k by
+// at least 1 / n_k - 2 eps_k (eps_k: error of the computed fractional coordinates), i.e. is
+// at least w_k / n_k - 2 eps_k w_k >= r + M - 2 eps_k w_k away.  The reference computes
+// d^2 from dx~ = (float)(r_j - r_i) instead of the exact difference, and rounds the image
+// sums and squares in fp64.  With
+//   M = max_k 2 eps_k w_k            (cell assignment)
+//     + e_f                          (dx~: |dx~ - dx| <= 2^-24 |dx| per component)
+//     + e_d                          (fp64 image sums)
+//     + 1e-5 r                       (fp64 squares and sums of d^2, r = sqrt(U) rounding)
+// every image but m' has a computed d^2 above U, so min27 <= U implies min27 = d^2(m') and
+// m' in {-1, 0, 1}^3; otherwise both are above U and neither is counted.  The kernel
+// computes d^2(m') with tri_image_d2 (same operations, same bits).
+//
+// Bounds.  Unless a frame is "far" (tri_far; such frames take the 27-image arithmetic for
+// every pair), wrapped coordinates lie within [-E_k / 2, 3 E_k / 2], E = (a_x, b_y, c_z),
+// so |dx_k| <= 2 E_k and e_f = 2^-24 * 2 |E|.  Image sums: three fp64 additions of terms
+// below 2 E_k + sum_k' |H_k'k| per component: e_d = 4 * 2^-53 |that vector|.  eps_k follows
+// the operations of tri_cell step by step (every rounding: 2^-53 of the bound on its
+// result), doubled to absorb second-order terms; fractional part and product with n_k add
+// 2^-53.  The shifts k are bounded by the magnitude bounds of s (|k| <= |s| + 1); a cell
+// whose bound exceeds kTriShiftMax gets no grid.
+struct TriPlan {
+    int nc[3];        // cells per axis (0: fewer than 3 fit)
+    int fit[3];       // cells per axis before the cap and the occupancy rule
+    double margin;    // M
+};
+
+int tri_grid_plan(const float *m9, double r_hi, int64_t n_max, TriPlan &out)
+{
+    MDH_REQUIRE(m9 != nullptr, MDH_EINVAL, "rdf: cell matrix is NULL");
+    MDH_REQUIRE(m9[1] == 0.f && m9[2] == 0.f && m9[5] == 0.f, MDH_EINVAL,
+                "rdf: the cell matrix is not lower triangular");
+    for (int k = 0; k < 9; ++k)
+        MDH_REQUIRE(std::isfinite(m9[k]), MDH_EINVAL, "rdf: the cell matrix is not finite");
+    MDH_REQUIRE(m9[0] > 0.f && m9[4] > 0.f && m9[8] > 0.f, MDH_EINVAL,
+                "rdf: the cell matrix is not a valid cell");
+    MDH_REQUIRE(r_hi >= 0.0 && std::isfinite(r_hi), MDH_EINVAL, "rdf: invalid r_max");
+    const double ax = m9[0], bx = m9[3], by = m9[4], cx = m9[6], cy = m9[7], cz = m9[8];
+    const double u = 1.0 / 9007199254740992.0;           // 2^-53
+    // magnitude bounds (B) and absolute errors (e) of the steps of tri_cell
+    const double X = 1.5 * ax, Y = 1.5 * by, Z = 1.5 * cz;
+    const double Bc = Z / cz * (1 + u), ec = u * Bc;                     // s_c = z / c_z
+    const double Bp1 = Bc * std::fabs(cy) * (1 + u), ep1 = std::fabs(cy) * ec + u * Bp1;
+    const double Bt = (Y + Bp1) * (1 + u), et = ep1 + u * Bt;            // y - s_c c_y
+    const double Bb = Bt / by * (1 + u), eb = et / by + u * Bb;          // s_b
+    const double Bq1 = Bb * std::fabs(bx) * (1 + u), eq1 = std::fabs(bx) * eb + u * Bq1;
+    const double Br1 = (X + Bq1) * (1 + u), er1 = eq1 + u * Br1;         // x - s_b b_x
+    const double Bq2 = Bc * std::fabs(cx) * (1 + u), eq2 = std::fabs(cx) * ec + u * Bq2;
+    const double Br2 = (Br1 + Bq2) * (1 + u), er2 = er1 + eq2 + u * Br2; // ... - s_c c_x
+    const double Ba = Br2 / ax * (1 + u), ea = er2 / ax + u * Ba;        // s_a
+    const double eps[3] = {2 * ea + u, 2 * eb + u, 2 * ec + u};
+    const double B[3] = {Ba, Bb, Bc};
+    // perpendicular widths V / |b x c|, V / |c x a|, c_z (lower bounds)
+    const double w[3] = {
+        ax * by * cz / std::sqrt(by * cz * by * cz + bx * cz * bx * cz +
+                                 (bx * cy - by * cx) * (bx * cy - by * cx)) * (1 - 1e-12),
+        by * cz / std::sqrt(cy * cy + cz * cz) * (1 - 1e-12), cz};
+    const double E = std::sqrt(ax * ax + by * by + cz * cz);
+    const double rows[3] = {2 * ax + ax + std::fabs(bx) + std::fabs(cx),
+                            2 * by + by + std::fabs(cy), 2 * cz + cz};
+    const double e_f = 2.0 * E / 16777216.0;
+    const double e_d = 4 * u * std::sqrt(rows[0] * rows[0] + rows[1] * rows[1] + rows[2] * rows[2]);
+    double e_a = 0.0;
+    for (int k = 0; k < 3; ++k) e_a = std::max(e_a, 2.0 * eps[k] * w[k]);
+    out.margin = e_a + e_f + e_d + 1e-5 * r_hi;
+    const double width = r_hi + out.margin;
+    bool shifts_ok = true;
+    for (int k = 0; k < 3; ++k) shifts_ok = shifts_ok && B[k] + 1.0 <= kTriShiftMax;
+    double ncell = 1;
+    for (int k = 0; k < 3; ++k) {
+        double f = std::floor(w[k] / width);
+        while (f >= 1.0 && w[k] / f < width) f -= 1.0;     // w_k / n_k >= r + M exactly
+        out.fit[k] = (int)std::min(f, 1e6);
+        out.nc[k] = std::min(out.fit[k], 160);
+        ncell *= out.nc[k];
+    }
+    if (!shifts_ok || std::min({out.nc[0], out.nc[1], out.nc[2]}) < 3) {
+        for (int k = 0; k < 3; ++k) out.nc[k] = 0;
+        return MDH_OK;
+    }
+    // keep at least ~2 particles per cell on average
+    const double want = std::max(27.0, (double)n_max / 2.0);
+    while (ncell > want) {
+        int kmax = 0;
+        for (int k = 1; k < 3; ++k) if (out.nc[k] > out.nc[kmax]) kmax = k;
+        if (out.nc[kmax] <= 3) break;
+        ncell = ncell / out.nc[kmax] * (out.nc[kmax] - 1);
+        out.nc[kmax]--;
+    }
+    return MDH_OK;
+}
+
+}  // namespace
+
+int rdf_triclinic_grid_impl(const float *cell9, double r_hi, int64_t n_max, int32_t *nc,
+                            double *margin)
+{
+    MDH_REQUIRE(nc != nullptr && margin != nullptr, MDH_EINVAL, "triclinic_grid: NULL output");
+    TriPlan pl;
+    if (int rc = tri_grid_plan(cell9, r_hi, n_max, pl)) return rc;
+    for (int k = 0; k < 3; ++k) nc[k] = pl.nc[k];
+    *margin = pl.margin;
+    return MDH_OK;
+}
+
+namespace {
+
+// Device layout of the scratch (RdfState::cell) on this path:
+//   cell[0] TriBox[F]   cell[5] TriGrid[F]   cell[1] int cnt[2][G][cstride] | far[G]
+//   cell[2] int start[2][G][cstride]   cell[3] int2 keyrank[G][n1]   cell[4] float4 sorted1
+//   cell[6] int kcode[G][n1] | [G][n2]   cell[7] keyrank2   cell[8] sorted2   cell[9] evals
+int tri_cells_accumulate(mdh_ctx *c, const std::vector<TriGrid> &grids, int64_t pad1,
+                         int64_t pad2)
+{
+    RdfState &R = c->rdf;
+    const int n_frames = (int)grids.size();
+    int ncell_max = 0;
+    for (const TriGrid &g : grids) ncell_max = std::max(ncell_max, g.ncell);
+    const int cstride = ncell_max + 1;
+    DevBuf &d_grids = R.cell[5];
+    if (int rc = d_grids.reserve(sizeof(TriGrid) * n_frames)) return rc;
+    // pageable source: the runtime stages it before returning
+    MDH_CUDA(cudaMemcpyAsync(d_grids.p, grids.data(), sizeof(TriGrid) * n_frames,
+                             cudaMemcpyHostToDevice, c->stream));
+    // frames per group: what one group reads and writes between the passes should stay
+    // in L2 (the rule of rdf_cells_accumulate; 44 bytes per particle here)
+    const int n_groups = R.same ? 1 : 2;
+    const int64_t n1 = R.n1, n2 = R.n2;
+    const double per_frame = 44.0 * (double)(n1 + (R.same ? 0 : n2)) + 8.0 * cstride * n_groups;
+    int G = (int)std::max(1.0, std::min(64.0, floor(R.cells_ws_mb * 1048576.0 / per_frame)));
+    G = std::min(G, n_frames);
+    const size_t cnt_words = (size_t)2 * G * cstride, reset_words = cnt_words + G;
+    if (int rc = R.cell[1].reserve(sizeof(int) * reset_words)) return rc;
+    if (int rc = R.cell[2].reserve(sizeof(int) * cnt_words)) return rc;
+    if (int rc = R.cell[3].reserve(sizeof(int2) * (size_t)n1 * G)) return rc;
+    if (int rc = R.cell[4].reserve(sizeof(float4) * (size_t)n1 * G)) return rc;
+    if (int rc = R.cell[6].reserve(sizeof(int) * (size_t)(n1 + (R.same ? 0 : n2)) * G))
+        return rc;
+    if (!R.same) {
+        if (int rc = R.cell[7].reserve(sizeof(int2) * (size_t)n2 * G)) return rc;
+        if (int rc = R.cell[8].reserve(sizeof(float4) * (size_t)n2 * G)) return rc;
+    }
+    int *d_cnt = R.cell[1].as<int>(), *d_far = d_cnt + cnt_words;
+    int *d_start = R.cell[2].as<int>();
+    int *d_k1 = R.cell[6].as<int>(), *d_k2 = R.same ? d_k1 : d_k1 + (size_t)n1 * G;
+    const size_t scan_smem = sizeof(int) * (kScanTile + kScanTile / 32);
+    MDH_CUDA(cudaFuncSetAttribute(cells_scan_kernel<TriGrid>,
+                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)scan_smem));
+    const bool excl = R.excl1 > 0, fast = R.fast_bins;
+    for (int g0 = 0; g0 < n_frames; g0 += G) {
+        const int ng = std::min(G, n_frames - g0);
+        MDH_CUDA(cudaMemsetAsync(d_cnt, 0, sizeof(int) * reset_words, c->stream));
+        const TriGrid *gg = d_grids.as<TriGrid>() + g0;
+        for (int grp = 0; grp < n_groups; ++grp) {
+            const float4 *pk = (grp ? R.pk2 : R.pk1).as<float4>() + (int64_t)g0 * (grp ? pad2 : pad1);
+            const int n = (int)(grp ? n2 : n1);
+            dim3 grid((unsigned)std::min((n + 255) / 256, 4096), ng);
+            tri_bin_kernel<<<grid, 256, 0, c->stream>>>(
+                pk, grp ? pad2 : pad1, n, gg, d_cnt + (size_t)grp * G * cstride, cstride,
+                R.cell[grp ? 7 : 3].as<int2>(), d_far);
+            MDH_CUDA(cudaGetLastError());
+            c->launches++;
+        }
+        ScanFilter F{};
+        F.out = nullptr;
+        cells_scan_kernel<TriGrid><<<dim3(ng, n_groups), 1024, scan_smem, c->stream>>>(
+            d_cnt, d_start, cstride, G, gg, F);
+        MDH_CUDA(cudaGetLastError());
+        c->launches++;
+        for (int grp = 0; grp < n_groups; ++grp) {
+            const float4 *pk = (grp ? R.pk2 : R.pk1).as<float4>() + (int64_t)g0 * (grp ? pad2 : pad1);
+            const int n = (int)(grp ? n2 : n1);
+            dim3 grid((unsigned)std::min((n + 255) / 256, 4096), ng);
+            tri_scatter_kernel<<<grid, 256, 0, c->stream>>>(
+                pk, grp ? pad2 : pad1, n, gg, d_start + (size_t)grp * G * cstride, cstride,
+                R.cell[grp ? 7 : 3].as<int2>(), R.cell[grp ? 8 : 4].as<float4>(),
+                grp ? d_k2 : d_k1);
+            MDH_CUDA(cudaGetLastError());
+            c->launches++;
+        }
+        TriCellParams P;
+        P.s1 = R.cell[4].as<float4>();
+        P.s2 = R.same ? P.s1 : R.cell[8].as<float4>();
+        P.k2 = d_k2;
+        P.n1 = (int)n1; P.n2 = (int)n2;
+        P.start2 = R.same ? d_start : d_start + (size_t)G * cstride;
+        P.cstride = cstride;
+        P.grids = gg;
+        P.far = d_far;
+        P.thr = R.thr.as<double>();
+        P.n_bins = R.n_bins;
+        P.guess = rdf_bin_guess(R);
+        P.counts = R.counts.as<unsigned long long>();
+        P.evals = R.cell[9].as<unsigned long long>();
+        P.half = R.same;
+        dim3 grid((unsigned)((n1 + kThreads - 1) / kThreads), (unsigned)ng);
+        int rc;
+        if (excl) rc = fast ? launch_tri_cells<true, true>(c, P, grid)
+                            : launch_tri_cells<true, false>(c, P, grid);
+        else rc = fast ? launch_tri_cells<false, true>(c, P, grid)
+                       : launch_tri_cells<false, false>(c, P, grid);
+        if (rc) return rc;
+    }
+    return MDH_OK;
+}
+
 }  // namespace
 
 // pack kernel of rdf_device.cuh is instantiated in this translation unit as well
@@ -157,7 +657,6 @@ int rdf_accumulate_triclinic_impl(mdh_ctx *c, const float *pos1, int64_t s1, con
     MDH_REQUIRE(R.drop_axis < 0, MDH_EINVAL, "rdf: drop_axis needs an orthorhombic cell");
     const size_t smem = align16(sizeof(double) * (R.n_bins + 1)) + 256 * sizeof(float4) +
                         sizeof(unsigned) * kWarps * (size_t)R.n_bins;
-    MDH_REQUIRE(smem <= kMaxSmem, MDH_EINVAL, "rdf: too many bins for the triclinic kernel");
 
     std::vector<TriBox> hb(n_frames);
     for (int f = 0; f < n_frames; ++f) {
@@ -170,6 +669,46 @@ int rdf_accumulate_triclinic_impl(mdh_ctx *c, const float *pos1, int64_t s1, con
         hb[f] = TriBox{(double)m[0], (double)m[3], (double)m[4], (double)m[6], (double)m[7],
                        (double)m[8]};
     }
+
+    // pair kernel: the cell list when asked for, or (auto) when every frame holds at least
+    // 4 cells per axis and there are enough pairs -- the orthorhombic rule, applied to the
+    // perpendicular widths
+    int mode = R.mode;
+    std::vector<TriGrid> grids;
+    if (mode != MDH_RDF_ALLPAIRS) {
+        const double r_hi = sqrt(R.thr_hi);
+        bool fit4 = tri_cells_smem_bytes(R.n_bins) <= kMaxSmem && R.n1 <= (1ll << 25) &&
+                    R.n2 <= (1ll << 25);
+        grids.resize(n_frames);
+        for (int f = 0; f < n_frames && (mode == MDH_RDF_CELLS || fit4); ++f) {
+            TriPlan pl;
+            if (int rc = tri_grid_plan(box9 + 9 * f, r_hi, std::max(R.n1, R.n2), pl)) {
+                if (mode == MDH_RDF_CELLS) return rc;
+                fit4 = false;                 // (auto) e.g. a non-finite tilt: all pairs
+                break;
+            }
+            if (mode == MDH_RDF_CELLS)
+                MDH_REQUIRE(pl.nc[0] >= 3, MDH_EINVAL,
+                            "rdf: cell-list mode needs every perpendicular width of the cell >= "
+                            "3*(r_max + %g) (frame %d: %d, %d, %d cells fit)", pl.margin, f,
+                            pl.fit[0], pl.fit[1], pl.fit[2]);
+            fit4 = fit4 && pl.nc[0] >= 3 && std::min({pl.fit[0], pl.fit[1], pl.fit[2]}) >= 4;
+            grids[f].h = hb[f];
+            for (int k = 0; k < 3; ++k) grids[f].nc[k] = pl.nc[k];
+            grids[f].ncell = pl.nc[0] * pl.nc[1] * pl.nc[2];
+        }
+        if (mode == MDH_RDF_AUTO)
+            mode = fit4 && (double)R.n1 * (double)R.n2 >= 4e6 ? MDH_RDF_CELLS : MDH_RDF_ALLPAIRS;
+    }
+    if (mode == MDH_RDF_CELLS) {
+        MDH_REQUIRE(tri_cells_smem_bytes(R.n_bins) <= kMaxSmem, MDH_EINVAL,
+                    "rdf: too many bins for the triclinic cell-list kernel");
+        MDH_REQUIRE(R.n1 <= (1ll << 25) && R.n2 <= (1ll << 25), MDH_EINVAL,
+                    "rdf: cell-list mode takes at most 2^25 particles per group");
+    } else {
+        MDH_REQUIRE(smem <= kMaxSmem, MDH_EINVAL, "rdf: too many bins for the triclinic kernel");
+    }
+
     DevBuf &d_box = R.cell[0];
     if (int rc = d_box.reserve(sizeof(TriBox) * n_frames)) return rc;
     MDH_CUDA(cudaMemcpyAsync(d_box.p, hb.data(), sizeof(TriBox) * n_frames,
@@ -178,6 +717,9 @@ int rdf_accumulate_triclinic_impl(mdh_ctx *c, const float *pos1, int64_t s1, con
 
     const int64_t pad1 = (R.n1 + 255) / 256 * 256, pad2 = (R.n2 + 255) / 256 * 256;
     const int n_groups = R.same ? 1 : 2;
+    // the cell-list path times its whole pipeline (pack and wrap included)
+    if (mode == MDH_RDF_CELLS)
+        if (int rc = c->t_rdf.begin(c->stream)) return rc;
     for (int g = 0; g < n_groups; ++g) {
         const float *pos = g ? pos2 : pos1;
         const int64_t stride = g ? s2 : s1, n = g ? R.n2 : R.n1, npad = g ? pad2 : pad1;
@@ -202,6 +744,10 @@ int rdf_accumulate_triclinic_impl(mdh_ctx *c, const float *pos1, int64_t s1, con
                                                      d_box.as<TriBox>());
         MDH_CUDA(cudaGetLastError());
         c->launches += 2;
+    }
+    if (mode == MDH_RDF_CELLS) {
+        if (int rc = tri_cells_accumulate(c, grids, pad1, pad2)) return rc;
+        return c->t_rdf.end(c->stream);
     }
 
     TriParams P;
