@@ -151,7 +151,11 @@ int mdh_launch_count(mdh_ctx *ctx, int64_t *launches);
  * excl1, excl2  exclusion block sizes: pairs with i/excl1 == j/excl2 are dropped
  *               (structure.py:100-102); 0, 0 disables.
  * drop_axis     -1, or 0/1/2: that coordinate is zeroed before the distance
- *               (structure.py:766-767; the caller passes the widened box edge).
+ *               (structure.py:766-767; the caller passes the widened box edge, or for
+ *               mdh_rdf_accumulate_triclinic the cell matrix of the widened dimensions).
+ *               Orthorhombic cells: every mode; the cell list then has one cell along the
+ *               dropped axis.  Triclinic cells: all pairs for every axis, the cell list
+ *               for drop_axis 2 only (see mdh_rdf_accumulate_triclinic).
  * mode, hist    MDH_RDF_* / MDH_HIST_* selectors.
  * Resets the accumulated counts.
  */
@@ -175,9 +179,15 @@ int mdh_rdf_accumulate(mdh_ctx *ctx, const float *pos1, int64_t frame_stride1,
  * MDH_RDF_CELLS uses a cell list in fractional coordinates and evaluates, per candidate,
  * the one image that can be in range (same counts; MDH_EINVAL if some frame fits fewer
  * than 3 cells on an axis, see mdh_rdf_triclinic_grid); MDH_RDF_AUTO takes the cell list
- * when every frame fits at least 4 cells per axis and n1*n2 >= 4e6.  drop_axis is not
- * available.  Restated from MDAnalysis' published algorithm and NOT pinned against
- * MDAnalysis (see DESIGN.md).
+ * when every frame fits at least 4 cells per axis and n1*n2 >= 4e6.  drop_axis: the
+ * coordinate is zeroed before the wrap (which may move it again on a tilted cell, as in
+ * the reference); every axis runs through all pairs.  With drop_axis 2 the cell list is
+ * a flat grid of the (a, b) plane (one cell along c, mdh_rdf_cells_grid); it needs
+ * c_z >= r_hi + M besides 3 cells per in-plane width (else MDH_EINVAL in MDH_RDF_CELLS,
+ * all pairs in MDH_RDF_AUTO, whose rule is otherwise the one above for the two kept
+ * widths).  drop_axis 0 or 1: MDH_RDF_CELLS is MDH_EINVAL, MDH_RDF_AUTO takes all pairs.
+ * Restated from MDAnalysis' published algorithm and NOT pinned against MDAnalysis (see
+ * DESIGN.md).
  */
 int mdh_rdf_accumulate_triclinic(mdh_ctx *ctx, const float *pos1, int64_t frame_stride1,
                                  const float *pos2, int64_t frame_stride2, int location,
@@ -192,6 +202,19 @@ int mdh_rdf_accumulate_triclinic(mdh_ctx *ctx, const float *pos1, int64_t frame_
  */
 int mdh_rdf_triclinic_grid(const float *cell /* [9] */, double r_hi, int64_t n_max,
                            int32_t *nc /* [3] */, double *margin);
+
+/*
+ * Cell-list grid of one frame for any cell and drop_axis (-1, 0, 1, 2), as
+ * mdh_rdf_accumulate (diagonal cell) or mdh_rdf_accumulate_triclinic (any other cell)
+ * would use it; device-free.  cell, r_hi, n_max as for mdh_rdf_triclinic_grid.  Writes the
+ * cells per axis (x, y, z or a, b, c; one along a dropped axis; all 0 when fewer than 3
+ * fit on a kept axis) and the margin M: every cell is at least r_hi + M wide on a kept
+ * axis (diagonal cells: M = 1e-5 r_hi).  MDH_EINVAL for a triclinic cell with drop_axis 0
+ * or 1 (no cell list) and for drop_axis 2 with c_z < r_hi + M.  With drop_axis -1 and a
+ * triclinic cell it gives what mdh_rdf_triclinic_grid gives.
+ */
+int mdh_rdf_cells_grid(const float *cell /* [9] */, double r_hi, int64_t n_max, int drop_axis,
+                       int32_t *nc /* [3] */, double *margin);
 
 int mdh_rdf_fetch(mdh_ctx *ctx, int64_t *counts /* [n_bins] host */);
 int mdh_rdf_reset(mdh_ctx *ctx);

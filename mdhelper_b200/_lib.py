@@ -48,6 +48,7 @@ SIGNATURES = {
     "mdh_rdf_accumulate": (_i32, [_p, _p, _i64, _p, _i64, _i32, _p, _i32]),
     "mdh_rdf_accumulate_triclinic": (_i32, [_p, _p, _i64, _p, _i64, _i32, _p, _i32]),
     "mdh_rdf_triclinic_grid": (_i32, [_p, _f64, _i64, _p, ctypes.POINTER(_f64)]),
+    "mdh_rdf_cells_grid": (_i32, [_p, _f64, _i64, _i32, _p, ctypes.POINTER(_f64)]),
     "mdh_rdf_fetch": (_i32, [_p, _p]),
     "mdh_rdf_reset": (_i32, [_p]),
     "mdh_rdf_counts_device": (_i32, [_p, ctypes.POINTER(_p)]),
@@ -160,6 +161,22 @@ def triclinic_grid(cell, r_hi: float, n_max: int):
     margin = _f64(0.0)
     check(lib().mdh_rdf_triclinic_grid(m.ctypes.data, float(r_hi), int(n_max), nc.ctypes.data,
                                        ctypes.byref(margin)))
+    return tuple(int(v) for v in nc), margin.value
+
+
+def cells_grid(cell, r_hi: float, n_max: int, drop_axis=None):
+    """Cell-list grid of one frame for any cell and ``drop_axis`` (``mdh_rdf_cells_grid``; no
+    device needed): ``(cells per axis, margin M)``.  A diagonal ``cell`` gets the grid of the
+    orthorhombic cell list, any other the triclinic one; one cell along a dropped axis,
+    ``(0, 0, 0)`` when fewer than 3 fit on a kept axis.  Raises ``ValueError`` where the
+    cell list is not offered: a triclinic cell with ``drop_axis`` 0 or 1, or ``drop_axis`` 2
+    with ``c_z < r_hi + M``."""
+    m = np.ascontiguousarray(cell, dtype=np.float32).reshape(9)
+    nc = np.zeros(3, dtype=np.int32)
+    margin = _f64(0.0)
+    check(lib().mdh_rdf_cells_grid(m.ctypes.data, float(r_hi), int(n_max),
+                                   -1 if drop_axis is None else int(drop_axis), nc.ctypes.data,
+                                   ctypes.byref(margin)))
     return tuple(int(v) for v in nc), margin.value
 
 

@@ -235,8 +235,16 @@ class RadialDistributionFunction(GpuAnalysisBase):
       every pair, ``mode="cells"`` a cell list in fractional coordinates that evaluates
       the one image per candidate that can be in range (same counts; every perpendicular
       width of the cell must hold 3 cells of ``range[1]`` plus a small margin), and
-      ``"auto"`` takes the cell list for cut-off runs on large systems.  ``drop_axis``
-      needs an orthorhombic cell.
+      ``"auto"`` takes the cell list for cut-off runs on large systems.
+    * ``drop_axis`` works with every cell shape and ``mode``, as in the reference: the
+      coordinate is zeroed, the dropped edge is widened to the longest one (a triclinic
+      cell keeps its angles) and the accumulated area is the product of the two other
+      edges -- for a hexagonal cell ``a * b``, not ``a * b * sin(gamma)``, which is what
+      the reference computes.  The cell list takes a dropped axis with one cell along it
+      (orthorhombic cells: any axis; triclinic cells: ``drop_axis=2`` only, with
+      ``c_z`` at least ``range[1]`` plus a small margin).  ``mode="cells"`` raises
+      ``ValueError`` for a triclinic cell with ``drop_axis`` 0 or 1, which
+      ``"auto"`` runs through all pairs.
     """
 
     def __init__(
@@ -358,13 +366,15 @@ class RadialDistributionFunction(GpuAnalysisBase):
             for d, o, v in zip(batch.dims, ortho, box.astype(np.float64).prod(axis=1)):
                 self._area_or_volume += v if o else box_volume(d)
         else:
-            if not ortho.all():
-                raise NotImplementedError("drop_axis needs an orthorhombic cell.")
-            # reference: structure.py:764-770
+            # reference: structure.py:764-770 -- the dropped edge widened to the longest one,
+            # the angles kept; the area is the product of the two other edges for every cell
+            # shape (a * b for a hexagonal cell, not a * b * sin(gamma): as the reference)
             box[:, self._drop_axis] = box.max(axis=1)
             keep = [k for k in (0, 1, 2) if k != self._drop_axis]
             for v in box[:, keep].astype(np.float64).prod(axis=1):
                 self._area_or_volume += v
+        dims = batch.dims.copy()
+        dims[:, :3] = box
         same = self._same
         ptrs, strides = batch.ptrs, batch.strides
         if self._com is not None:
@@ -393,10 +403,11 @@ class RadialDistributionFunction(GpuAnalysisBase):
                 self._ctx.rdf_accumulate(p1, strides[0], p2, s2, box[f0:f1], f1 - f0,
                                          device=device, keepalive=batch.keepalive)
             else:
-                # triclinic: coordinates wrapped into the cell, shortest of 27 images
+                # triclinic: coordinates wrapped into the cell (of the widened dimensions
+                # with drop_axis), shortest of 27 images
                 self._ctx.rdf_accumulate_triclinic(
                     p1, strides[0], p1 if same else p2, strides[0] if same else s2,
-                    _cell_matrices(batch.dims[f0:f1]), f1 - f0, device=device,
+                    _cell_matrices(dims[f0:f1]), f1 - f0, device=device,
                     keepalive=batch.keepalive)
             f0 = f1
         _record(batch)

@@ -339,6 +339,12 @@ int mdh_rdf_triclinic_grid(const float *cell, double r_hi, int64_t n_max, int32_
     return rdf_triclinic_grid_impl(cell, r_hi, n_max, nc, margin);
 }
 
+int mdh_rdf_cells_grid(const float *cell, double r_hi, int64_t n_max, int drop_axis,
+                       int32_t *nc, double *margin)
+{
+    return rdf_cells_grid_impl(cell, r_hi, n_max, drop_axis, nc, margin);
+}
+
 int mdh_rdf_fetch(mdh_ctx *c, int64_t *counts)
 {
     CTX_GUARD(c);

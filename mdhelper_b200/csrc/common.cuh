@@ -282,6 +282,8 @@ int rdf_accumulate_triclinic_impl(mdh_ctx *c, const float *pos1, int64_t s1, con
                                   int64_t s2, int location, const float *box9, int n_frames);
 int rdf_triclinic_grid_impl(const float *cell9, double r_hi, int64_t n_max, int32_t *nc,
                             double *margin);
+int rdf_cells_grid_impl(const float *cell9, double r_hi, int64_t n_max, int drop_axis,
+                        int32_t *nc, double *margin);
 // rdf_filter.cu
 int rdf_filter_sqrt_error(mdh_ctx *c, double *err);
 bool rdf_filter_configure(RdfState &R, const double *thr, double sqrt_err);

@@ -443,10 +443,11 @@ int rdf_accumulate_impl(mdh_ctx *c, const float *pos1, int64_t s1, const float *
 
     int mode = R.mode;
     if (mode == MDH_RDF_AUTO) {
-        // cells pay off when the cut-off sphere is a small part of the box
+        // cells pay off when the cut-off sphere (circle, with a dropped axis) is a small part
+        // of the box; min_edge leaves the dropped axis out
         const double r_cut = sqrt(R.thr_hi);
         const bool cells_ok = min_edge / (r_cut * 1.00001) >= 4.0 &&
-                              (double)R.n1 * (double)R.n2 >= 4e6 && R.drop_axis < 0;
+                              (double)R.n1 * (double)R.n2 >= 4e6;
         mode = cells_ok ? MDH_RDF_CELLS : MDH_RDF_ALLPAIRS;
     }
     // Host input is cut into pieces so that the copy of one piece (copy stream) overlaps

@@ -3,7 +3,8 @@
 // Same per-pair arithmetic and binning as rdf.cu / rdf_filter.cu (rdf_device.cuh); only
 // the set of candidate pairs shrinks: each frame's particles are counting-sorted into
 // cells of edge >= r_cut*(1+1e-5) and every cell meets the 27 surrounding cells of the j
-// group.  This is the role MDAnalysis' grid search ("nsgrid") plays behind
+// group (with drop_axis: one cell along the dropped axis, and the 9 cells of the plane).
+// This is the role MDAnalysis' grid search ("nsgrid") plays behind
 // capped_distance for the reference (call site
 // /root/reference/src/mdhelper/analysis/structure.py:93-96; SURVEY.md Appendix A items 2
 // and 4).  Counts are identical to the all-pairs kernels by construction: a pair closer
@@ -53,10 +54,15 @@ using namespace rdfdev;
 
 namespace {
 
+// Grid axis k runs along physical axis axis[k]; box, inv_w and nc are per GRID axis.  The
+// axes are the physical ones in order, except with a dropped axis (two-dimensional runs):
+// that one becomes grid axis 2 with a single cell, so that the stencils keep their runs of
+// three x-adjacent cells along a kept axis and only have to leave out the rows at dz != 0.
 struct CellGrid {          // per frame
     double box[3];
     double inv_w[3];       // nc / box
     int nc[3];
+    int axis[3];
     int ncell;
 };
 
@@ -72,10 +78,28 @@ __device__ __forceinline__ int cell_coord(float x, double box, double inv_w, int
 __device__ __forceinline__ int cell_id(float x, float y, float z, const CellGrid &g, int &cx,
                                        int &cy, int &cz)
 {
-    cx = cell_coord(x, g.box[0], g.inv_w[0], g.nc[0]);
-    cy = cell_coord(y, g.box[1], g.inv_w[1], g.nc[1]);
-    cz = cell_coord(z, g.box[2], g.inv_w[2], g.nc[2]);
+    auto pick = [&](int a) { return a == 0 ? x : (a == 1 ? y : z); };
+    cx = cell_coord(pick(g.axis[0]), g.box[0], g.inv_w[0], g.nc[0]);
+    cy = cell_coord(pick(g.axis[1]), g.box[1], g.inv_w[1], g.nc[1]);
+    cz = cell_coord(pick(g.axis[2]), g.box[2], g.inv_w[2], g.nc[2]);
     return (cz * g.nc[1] + cy) * g.nc[0] + cx;
+}
+
+// the coordinate the pair arithmetic sees: a dropped axis is zeroed first, as
+// rdf_pack_kernel does for the all-pairs kernels, then the grid-search wrap if the frame
+// takes it (ortho_pbc_f32 keeps +0 at +0)
+__device__ __forceinline__ float4 cells_coords(float x, float y, float z, int drop_axis,
+                                               const FrameBox &fb)
+{
+    if (drop_axis == 0) x = 0.f;
+    if (drop_axis == 1) y = 0.f;
+    if (drop_axis == 2) z = 0.f;
+    if (fb.prewrap) {
+        x = ortho_pbc_f32(x, fb.box[0]);
+        y = ortho_pbc_f32(y, fb.box[1]);
+        z = ortho_pbc_f32(z, fb.box[2]);
+    }
+    return make_float4(x, y, z, 0.f);
 }
 
 // ---- counting sort, straight from the raw coordinates ------------------------------
@@ -101,14 +125,14 @@ __global__ void __launch_bounds__(256)
     cells_bin_kernel(const float *__restrict__ raw, int64_t frame_stride, int n,
                      const CellGrid *__restrict__ grids, int *__restrict__ cnt, int cstride,
                      int2 *__restrict__ keyrank, unsigned *__restrict__ ext,
-                     const FrameBox *__restrict__ boxes)
+                     const FrameBox *__restrict__ boxes, int drop_axis)
 {
     __shared__ float stage[3 * 256];
     __shared__ unsigned red[8][6];
     const int frame = blockIdx.y, tid = threadIdx.x;
     const CellGrid g = grids[frame];
+    const FrameBox fb = boxes[frame];
     const float *src = raw + (int64_t)frame * frame_stride;
-    const bool prewrap = boxes[frame].prewrap != 0;
     unsigned lo[3] = {0xffffffffu, 0xffffffffu, 0xffffffffu}, hi[3] = {0u, 0u, 0u};
     for (int64_t i0 = (int64_t)blockIdx.x * 256; i0 < n; i0 += (int64_t)gridDim.x * 256) {
         load_xyz_256(src, i0, n, stage, tid);
@@ -118,12 +142,9 @@ __global__ void __launch_bounds__(256)
         // of a molecule, lattice-ordered fluids), and 32 atomics on a few addresses serialise
         const unsigned active = __ballot_sync(0xffffffffu, i < n);
         if (i < n) {
-            float x = stage[3 * tid], y = stage[3 * tid + 1], z = stage[3 * tid + 2];
-            if (prewrap) {
-                x = ortho_pbc_f32(x, g.box[0]);
-                y = ortho_pbc_f32(y, g.box[1]);
-                z = ortho_pbc_f32(z, g.box[2]);
-            }
+            const float4 v = cells_coords(stage[3 * tid], stage[3 * tid + 1], stage[3 * tid + 2],
+                                          drop_axis, fb);
+            const float x = v.x, y = v.y, z = v.z;
             int cx, cy, cz;
             const int cell = cell_id(x, y, z, g, cx, cy, cz);
             const unsigned peers = __match_any_sync(active, cell);
@@ -163,7 +184,7 @@ __global__ void __launch_bounds__(256)
     cells_scatter_kernel(const float *__restrict__ raw, int64_t frame_stride, int n, int64_t excl,
                          const int *__restrict__ start, int cstride,
                          const int2 *__restrict__ keyrank, float4 *__restrict__ sorted,
-                         const FrameBox *__restrict__ boxes)
+                         const FrameBox *__restrict__ boxes, int drop_axis)
 {
     __shared__ float stage[3 * 256];
     const int frame = blockIdx.y, tid = threadIdx.x;
@@ -175,13 +196,9 @@ __global__ void __launch_bounds__(256)
         const int64_t i = i0 + tid;
         if (i < n) {
             const int2 kr = keyrank[(int64_t)frame * n + i];
-            float4 v;
-            v.x = stage[3 * tid]; v.y = stage[3 * tid + 1]; v.z = stage[3 * tid + 2];
-            if (boxes[frame].prewrap) {          // the same values the binning pass saw
-                v.x = ortho_pbc_f32(v.x, boxes[frame].box[0]);
-                v.y = ortho_pbc_f32(v.y, boxes[frame].box[1]);
-                v.z = ortho_pbc_f32(v.z, boxes[frame].box[2]);
-            }
+            // the same values the binning pass saw
+            float4 v = cells_coords(stage[3 * tid], stage[3 * tid + 1], stage[3 * tid + 2],
+                                    drop_axis, boxes[frame]);
             v.w = __int_as_float((int)(excl > 0 ? i / excl : i));
             sorted[(int64_t)frame * n + st[kr.x] + kr.y] = v;
         }
@@ -318,9 +335,12 @@ __global__ void __launch_bounds__(kThreads, 2) rdf_cells_kernel(const CellParams
         sweep(bw, (valid && xw >= 0) ? start[row + xw + 1] - bw : 0, w, w);
     };
 
+    // a single cell along grid z (a dropped axis): the rows at dz = -1 and +1 would be the
+    // own row again -- the stencil is the 9 cells (half: 4 + own) of the plane
+    const int dz_max = g.nc[2] > 1 ? 1 : 0;
     if (!P.half) {
         // full stencil: every ordered (i, j) pair once
-        for (int dz = -1; dz <= 1; ++dz)
+        for (int dz = -dz_max; dz <= dz_max; ++dz)
             for (int dy = -1; dy <= 1; ++dy)
                 sweep_row(wrap(cy + dy, g.nc[1]), wrap(cz + dz, g.nc[2]), 1u);
     } else {
@@ -328,8 +348,9 @@ __global__ void __launch_bounds__(kThreads, 2) rdf_cells_kernel(const CellParams
         // lexicographic order visit every unordered pair of distinct cells exactly
         // once (the reverse offset belongs to the partner cell); weight 2 stands for
         // both orders.  The own cell contributes j >= i: the self pair once.
-        for (int dy = -1; dy <= 1; ++dy)
-            sweep_row(wrap(cy + dy, g.nc[1]), wrap(cz + 1, g.nc[2]), 2u);
+        if (dz_max)
+            for (int dy = -1; dy <= 1; ++dy)
+                sweep_row(wrap(cy + dy, g.nc[1]), wrap(cz + 1, g.nc[2]), 2u);
         sweep_row(wrap(cy + 1, g.nc[1]), cz, 2u);
         const int row = (cz * g.nc[1] + cy) * g.nc[0];
         const int xr = wrap(cx + 1, g.nc[0]);
@@ -584,8 +605,9 @@ __global__ void __launch_bounds__(kCpThreads, MDH_CP_BLOCKS)
                 const int row_i = r >> 1;            // 0..8 = (dz + 1) * 3 + (dy + 1)
                 const int dz = row_i / 3 - 1, dy = row_i % 3 - 1;
                 // same group: forward half only -- the rows at z + 1 (all dy), the row
-                // (y + 1, z) and the cell (x + 1, y, z) of the own row
-                bool use = !HALF || dz == 1 || (dz == 0 && dy >= 0);
+                // (y + 1, z) and the cell (x + 1, y, z) of the own row.  One cell along z
+                // (a dropped axis): the rows of the own plane only
+                bool use = (!HALF || dz == 1 || (dz == 0 && dy >= 0)) && (ncz > 1 || dz == 0);
                 int xa, xb;                          // cells [xa, xb] of the row
                 const int row = (wrap(cz + dz, ncz) * ncy + wrap(cy + dy, ncy)) * ncx;
                 if (HALF && dz == 0 && dy == 0) {
@@ -1012,6 +1034,38 @@ int cellpair_sub_bins(int n_bins, int sb_max, int cap)
 
 }  // namespace
 
+// Grid of the orthorhombic cell list for one frame, per PHYSICAL axis: cells of edge at least
+// r_cut = r_hi * (1 + 1e-5), at least 3 and at most 160 per kept axis, a single cell along a
+// dropped axis (drop_axis 0/1/2, or -1), and no more cells than keep about 2 particles per
+// cell (n_max: the larger group) while every kept axis has more than 3.  Returns the first
+// kept axis on which fewer than 3 cells fit (nc is then incomplete), or -1.
+int rdf_ortho_grid_plan(const double box[3], double r_hi, int64_t n_max, int drop_axis,
+                        int nc[3])
+{
+    const double r_cut = r_hi * 1.00001;
+    double ncell = 1;
+    for (int k = 0; k < 3; ++k) {
+        if (k == drop_axis) {
+            nc[k] = 1;
+            continue;
+        }
+        const double fit = std::floor(box[k] / r_cut);
+        if (!(fit >= 3.0)) return k;
+        nc[k] = (int)std::min(fit, 160.0);
+        ncell *= nc[k];
+    }
+    // keep at least ~2 particles per cell on average
+    const double want = std::max(drop_axis < 0 ? 27.0 : 9.0, (double)n_max / 2.0);
+    while (ncell > want) {
+        int kmax = 0;
+        for (int k = 1; k < 3; ++k) if (nc[k] > nc[kmax]) kmax = k;
+        if (nc[kmax] <= 3) break;
+        ncell = ncell / nc[kmax] * (nc[kmax] - 1);
+        nc[kmax]--;
+    }
+    return -1;
+}
+
 // Device layout of the cell-list scratch (RdfState::cell):
 //   cell[0] CellGrid[F]            cell[1] int cnt[2][G][cstride] | unsigned ext[2][G][6] | work
 //   cell[2] int start[2][G][cstride]   cell[3] int2 keyrank[G][n1]   cell[4] float4 sorted1[G][n1]
@@ -1021,33 +1075,28 @@ int rdf_cells_accumulate(mdh_ctx *c, const float *raw1, int64_t stride1, const f
                          int64_t stride2, int f0, int n_frames, bool use_filter, double sqrt_err)
 {
     RdfState &R = c->rdf;
-    MDH_REQUIRE(R.drop_axis < 0, MDH_EINVAL, "rdf: cell-list mode does not support drop_axis");
     MDH_REQUIRE(R.n1 <= (1ll << 25) && R.n2 <= (1ll << 25), MDH_EINVAL,
                 "rdf: cell-list mode takes at most 2^25 particles per group");
-    const double r_cut = sqrt(R.thr_hi) * 1.00001;
+    // grid axis k <- physical axis: a dropped axis goes last (see CellGrid)
+    static const int kAxes[4][3] = {{0, 1, 2}, {1, 2, 0}, {0, 2, 1}, {0, 1, 2}};
+    const int *axes = kAxes[R.drop_axis + 1];
+    const bool flat = R.drop_axis >= 0;
     std::vector<CellGrid> grids(n_frames);
     int ncell_max = 0;
     for (int f = 0; f < n_frames; ++f) {
         CellGrid &g = grids[f];
-        double ncell = 1;
+        int nc[3];
+        const int short_axis = rdf_ortho_grid_plan(R.h_boxes[f0 + f].box, sqrt(R.thr_hi),
+                                                   std::max(R.n1, R.n2), R.drop_axis, nc);
+        MDH_REQUIRE(short_axis < 0, MDH_EINVAL,
+                    "rdf: cell-list mode needs box edge >= 3*r_max (frame %d axis %d)", f,
+                    short_axis);
         for (int k = 0; k < 3; ++k) {
-            g.box[k] = R.h_boxes[f0 + f].box[k];
-            int nc = (int)floor(g.box[k] / r_cut);
-            MDH_REQUIRE(nc >= 3, MDH_EINVAL,
-                        "rdf: cell-list mode needs box edge >= 3*r_max (frame %d axis %d)", f, k);
-            g.nc[k] = std::min(nc, 160);
-            ncell *= g.nc[k];
+            g.axis[k] = axes[k];
+            g.box[k] = R.h_boxes[f0 + f].box[axes[k]];
+            g.nc[k] = nc[axes[k]];
+            g.inv_w[k] = g.nc[k] / g.box[k];
         }
-        // keep at least ~2 particles per cell on average
-        const double want = std::max(27.0, (double)std::max(R.n1, R.n2) / 2.0);
-        while (ncell > want) {
-            int kmax = 0;
-            for (int k = 1; k < 3; ++k) if (g.nc[k] > g.nc[kmax]) kmax = k;
-            if (g.nc[kmax] <= 3) break;
-            ncell = ncell / g.nc[kmax] * (g.nc[kmax] - 1);
-            g.nc[kmax]--;
-        }
-        for (int k = 0; k < 3; ++k) g.inv_w[k] = g.nc[k] / g.box[k];
         g.ncell = g.nc[0] * g.nc[1] * g.nc[2];
         ncell_max = std::max(ncell_max, g.ncell);
     }
@@ -1092,7 +1141,8 @@ int rdf_cells_accumulate(mdh_ctx *c, const float *raw1, int64_t stride1, const f
 
     // candidates per cell the buffers are sized for: mean + 6 sigma (Poisson) + slack
     const double per_cell1 = (double)R.n1 / ncell_max, per_cell2 = (double)R.n2 / ncell_max;
-    const double expect = per_cell1 + (R.same ? 13.0 : 27.0) * per_cell2;
+    const double expect = per_cell1 + (flat ? (R.same ? 4.0 : 9.0) : (R.same ? 13.0 : 27.0)) *
+                                          per_cell2;
     int cap = (int)(expect + 6.0 * sqrt(expect) + 24.0);
     cap = std::min(1024, std::max(96, (cap + 31) / 32 * 32));
     int sb_c = use_filter ? cellpair_sub_bins(R.n_bins, R.fc.sb, cap) : -1;
@@ -1126,7 +1176,7 @@ int rdf_cells_accumulate(mdh_ctx *c, const float *raw1, int64_t stride1, const f
             cells_bin_kernel<<<grid, 256, 0, c->stream>>>(
                 raw, grp ? stride2 : stride1, n, gg, d_cnt + (size_t)grp * G * cstride, cstride,
                 R.cell[grp ? 7 : 3].as<int2>(), use_filter ? d_ext + (size_t)grp * G * 6 : nullptr,
-                R.boxes.as<FrameBox>() + f0 + g0);
+                R.boxes.as<FrameBox>() + f0 + g0, R.drop_axis);
             MDH_CUDA(cudaGetLastError());
             c->launches++;
         }
@@ -1160,7 +1210,8 @@ int rdf_cells_accumulate(mdh_ctx *c, const float *raw1, int64_t stride1, const f
             cells_scatter_kernel<<<grid, 256, 0, c->stream>>>(
                 raw, grp ? stride2 : stride1, n, grp ? R.excl2 : R.excl1,
                 d_start + (size_t)grp * G * cstride, cstride, R.cell[grp ? 7 : 3].as<int2>(),
-                R.cell[grp ? 8 : 4].as<float4>(), R.boxes.as<FrameBox>() + f0 + g0);
+                R.cell[grp ? 8 : 4].as<float4>(), R.boxes.as<FrameBox>() + f0 + g0,
+                R.drop_axis);
             MDH_CUDA(cudaGetLastError());
             c->launches++;
         }

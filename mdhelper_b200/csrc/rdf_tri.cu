@@ -383,14 +383,18 @@ __global__ void __launch_bounds__(kThreads, 2) rdf_tri_cells_kernel(const TriCel
                 sweep(bw, start[row + xw + 1] - bw, __vadd4(code(wa, wb, wc), kneg), w, w);
             }
         };
+        // one cell along c (drop_axis = 2, tri_grid_plan_flat): the 9 cells (half: 4 + own)
+        // of the (a, b) plane; the c component of every m' is 0
+        const int dz_max = g.nc[2] > 1 ? 1 : 0;
         if (!P.half) {
-            for (int dz = -1; dz <= 1; ++dz)
+            for (int dz = -dz_max; dz <= dz_max; ++dz)
                 for (int dy = -1; dy <= 1; ++dy) sweep_row(dy, dz, 1u);
         } else {
             // forward offsets (dz, dy, dx) > 0 in lexicographic order, weight 2 for both
             // orders ((i, j) and (j, i) have the same 27-image minimum: float rounding is
             // odd-symmetric); the own cell from j = i: the self pair once
-            for (int dy = -1; dy <= 1; ++dy) sweep_row(dy, 1, 2u);
+            if (dz_max)
+                for (int dy = -1; dy <= 1; ++dy) sweep_row(dy, 1, 2u);
             sweep_row(1, 0, 2u);
             const int row = (cz * g.nc[1] + cy) * g.nc[0];
             int wa;
@@ -456,9 +460,10 @@ struct TriPlan {
     int nc[3];        // cells per axis (0: fewer than 3 fit)
     int fit[3];       // cells per axis before the cap and the occupancy rule
     double margin;    // M
+    bool c_ok;        // flat grid (tri_grid_plan_flat): c_z >= r + M
 };
 
-int tri_grid_plan(const float *m9, double r_hi, int64_t n_max, TriPlan &out)
+int tri_check_matrix(const float *m9, double r_hi)
 {
     MDH_REQUIRE(m9 != nullptr, MDH_EINVAL, "rdf: cell matrix is NULL");
     MDH_REQUIRE(m9[1] == 0.f && m9[2] == 0.f && m9[5] == 0.f, MDH_EINVAL,
@@ -468,6 +473,42 @@ int tri_grid_plan(const float *m9, double r_hi, int64_t n_max, TriPlan &out)
     MDH_REQUIRE(m9[0] > 0.f && m9[4] > 0.f && m9[8] > 0.f, MDH_EINVAL,
                 "rdf: the cell matrix is not a valid cell");
     MDH_REQUIRE(r_hi >= 0.0 && std::isfinite(r_hi), MDH_EINVAL, "rdf: invalid r_max");
+    return MDH_OK;
+}
+
+// cells per axis from the (lower bounds of the) widths w: w_k / n_k >= width exactly, at
+// most 160, then fewer until about 2 particles per cell remain or the axes are down to 3;
+// `axes` axes are cut (3, or 2 with one cell along c)
+void tri_cells_per_axis(const double *w, double width, int64_t n_max, int axes, TriPlan &out)
+{
+    double ncell = 1;
+    for (int k = 0; k < axes; ++k) {
+        double f = std::floor(w[k] / width);
+        while (f >= 1.0 && w[k] / f < width) f -= 1.0;     // w_k / n_k >= r + M exactly
+        out.fit[k] = (int)std::min(f, 1e6);
+        out.nc[k] = std::min(out.fit[k], 160);
+        ncell *= out.nc[k];
+    }
+    for (int k = axes; k < 3; ++k) out.fit[k] = out.nc[k] = 1;
+    if (std::min({out.nc[0], out.nc[1], axes == 3 ? out.nc[2] : 3}) < 3) {
+        for (int k = 0; k < 3; ++k) out.nc[k] = 0;
+        return;
+    }
+    // keep at least ~2 particles per cell on average
+    const double want = std::max(axes == 3 ? 27.0 : 9.0, (double)n_max / 2.0);
+    while (ncell > want) {
+        int kmax = 0;
+        for (int k = 1; k < axes; ++k) if (out.nc[k] > out.nc[kmax]) kmax = k;
+        if (out.nc[kmax] <= 3) break;
+        ncell = ncell / out.nc[kmax] * (out.nc[kmax] - 1);
+        out.nc[kmax]--;
+    }
+}
+
+int tri_grid_plan(const float *m9, double r_hi, int64_t n_max, TriPlan &out)
+{
+    if (int rc = tri_check_matrix(m9, r_hi)) return rc;
+    out.c_ok = true;
     const double ax = m9[0], bx = m9[3], by = m9[4], cx = m9[6], cy = m9[7], cz = m9[8];
     const double u = 1.0 / 9007199254740992.0;           // 2^-53
     // magnitude bounds (B) and absolute errors (e) of the steps of tri_cell
@@ -499,27 +540,67 @@ int tri_grid_plan(const float *m9, double r_hi, int64_t n_max, TriPlan &out)
     const double width = r_hi + out.margin;
     bool shifts_ok = true;
     for (int k = 0; k < 3; ++k) shifts_ok = shifts_ok && B[k] + 1.0 <= kTriShiftMax;
-    double ncell = 1;
-    for (int k = 0; k < 3; ++k) {
-        double f = std::floor(w[k] / width);
-        while (f >= 1.0 && w[k] / f < width) f -= 1.0;     // w_k / n_k >= r + M exactly
-        out.fit[k] = (int)std::min(f, 1e6);
-        out.nc[k] = std::min(out.fit[k], 160);
-        ncell *= out.nc[k];
-    }
-    if (!shifts_ok || std::min({out.nc[0], out.nc[1], out.nc[2]}) < 3) {
+    tri_cells_per_axis(w, width, n_max, 3, out);
+    if (!shifts_ok)
         for (int k = 0; k < 3; ++k) out.nc[k] = 0;
-        return MDH_OK;
-    }
-    // keep at least ~2 particles per cell on average
-    const double want = std::max(27.0, (double)n_max / 2.0);
-    while (ncell > want) {
-        int kmax = 0;
-        for (int k = 1; k < 3; ++k) if (out.nc[k] > out.nc[kmax]) kmax = k;
-        if (out.nc[kmax] <= 3) break;
-        ncell = ncell / out.nc[kmax] * (out.nc[kmax] - 1);
-        out.nc[kmax]--;
-    }
+    return MDH_OK;
+}
+
+// ---- the flat grid of drop_axis = 2 ------------------------------------------------------
+//
+// The zeroed z stays exactly 0 through tri_wrap_kernel (s = floor(0 / c_z) = 0, and the a
+// and b rows have no z component), so every wrapped particle lies in the plane z = 0, has
+// s_c = 0 exactly in tri_cell and the shift k_c = 0.  The grid has one cell along c and the
+// stencil is the 9 cells of the (a, b) plane, so every m' has m'_c = 0.
+//
+// Images with a c shift iz != 0.  dx_2 = (float)(0 - 0) = 0, so the reference's
+// r_z = dx_2 + c_z iz = +-c_z exactly, c_z^2 is exact in fp64 (24-bit x 24-bit), and the
+// computed d^2 = fl(fl(r_x^2 + r_y^2) + c_z^2) >= c_z^2 (rounding is monotone, the other
+// terms are >= 0).  With c_z >= r + M > r such an image is above U: never counted, and
+// never the 27-image minimum when that is in range.
+//
+// Images with iz = 0.  These and p_i all lie in the plane, so the argument of tri_grid_plan
+// holds in two dimensions with the in-plane widths of the (a, b) lattice, w_a = a_x b_y / |b|
+// and w_b = b_y (at least the three-dimensional perpendicular widths): per axis a, b the
+// 3 x 3 block of cells around p_i's cell spans less than one period (n_k >= 3), every image
+// but m' differs from p_i in s_a or s_b by at least 1 / n_k - 2 eps_k, i.e. lies at least
+// r + M - 2 eps_k w_k away.  The terms of M, for z = 0 and (not "far") x in
+// [-a_x / 2, 3 a_x / 2], y in [-b_y / 2, 3 b_y / 2]:
+//   eps_b, eps_a   tri_cell with s_c = 0 exactly: s_b = y / b_y (one rounding) and
+//                  s_a = (x - s_b b_x) / a_x (the term s_c c_x is 0, exact); each rounding
+//                  2^-53 of the bound on its result, doubled, plus 2^-53 for the
+//                  fractional part and the product with n_k (as tri_grid_plan);
+//   e_f            2^-24 |dx| with |dx_k| <= 2 E_k, E = (a_x, b_y): 2^-23 |E| (dx_2 = 0);
+//   e_d            the image sums (dx_0 + a_x ia) + b_x ib (+ 0, exact) and dx_1 + b_y ib:
+//                  4 * 2^-53 |(3 a_x + |b_x|, 3 b_y)|;
+//   1e-5 r         fp64 squares and sums of d^2, as tri_grid_plan.
+// M = max(2 eps_a w_a, 2 eps_b w_b) + e_f + e_d + 1e-5 r; cells of width >= r + M per kept
+// axis, and c_ok = (c_z >= r + M).  (c_z > r alone would do by the argument above; the plan
+// asks the same width of all three axes.)  drop_axis 0 or 1 gets no grid: the wrap then
+// moves the zeroed coordinate again, and the particles do not lie in a lattice plane.
+int tri_grid_plan_flat(const float *m9, double r_hi, int64_t n_max, TriPlan &out)
+{
+    if (int rc = tri_check_matrix(m9, r_hi)) return rc;
+    const double ax = m9[0], bx = m9[3], by = m9[4], cz = m9[8];
+    const double u = 1.0 / 9007199254740992.0;           // 2^-53
+    const double X = 1.5 * ax, Y = 1.5 * by;
+    const double Bb = Y / by * (1 + u), eb = u * Bb;                     // s_b = y / b_y
+    const double Bq1 = Bb * std::fabs(bx) * (1 + u), eq1 = std::fabs(bx) * eb + u * Bq1;
+    const double Br1 = (X + Bq1) * (1 + u), er1 = eq1 + u * Br1;         // x - s_b b_x
+    const double Ba = Br1 / ax * (1 + u), ea = er1 / ax + u * Ba;        // s_a
+    const double eps[2] = {2 * ea + u, 2 * eb + u};
+    const double B[2] = {Ba, Bb};
+    const double w[2] = {ax * by / std::sqrt(bx * bx + by * by) * (1 - 1e-12), by};
+    const double e_f = 2.0 * std::sqrt(ax * ax + by * by) / 16777216.0;
+    const double rx = 3 * ax + std::fabs(bx), ry = 3 * by;
+    const double e_d = 4 * u * std::sqrt(rx * rx + ry * ry);
+    const double e_a = std::max(2.0 * eps[0] * w[0], 2.0 * eps[1] * w[1]);
+    out.margin = e_a + e_f + e_d + 1e-5 * r_hi;
+    const double width = r_hi + out.margin;
+    out.c_ok = cz >= width;
+    tri_cells_per_axis(w, width, n_max, 2, out);
+    if (!(B[0] + 1.0 <= kTriShiftMax && B[1] + 1.0 <= kTriShiftMax))
+        for (int k = 0; k < 3; ++k) out.nc[k] = 0;
     return MDH_OK;
 }
 
@@ -531,6 +612,39 @@ int rdf_triclinic_grid_impl(const float *cell9, double r_hi, int64_t n_max, int3
     MDH_REQUIRE(nc != nullptr && margin != nullptr, MDH_EINVAL, "triclinic_grid: NULL output");
     TriPlan pl;
     if (int rc = tri_grid_plan(cell9, r_hi, n_max, pl)) return rc;
+    for (int k = 0; k < 3; ++k) nc[k] = pl.nc[k];
+    *margin = pl.margin;
+    return MDH_OK;
+}
+
+int rdf_ortho_grid_plan(const double box[3], double r_hi, int64_t n_max, int drop_axis,
+                        int nc[3]);                           // rdf_cells.cu
+
+int rdf_cells_grid_impl(const float *cell9, double r_hi, int64_t n_max, int drop_axis,
+                        int32_t *nc, double *margin)
+{
+    MDH_REQUIRE(nc != nullptr && margin != nullptr, MDH_EINVAL, "cells_grid: NULL output");
+    MDH_REQUIRE(drop_axis >= -1 && drop_axis <= 2, MDH_EINVAL, "rdf: invalid drop_axis");
+    if (int rc = tri_check_matrix(cell9, r_hi)) return rc;
+    if (cell9[3] == 0.f && cell9[6] == 0.f && cell9[7] == 0.f) {
+        // orthorhombic: the grid of mdh_rdf_accumulate (rdf_cells_accumulate)
+        const double box[3] = {cell9[0], cell9[4], cell9[8]};
+        int g[3];
+        const bool ok = rdf_ortho_grid_plan(box, r_hi, n_max, drop_axis, g) < 0;
+        for (int k = 0; k < 3; ++k) nc[k] = ok ? g[k] : 0;
+        *margin = r_hi * 1.00001 - r_hi;
+        return MDH_OK;
+    }
+    MDH_REQUIRE(drop_axis < 0 || drop_axis == 2, MDH_EINVAL,
+                "rdf: the triclinic cell list takes drop_axis 2 (z) only; drop_axis %d runs "
+                "through all pairs", drop_axis);
+    TriPlan pl;
+    if (int rc = drop_axis == 2 ? tri_grid_plan_flat(cell9, r_hi, n_max, pl)
+                                : tri_grid_plan(cell9, r_hi, n_max, pl))
+        return rc;
+    MDH_REQUIRE(pl.c_ok, MDH_EINVAL,
+                "rdf: the triclinic cell list with drop_axis 2 needs c_z >= r_max + %g "
+                "(c_z = %g)", pl.margin, (double)cell9[8]);
     for (int k = 0; k < 3; ++k) nc[k] = pl.nc[k];
     *margin = pl.margin;
     return MDH_OK;
@@ -654,7 +768,6 @@ int rdf_accumulate_triclinic_impl(mdh_ctx *c, const float *pos1, int64_t s1, con
                 "rdf: coordinate pointer is NULL");
     MDH_REQUIRE(s1 >= 3 * R.n1 && (R.same || s2 >= 3 * R.n2), MDH_EINVAL,
                 "rdf: frame_stride < 3*n");
-    MDH_REQUIRE(R.drop_axis < 0, MDH_EINVAL, "rdf: drop_axis needs an orthorhombic cell");
     const size_t smem = align16(sizeof(double) * (R.n_bins + 1)) + 256 * sizeof(float4) +
                         sizeof(unsigned) * kWarps * (size_t)R.n_bins;
 
@@ -673,26 +786,40 @@ int rdf_accumulate_triclinic_impl(mdh_ctx *c, const float *pos1, int64_t s1, con
     // pair kernel: the cell list when asked for, or (auto) when every frame holds at least
     // 4 cells per axis and there are enough pairs -- the orthorhombic rule, applied to the
     // perpendicular widths
+    // (with drop_axis = 2: the flat grid of tri_grid_plan_flat, 4 cells per kept width and
+    // c_z >= r + M; drop_axis 0 or 1 has no cell list)
     int mode = R.mode;
     std::vector<TriGrid> grids;
+    if (mode == MDH_RDF_CELLS)
+        MDH_REQUIRE(R.drop_axis < 0 || R.drop_axis == 2, MDH_EINVAL,
+                    "rdf: the triclinic cell list takes drop_axis 2 (z) only; use mode "
+                    "\"allpairs\" or \"auto\" for drop_axis %d", R.drop_axis);
+    if (mode == MDH_RDF_AUTO && R.drop_axis >= 0 && R.drop_axis != 2) mode = MDH_RDF_ALLPAIRS;
     if (mode != MDH_RDF_ALLPAIRS) {
         const double r_hi = sqrt(R.thr_hi);
+        const bool flat = R.drop_axis == 2;
         bool fit4 = tri_cells_smem_bytes(R.n_bins) <= kMaxSmem && R.n1 <= (1ll << 25) &&
                     R.n2 <= (1ll << 25);
         grids.resize(n_frames);
         for (int f = 0; f < n_frames && (mode == MDH_RDF_CELLS || fit4); ++f) {
             TriPlan pl;
-            if (int rc = tri_grid_plan(box9 + 9 * f, r_hi, std::max(R.n1, R.n2), pl)) {
+            if (int rc = flat ? tri_grid_plan_flat(box9 + 9 * f, r_hi, std::max(R.n1, R.n2), pl)
+                              : tri_grid_plan(box9 + 9 * f, r_hi, std::max(R.n1, R.n2), pl)) {
                 if (mode == MDH_RDF_CELLS) return rc;
                 fit4 = false;                 // (auto) e.g. a non-finite tilt: all pairs
                 break;
             }
-            if (mode == MDH_RDF_CELLS)
+            if (mode == MDH_RDF_CELLS) {
                 MDH_REQUIRE(pl.nc[0] >= 3, MDH_EINVAL,
                             "rdf: cell-list mode needs every perpendicular width of the cell >= "
                             "3*(r_max + %g) (frame %d: %d, %d, %d cells fit)", pl.margin, f,
                             pl.fit[0], pl.fit[1], pl.fit[2]);
-            fit4 = fit4 && pl.nc[0] >= 3 && std::min({pl.fit[0], pl.fit[1], pl.fit[2]}) >= 4;
+                MDH_REQUIRE(pl.c_ok, MDH_EINVAL,
+                            "rdf: cell-list mode with drop_axis 2 needs c_z >= r_max + %g "
+                            "(frame %d: c_z = %g)", pl.margin, f, (double)box9[9 * f + 8]);
+            }
+            fit4 = fit4 && pl.nc[0] >= 3 && pl.c_ok &&
+                   std::min({pl.fit[0], pl.fit[1], flat ? 4 : pl.fit[2]}) >= 4;
             grids[f].h = hb[f];
             for (int k = 0; k < 3; ++k) grids[f].nc[k] = pl.nc[k];
             grids[f].ncell = pl.nc[0] * pl.nc[1] * pl.nc[2];
@@ -737,8 +864,11 @@ int rdf_accumulate_triclinic_impl(mdh_ctx *c, const float *pos1, int64_t s1, con
         }
         if (int rc = pk.reserve(sizeof(float4) * npad * n_frames)) return rc;
         dim3 grid((unsigned)std::min<int64_t>((npad + 255) / 256, 2048), n_frames);
+        // a dropped coordinate is zeroed here; the wrap below may move it again (drop_axis 0
+        // or 1 on a tilted cell), as the reference's wrap does
         rdf_pack_kernel<<<grid, 256, 0, c->stream>>>(dsrc, dstride, pk.as<float4>(), n, npad,
-                                                     g ? R.excl2 : R.excl1, -1, nullptr, nullptr);
+                                                     g ? R.excl2 : R.excl1, R.drop_axis, nullptr,
+                                                     nullptr);
         MDH_CUDA(cudaGetLastError());
         tri_wrap_kernel<<<grid, 256, 0, c->stream>>>(pk.as<float4>(), npad, (int)n,
                                                      d_box.as<TriBox>());
