@@ -238,6 +238,10 @@ int mdh_rdf_set_prewrap(mdh_ctx *ctx, int mode);
  * declined (left to the exact kernel), stats[5] 1 if the current configuration is
  * eligible for the filter.  Since the last configure / reset. */
 int mdh_rdf_filter_stats(mdh_ctx *ctx, int64_t *stats /* [6] host */);
+/* frames[0] frames the all-pairs filter kernel evaluated with the half-box minimum image
+ * (every coordinate difference within 1.5 box lengths), frames[1] frames it evaluated
+ * with the rint form.  Since the last configure / reset. */
+int mdh_rdf_filter_modes(mdh_ctx *ctx, int64_t *frames /* [2] host */);
 
 /* ---- seam #2: direct-sum structure factor ------------------------------------ */
 

@@ -56,6 +56,7 @@ SIGNATURES = {
     "mdh_rdf_set_filter": (_i32, [_p, _i32]),
     "mdh_rdf_set_prewrap": (_i32, [_p, _i32]),
     "mdh_rdf_filter_stats": (_i32, [_p, _p]),
+    "mdh_rdf_filter_modes": (_i32, [_p, _p]),
     "mdh_sq_configure": (_i32, [_p, _i64, _i32, _p, _i32, _p, _p, _p, _i32, _p, _i32]),
     "mdh_sq_accumulate": (_i32, [_p, _p, _i64, _i32, _i32]),
     "mdh_sq_accumulate_f64": (_i32, [_p, _p, _i64, _i32, _i32]),
@@ -290,10 +291,12 @@ class Context:
         check(self._lib.mdh_rdf_set_prewrap(self._h, WRAP_MODES[mode]))
 
     def rdf_filter_stats(self) -> dict:
-        out = np.zeros(6, dtype=np.int64)
-        check(self._lib.mdh_rdf_filter_stats(self._h, out.ctypes.data))
+        out = np.zeros(8, dtype=np.int64)
+        check(self._lib.mdh_rdf_filter_stats(self._h, out[:6].ctypes.data))
+        check(self._lib.mdh_rdf_filter_modes(self._h, out[6:].ctypes.data))
         return dict(zip(("deferred_entries", "inline_entries", "audit_violations",
-                         "audit_uncertain_pairs", "declined_frames", "eligible"),
+                         "audit_uncertain_pairs", "declined_frames", "eligible",
+                         "halfbox_frames", "rint_frames"),
                         (int(v) for v in out)))
 
     def rdf_pair_evaluations(self) -> int:

@@ -422,6 +422,19 @@ int mdh_rdf_filter_stats(mdh_ctx *c, int64_t *stats)
     return MDH_OK;
 }
 
+int mdh_rdf_filter_modes(mdh_ctx *c, int64_t *frames)
+{
+    CTX_GUARD(c);
+    MDH_REQUIRE(frames != nullptr, MDH_EINVAL, "frames is NULL");
+    MDH_REQUIRE(c->rdf.configured, MDH_ESTATE, "rdf: not configured");
+    unsigned long long h[8] = {0};
+    MDH_CUDA(cudaMemcpyAsync(h, c->rdf.fstats.p, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
+    MDH_CUDA(cudaStreamSynchronize(c->stream));
+    frames[0] = (int64_t)h[5];
+    frames[1] = (int64_t)h[6];
+    return MDH_OK;
+}
+
 /* ---- seam #2 ---- */
 
 int mdh_sq_configure(mdh_ctx *c, int64_t n_total, int n_groups, const int64_t *group_offsets,

@@ -73,6 +73,9 @@ struct FrameFilter {
                            // the uncertainty window is [0, 2m] in its fraction bits
     unsigned wlim;         // pair is uncertain iff (bits & (2^k - 1)) < wlim = 2m + 1;
                            // 0 = frame not eligible (the exact kernel handles it)
+    float nhalf[3];        // -box_k / 2
+    int halfbox;           // 1: the all-pairs kernel takes the half-box minimum image
+                           // (every |df_k| <= 1.5 box_k; offm / wlim are from its bound)
 };
 
 struct FilterConst {       // per configuration (host)
@@ -119,7 +122,7 @@ struct RdfState {
     FilterConst fc;
     DevBuf ext1, ext2;     // unsigned[F][6]: coordinate extents of each frame (keys)
     DevBuf filt;           // FrameFilter[F]
-    DevBuf fstats;         // unsigned long long[4], see PairParams::fstats
+    DevBuf fstats;         // unsigned long long[8], see PairParams::fstats
 };
 
 struct SqWorkItem {        // one thread's tile of the lattice kernels: two (nx, ny)

@@ -360,6 +360,13 @@ __device__ __forceinline__ f32x2 fma2(f32x2 a, f32x2 b, f32x2 c)
     return d;
 }
 
+__device__ __forceinline__ f32x2 abs2(f32x2 v)
+{
+    float lo, hi;
+    upk2(v, lo, hi);
+    return pk2(fabsf(lo), fabsf(hi));     // ptxas folds this into the |x| operand of FADD2
+}
+
 // The fp32 evaluation of TWO pairs at once: coordinate differences d = b + a per axis
 // with a = the NEGATED coordinates of the group-1 particle(s) and b = the group-2
 // particle(s) -- the all-pairs kernel packs two group-1 particles against one tile row
@@ -367,20 +374,35 @@ __device__ __forceinline__ f32x2 fma2(f32x2 a, f32x2 b, f32x2 c)
 // neighbours.  Returns the fixed-point bin coordinates u0, u1 (relative to slot 0 when
 // LOWER, else with the bits of 1.5*2^(23-k) still added).  Main loops and exact
 // re-evaluations go through this one function, so they see identical bits.
-// first half: packed squared minimum-image distances of two pairs
+// first half: packed squared minimum-image distances of two pairs.  Two forms of the
+// minimum image (FrameFilter::halfbox; the error bound of each: filter_prepare_frame):
+//   HALF = false  m = fma(-box, rint(df * inv), df)        4 packed instructions per axis
+//   HALF = true   m = ||df| - box/2| - box/2               2 packed instructions per axis,
+//                 |m| is the minimum image for |df| <= 1.5 box (only |m| matters for m^2)
+template <bool HALF>
 __device__ __forceinline__ f32x2 filter_d2(f32x2 ax, f32x2 ay, f32x2 az, f32x2 bx, f32x2 by,
                                            f32x2 bz, const FrameFilter &ff)
 {
-    const f32x2 magic = pk2(kMagicF, kMagicF), nmagic = pk2(-kMagicF, -kMagicF);
     const f32x2 dx = add2(bx, ax);
     const f32x2 dy = add2(by, ay);
     const f32x2 dz = add2(bz, az);
-    const f32x2 rx = add2(fma2(dx, pk2(ff.inv[0], ff.inv[0]), magic), nmagic);
-    const f32x2 ry = add2(fma2(dy, pk2(ff.inv[1], ff.inv[1]), magic), nmagic);
-    const f32x2 rz = add2(fma2(dz, pk2(ff.inv[2], ff.inv[2]), magic), nmagic);
-    const f32x2 mx = fma2(pk2(ff.nbox[0], ff.nbox[0]), rx, dx);
-    const f32x2 my = fma2(pk2(ff.nbox[1], ff.nbox[1]), ry, dy);
-    const f32x2 mz = fma2(pk2(ff.nbox[2], ff.nbox[2]), rz, dz);
+    f32x2 mx, my, mz;
+    if (HALF) {
+        const f32x2 hx = pk2(ff.nhalf[0], ff.nhalf[0]);
+        const f32x2 hy = pk2(ff.nhalf[1], ff.nhalf[1]);
+        const f32x2 hz = pk2(ff.nhalf[2], ff.nhalf[2]);
+        mx = add2(abs2(add2(abs2(dx), hx)), hx);
+        my = add2(abs2(add2(abs2(dy), hy)), hy);
+        mz = add2(abs2(add2(abs2(dz), hz)), hz);
+    } else {
+        const f32x2 magic = pk2(kMagicF, kMagicF), nmagic = pk2(-kMagicF, -kMagicF);
+        const f32x2 rx = add2(fma2(dx, pk2(ff.inv[0], ff.inv[0]), magic), nmagic);
+        const f32x2 ry = add2(fma2(dy, pk2(ff.inv[1], ff.inv[1]), magic), nmagic);
+        const f32x2 rz = add2(fma2(dz, pk2(ff.inv[2], ff.inv[2]), magic), nmagic);
+        mx = fma2(pk2(ff.nbox[0], ff.nbox[0]), rx, dx);
+        my = fma2(pk2(ff.nbox[1], ff.nbox[1]), ry, dy);
+        mz = fma2(pk2(ff.nbox[2], ff.nbox[2]), rz, dz);
+    }
     return fma2(mz, mz, fma2(my, my, mul2(mx, mx)));
 }
 
@@ -399,13 +421,13 @@ __device__ __forceinline__ void filter_bin2(f32x2 d2, float scale, float offm, u
     u1 = __float_as_uint(b) - (LOWER ? cbits : 0u);
 }
 
-template <bool LOWER>
+template <bool LOWER, bool HALF = false>
 __device__ __forceinline__ void filter_eval2(f32x2 ax, f32x2 ay, f32x2 az, f32x2 bx, f32x2 by,
                                              f32x2 bz, const FrameFilter &ff, float scale,
                                              float offm, unsigned cbits, unsigned &u0,
                                              unsigned &u1)
 {
-    filter_bin2<LOWER>(filter_d2(ax, ay, az, bx, by, bz, ff), scale, offm, cbits, u0, u1);
+    filter_bin2<LOWER>(filter_d2<HALF>(ax, ay, az, bx, by, bz, ff), scale, offm, cbits, u0, u1);
 }
 
 // Per-frame parameters of the fp32 filter from the frame's box and coordinate extents
@@ -413,6 +435,8 @@ __device__ __forceinline__ void filter_eval2(f32x2 ax, f32x2 ay, f32x2 az, f32x2
 // {min x, y, z, max x, y, z} of the two groups.
 struct FilterPrep {            // per configuration (host)
     int k;
+    int halfbox;               // frames may take the half-box minimum image (all-pairs
+                               // kernel; the cell-list kernels evaluate the rint form only)
     double scale;              // n_bins / (r_hi - r_lo)
     double d_max;              // largest distance that can still be binned
     double sqrt_err;           // measured relative error of sqrt.approx.ftz.f32
@@ -423,8 +447,8 @@ __device__ inline FrameFilter filter_prepare_frame(const FrameBox &fb, const uns
                                                    const unsigned *e2, const FilterPrep &Q)
 {
     const double e24 = 1.0 / 16777216.0;
-    bool ok = true;
-    double a2 = 0.0;
+    bool ok = true, half = Q.halfbox != 0;
+    double a2 = 0.0, h2 = 0.0;
     FrameFilter ff;
     for (int k = 0; k < 3; ++k) {
         const float e4[4] = {ext_unkey(e1[k]), ext_unkey(e1[3 + k]), ext_unkey(e2[k]),
@@ -434,20 +458,33 @@ __device__ inline FrameFilter filter_prepare_frame(const FrameBox &fb, const uns
             if ((__float_as_uint(e4[q]) & 0x7f800000u) == 0x7f800000u) ok = false;
         const double lo1 = (double)e4[0], hi1 = (double)e4[1];
         const double lo2 = (double)e4[2], hi2 = (double)e4[3];
+        // D >= every |df| of the frame, the float32 rounding of df included
         const double D = fmax(fmax(hi2 - lo1, hi1 - lo2), 0.0) * (1.0 + 2.0 * e24);
         const double box = fb.box[k], inv = fb.inv[k];
         // the magic-number rounding needs |df * inv| well inside 2^22
         if (!(D * inv < 1048576.0)) ok = false;
         const double eps_b = fabs(box * inv - 1.0);       // exact: 24-bit x 24-bit
-        // last term: the fp64 product inv*df of the reference may round across a
+        // first term: the fp32 rounding of the minimum image; then the reference vs the
+        // exact minimum image of df: eps_b * D from its float32 inverse box, D * 2^-51
+        // from its fp64 roundings -- the product inv*df may also round across a
         // half-integer that the exact product does not cross (|m| changes by at most
         // box * 2^-52 * |inv*df| <= 2^-51 D)
+        // rint form: one rounding of fma(-box, r, df), |m_f| <= box/2 + eps_b D + 2^-24 D
         const double a = e24 * (0.5 * box + eps_b * D + e24 * D) * (1.0 + 1e-6) + eps_b * D +
                          D / 2251799813685248.0 + 1e-30;
         a2 += a * a;
+        // half-box form, |df| <= D <= 1.5 box: e = |df| - h, m = |e| - h with h = box/2.
+        // By Sterbenz at most one of the two rounds, and the rounded result lies in
+        // [h/2, h] (|df| < h/2: e; h/2 <= |df| <= box: m) or in [h, 2h] (|df| > box: e).
+        if (!(D <= 1.5 * box)) half = false;
+        const double ah = e24 * (D <= box ? 0.5 * box : box) * (1.0 + 1e-6) + eps_b * D +
+                          D / 2251799813685248.0 + 1e-30;
+        h2 += ah * ah;
         ff.nbox[k] = -(float)box;                          // box is a float32 value
         ff.inv[k] = (float)inv;
+        ff.nhalf[k] = -0.5f * (float)box;                  // exact
     }
+    if (half) a2 = h2;
     const double two_k = (double)(1u << Q.k);
     const double mu = Q.scale * (sqrt(a2) + Q.d_max * (1.5 * e24 * 1.001 + Q.sqrt_err)) +
                       e24 * Q.scale * Q.d_max * 1.001 + 1.0 / two_k + 1e-9;
@@ -461,6 +498,7 @@ __device__ inline FrameFilter filter_prepare_frame(const FrameBox &fb, const uns
         ff.offm = 0.f;
         ff.wlim = 0u;
     }
+    ff.halfbox = ok && half ? 1 : 0;
     return ff;
 }
 
@@ -499,7 +537,8 @@ struct PairParams {
     int fast_bins;                 // slot_fast certified (used by the exact re-evaluation)
     unsigned long long *fstats;    // [0] deferred entries, [1] inline fixes, [2] audit
                                    // violations, [3] audited uncertain pairs, [4] frames
-                                   // declined by the filter
+                                   // declined by the filter, [5] / [6] frames the all-pairs
+                                   // filter evaluated in the half-box / rint form
 };
 
 }  // namespace rdfdev

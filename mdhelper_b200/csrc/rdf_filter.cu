@@ -5,13 +5,18 @@
 // only when a rigorous error bound proves that the reference's fp64 distance falls in
 // the same bin; every other pair ("uncertain": within the bound of a bin edge, about
 // 1 in 1,500 for the benchmark configurations) is re-evaluated with the exact
-// arithmetic of rdf_device.cuh::pair_d2 and corrected.  The fp32 path costs ~16
-// issue slots per pair (8 packed f32x2 instructions on the FMA pipe, ~5 on the ALU
-// pipe, one MUFU, one RED) instead of 21 FP64-pipe instructions plus conversions (46
+// arithmetic of rdf_device.cuh::pair_d2 and corrected.  The fp32 path costs ~15
+// issue slots per pair (6.5 packed f32x2 instructions on the FMA pipe in the half-box
+// form, 8 in the rint form, ~5 on the ALU pipe, one MUFU, one RED) instead of 21 FP64-pipe instructions plus conversions (46
 // in total) -- it removes the FP64 pipe as the bound.
 //
-// fp32 evaluation (rdf_device.cuh::filter_eval2, two pairs per instruction), per axis:
+// fp32 evaluation (rdf_device.cuh::filter_eval2, two pairs per instruction), per axis
+// one of two forms of the minimum image, chosen per frame (FrameFilter::halfbox):
 //     df = xj - xi                      the reference's own float32 difference (exact copy)
+//   half-box form, when every |df| of the frame is <= 1.5 box (h = box/2, exact):
+//     e  = |df| - h                     FADD2 with an |x| operand
+//     m  = |e| - h                      FADD2; |m| is the minimum-image distance
+//   rint form, all other frames (unwrapped trajectories):
 //     t  = fma(df, inv, 1.5*2^23)       -> 1.5*2^23 + rint(df * inv), one rounding
 //     r  = t - 1.5*2^23                 exact
 //     m  = fma(-box, r, df)             minimum image, one rounding
@@ -27,6 +32,8 @@
 // float32 inverse box makes its minimum image differ from df - box*r by eps_b*df),
 // D_k the largest |df| of the frame (coordinate extents from the pack kernel):
 //     | |m_f| - |m_ref| |  <=  a_k = 2^-24 (box_k/2 + eps_b D_k + 2^-24 D_k) + eps_b D_k
+//                                (half-box form: 2^-24 box_k/2 when D_k <= box_k, else
+//                                 2^-23 box_k/2, + eps_b D_k; at most one FADD rounds)
 //     | |m_f|_2 - d_ref |  <=  |a|_2                          (reverse triangle inequality)
 //     fp32 sum of squares: relative 3*2^-24 on d2 -> 1.5*2^-24 on d
 //     sqrt.approx: relative error measured exhaustively at start-up (<= 2^-22 required)
@@ -67,7 +74,7 @@ __host__ __device__ inline size_t filter_smem_bytes(int n_bins, int cb)
 // Exact re-evaluation of the IPT pairs behind one deferred entry (thread te of the
 // block, tile row jj): every pair the main loop saw as uncertain has been added to
 // the slot the fp32 arithmetic suggested; move it if the fp64 arithmetic disagrees.
-template <bool EXCL, bool LOWER, int IPT>
+template <bool EXCL, bool LOWER, int IPT, bool HALF>
 __device__ __noinline__ void filter_fix(const PairParams &P, int frame, int it, unsigned entry,
                                         const float4 *tile, const double *sT, unsigned hist32,
                                         unsigned weight)
@@ -86,7 +93,7 @@ __device__ __noinline__ void filter_fix(const PairParams &P, int frame, int it, 
         const int i0 = it * TILE + ip * kThreads + te, i1 = i0 + kThreads;
         const float4 a0 = f1[min(i0, P.n1 - 1)], a1 = f1[min(i1, P.n1 - 1)];
         unsigned uu[2];
-        filter_eval2<LOWER>(pk2(-a0.x, -a1.x), pk2(-a0.y, -a1.y), pk2(-a0.z, -a1.z),
+        filter_eval2<LOWER, HALF>(pk2(-a0.x, -a1.x), pk2(-a0.y, -a1.y), pk2(-a0.z, -a1.z),
                             pk2(pj.x, pj.x), pk2(pj.y, pj.y), pk2(pj.z, pj.z), ff, fc.scale,
                             ff.offm, fc.cbits, uu[0], uu[1]);
         for (int h = 0; h < 2; ++h) {
@@ -111,17 +118,12 @@ __device__ __noinline__ void filter_fix(const PairParams &P, int frame, int it, 
     }
 }
 
-template <bool EXCL, bool LOWER, bool AUDIT, int IPT, int OCC>
-__global__ void __launch_bounds__(kThreads, OCC)
-    rdf_filter_kernel(const __grid_constant__ PairParams P)
+// One block of rdf_filter_kernel with the frame's form of the minimum image.
+template <bool EXCL, bool LOWER, bool AUDIT, int IPT, bool HALF>
+__device__ __forceinline__ void filter_block(const PairParams &P, const FrameFilter &ff)
 {
     constexpr int TILE = kThreads * IPT;
     const int frame = blockIdx.y;
-    const FrameFilter ff = P.filt[frame];
-    if (ff.wlim == 0u) {                  // left to the exact kernel (whole block)
-        if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&P.fstats[4], 1ull);
-        return;
-    }
 
     extern __shared__ __align__(16) unsigned char smem[];
     const int n_bins = P.n_bins;
@@ -229,7 +231,7 @@ __global__ void __launch_bounds__(kThreads, OCC)
             for (int r = 0; r < NR; ++r)
 #pragma unroll
                 for (int ip = 0; ip < IPT / 2; ++ip)
-                    dd[r][ip] = filter_d2(nx[ip], ny[ip], nz[ip], pk2(pj[r].x, pj[r].x),
+                    dd[r][ip] = filter_d2<HALF>(nx[ip], ny[ip], nz[ip], pk2(pj[r].x, pj[r].x),
                                           pk2(pj[r].y, pj[r].y), pk2(pj[r].z, pj[r].z), ff);
         };
         // Stage A2: square roots (MUFU) and fixed-point bin coordinates.
@@ -291,7 +293,7 @@ __global__ void __launch_bounds__(kThreads, OCC)
                         const unsigned idx = atomicAdd(sCount, 1u);
                         if (idx < (unsigned)kListCap) sList[idx] = entry;
                         else
-                            filter_fix<EXCL, LOWER, IPT>(P, frame, it, entry, tile, sT, hist32,
+                            filter_fix<EXCL, LOWER, IPT, HALF>(P, frame, it, entry, tile, sT, hist32,
                                                          weight);
                     }
                 }
@@ -363,7 +365,7 @@ __global__ void __launch_bounds__(kThreads, OCC)
         const unsigned n_push = *sCount;
         const unsigned n_list = min(n_push, (unsigned)kListCap);
         for (unsigned e = tid; e < n_list; e += kThreads)
-            filter_fix<EXCL, LOWER, IPT>(P, frame, it, sList[e], tile, sT, hist32, weight);
+            filter_fix<EXCL, LOWER, IPT, HALF>(P, frame, it, sList[e], tile, sT, hist32, weight);
         if (tid == 0 && n_push) {
             atomicAdd(&P.fstats[0], (unsigned long long)n_list);
             if (n_push > n_list) atomicAdd(&P.fstats[1], (unsigned long long)(n_push - n_list));
@@ -386,6 +388,23 @@ __global__ void __launch_bounds__(kThreads, OCC)
         if (audit_bad) atomicAdd(&P.fstats[2], audit_bad);
         if (audit_unc) atomicAdd(&P.fstats[3], audit_unc);
     }
+}
+
+template <bool EXCL, bool LOWER, bool AUDIT, int IPT, int OCC>
+__global__ void __launch_bounds__(kThreads, OCC)
+    rdf_filter_kernel(const __grid_constant__ PairParams P)
+{
+    const FrameFilter ff = P.filt[blockIdx.y];
+    if (ff.wlim == 0u) {                  // left to the exact kernel (whole block)
+        if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&P.fstats[4], 1ull);
+        return;
+    }
+    if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&P.fstats[ff.halfbox ? 5 : 6], 1ull);
+    // the frame's flag is uniform over the block: one branch, then straight-line code
+    if (ff.halfbox)
+        filter_block<EXCL, LOWER, AUDIT, IPT, true>(P, ff);
+    else
+        filter_block<EXCL, LOWER, AUDIT, IPT, false>(P, ff);
 }
 
 // Largest relative error of sqrt.approx.ftz.f32 over two binades [1, 4) -- all 2^24
@@ -525,6 +544,7 @@ FilterPrep rdf_filter_prep(const RdfState &R, double sqrt_err)
 {
     FilterPrep q;
     q.k = R.fc.k;
+    q.halfbox = 0;
     q.scale = R.n_bins / (R.r_hi - R.r_lo);
     q.d_max = R.r_hi + 2.0 / q.scale;
     q.sqrt_err = sqrt_err;
@@ -544,6 +564,7 @@ int rdf_filter_prepare(mdh_ctx *c, int f0, int n_frames, double sqrt_err)
     Q.out = R.filt.as<FrameFilter>();
     Q.n_frames = n_frames;
     Q.prep = rdf_filter_prep(R, sqrt_err);
+    Q.prep.halfbox = 1;            // the all-pairs kernel evaluates both forms
     rdf_filter_prepare_kernel<<<(n_frames + 127) / 128, 128, 0, c->stream>>>(Q);
     MDH_CUDA(cudaGetLastError());
     c->launches++;
