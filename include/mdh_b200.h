@@ -242,6 +242,10 @@ int mdh_rdf_filter_stats(mdh_ctx *ctx, int64_t *stats /* [6] host */);
  * (every coordinate difference within 1.5 box lengths), frames[1] frames it evaluated
  * with the rint form.  Since the last configure / reset. */
 int mdh_rdf_filter_modes(mdh_ctx *ctx, int64_t *frames /* [2] host */);
+/* frames[0] half-box frames the all-pairs filter kernel evaluated without the slot clamp
+ * (its block histogram has a word for every slot the frame can reach; a subset of
+ * mdh_rdf_filter_modes' frames[0]).  Since the last configure / reset. */
+int mdh_rdf_filter_unclamped(mdh_ctx *ctx, int64_t *frames /* [1] host */);
 
 /* ---- seam #2: direct-sum structure factor ------------------------------------ */
 

@@ -76,6 +76,9 @@ struct FrameFilter {
     float nhalf[3];        // -box_k / 2
     int halfbox;           // 1: the all-pairs kernel takes the half-box minimum image
                            // (every |df_k| <= 1.5 box_k; offm / wlim are from its bound)
+    int unclamped;         // 1: (half-box frames only) every slot the fp32 arithmetic can
+                           // produce is a word of the all-pairs kernel's histogram, so its
+                           // hot loop needs no clamp (rdf_device.cuh::filter_reach)
 };
 
 struct FilterConst {       // per configuration (host)
@@ -86,8 +89,16 @@ struct FilterConst {       // per configuration (host)
     int k;                 // fraction bits of the fixed-point bin coordinate
     int sb;                // log2(sub-bins per bin) of the cell-pair kernel's per-warp histograms
     int cb;                // all-pairs filter kernel: log2(columns per slot) of the block's histogram
-    int lg;                // 2^lg >= n_bins + 2
-    int lower;             // r_lo > 0: pairs below the range exist
+    int lg;                // 2^lg >= hslots
+    int lower;             // the bin coordinate can be negative (r_lo > 0 and lo == 0)
+    // all-pairs filter kernel (rdf_filter.cu::filter_plan, per batch of frames); the
+    // cell-list kernels keep lo = 0, hslots = n_bins + 2
+    int lo;                // slot = bin + 1 + lo: the offset is shifted by lo whole slots
+                           // so that the coordinate of a distance >= 0 is never negative
+    int hslots;            // slots of the block histogram; slots outside
+                           // [lo + 1, lo + n_bins] are scratch words, never read
+    int unclamped;         // hslots covers every slot a half-box frame of the batch
+                           // can reach (FrameFilter::unclamped may be set)
 };
 
 struct RdfState {
@@ -120,6 +131,7 @@ struct RdfState {
     bool filter_ok = false;  // this configuration is eligible
     int filter_occ = 2;      // blocks per SM the filter kernel is compiled for (2 or 3)
     FilterConst fc;
+    FilterConst fca;       // the all-pairs filter kernel's layout for the current batch
     DevBuf ext1, ext2;     // unsigned[F][6]: coordinate extents of each frame (keys)
     DevBuf filt;           // FrameFilter[F]
     DevBuf fstats;         // unsigned long long[8], see PairParams::fstats

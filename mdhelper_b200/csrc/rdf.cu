@@ -542,7 +542,7 @@ static int rdf_accumulate_piece(mdh_ctx *c, const float *pos1, int64_t s1, const
         dim3 grid((unsigned)(n_itiles * P.n_jchunks), (unsigned)n_frames);
         const bool excl = R.excl1 > 0;
         P.filt = nullptr;
-        P.fc = R.fc;
+        P.fc = use_filter ? R.fca : R.fc;       // R.fca: set by rdf_filter_prepare
         P.fast_bins = R.fast_bins ? 1 : 0;
         P.fstats = R.fstats.as<unsigned long long>();
         if (use_filter) {

@@ -441,14 +441,42 @@ struct FilterPrep {            // per configuration (host)
     double d_max;              // largest distance that can still be binned
     double sqrt_err;           // measured relative error of sqrt.approx.ftz.f32
     double offbase;            // FilterConst::offbase
+    double fscale;             // FilterConst::scale (the float32 value)
+    int hslots;                // FilterConst::hslots if half-box frames may run unclamped, else 0
 };
+
+// Upper bound of the fixed-point bin coordinate (in bins, relative to slot 0) that
+// filter_d2 + filter_bin2 can produce when every computed |m_k| <= mb[k]; c0 = offm -
+// 1.5*2^(23-k) is the frame's offset coordinate.  floor() of it is the largest slot the
+// frame can reach (DESIGN.md section 4.1b):
+//     d2  <= (mx^2 + my^2 + mz^2) (1 + 2^-24)^3      mul, fma, fma, each rounding up
+//     s   <= sqrt(d2) (1 + sqrt_err)                   sqrt.approx, measured
+//     u   <= s * scale + c0 + 2^-(k+1)                 fma in the binade of 1.5*2^(23-k)
+// scale is the float32 value the kernel multiplies by, so its rounding is exact here.
+__host__ __device__ inline double filter_reach(const double mb[3], double fscale, double c0,
+                                               double sqrt_err, int k)
+{
+    const double e24 = 1.0 / 16777216.0;
+    const double d2 = (mb[0] * mb[0] + mb[1] * mb[1] + mb[2] * mb[2]) * (1.0 + 4.0 * e24);
+    const double s = sqrt(d2) * (1.0 + sqrt_err);
+    // (1 + 1e-12): the fp64 roundings of this evaluation
+    return (s * fscale + c0) * (1.0 + 1e-12) + 1.0 / (double)(2u << k);
+}
+
+// Bound on the computed |m_k| of the half-box form for a frame whose |df_k| <= D_k <= 1.5
+// box_k (h = box_k / 2): both FADDs round towards a result in [-h, h], and for |df| < h
+// the result is within 2^-24 h (one rounding) of |df|.
+__host__ __device__ inline double filter_halfbox_mbound(double D, double h)
+{
+    return fmin(D + h / 8388608.0, h) * (1.0 + 1.0 / 8388608.0);
+}
 
 __device__ inline FrameFilter filter_prepare_frame(const FrameBox &fb, const unsigned *e1,
                                                    const unsigned *e2, const FilterPrep &Q)
 {
     const double e24 = 1.0 / 16777216.0;
     bool ok = true, half = Q.halfbox != 0;
-    double a2 = 0.0, h2 = 0.0;
+    double a2 = 0.0, h2 = 0.0, mb[3];
     FrameFilter ff;
     for (int k = 0; k < 3; ++k) {
         const float e4[4] = {ext_unkey(e1[k]), ext_unkey(e1[3 + k]), ext_unkey(e2[k]),
@@ -480,6 +508,7 @@ __device__ inline FrameFilter filter_prepare_frame(const FrameBox &fb, const uns
         const double ah = e24 * (D <= box ? 0.5 * box : box) * (1.0 + 1e-6) + eps_b * D +
                           D / 2251799813685248.0 + 1e-30;
         h2 += ah * ah;
+        mb[k] = filter_halfbox_mbound(D, 0.5 * box);
         ff.nbox[k] = -(float)box;                          // box is a float32 value
         ff.inv[k] = (float)inv;
         ff.nhalf[k] = -0.5f * (float)box;                  // exact
@@ -499,6 +528,11 @@ __device__ inline FrameFilter filter_prepare_frame(const FrameBox &fb, const uns
         ff.wlim = 0u;
     }
     ff.halfbox = ok && half ? 1 : 0;
+    // the frame's own reachable slot must be a word of the launch's histogram
+    const double magic = 1.5 * (double)(1u << (23 - Q.k));
+    ff.unclamped = ff.halfbox && Q.hslots > 0 &&
+                   filter_reach(mb, Q.fscale, (double)ff.offm - magic, Q.sqrt_err, Q.k) <
+                       (double)Q.hslots;
     return ff;
 }
 
@@ -517,7 +551,6 @@ __device__ __forceinline__ void red_shared_hot(unsigned smem_addr, unsigned v)
 {
     asm volatile("red.shared.add.u32 [%0], %1;" :: "r"(smem_addr), "r"(v));
 }
-
 // ---- parameters of the all-pairs kernels (rdf.cu, rdf_filter.cu) -------------------
 
 struct PairParams {
@@ -538,7 +571,9 @@ struct PairParams {
     unsigned long long *fstats;    // [0] deferred entries, [1] inline fixes, [2] audit
                                    // violations, [3] audited uncertain pairs, [4] frames
                                    // declined by the filter, [5] / [6] frames the all-pairs
-                                   // filter evaluated in the half-box / rint form
+                                   // filter evaluated in the half-box / rint form,
+                                   // [7] half-box frames it evaluated unclamped
+                                   // (counted by rdf_filter_prepare_kernel)
 };
 
 }  // namespace rdfdev

@@ -4,7 +4,7 @@
 // The counts are the reference's, bit for bit: a pair is binned from fp32 arithmetic
 // only when a rigorous error bound proves that the reference's fp64 distance falls in
 // the same bin; every other pair ("uncertain": within the bound of a bin edge, about
-// 1 in 1,500 for the benchmark configurations) is re-evaluated with the exact
+// 1 in 1,000 for the benchmark configurations) is re-evaluated with the exact
 // arithmetic of rdf_device.cuh::pair_d2 and corrected.  The fp32 path costs ~15
 // issue slots per pair (6.5 packed f32x2 instructions on the FMA pipe in the half-box
 // form, 8 in the rint form, ~5 on the ALU pipe, one MUFU, one RED) instead of 21 FP64-pipe instructions plus conversions (46
@@ -23,9 +23,17 @@
 // then d2 = mx*mx + my*my + mz*mz (fma chain), s = sqrt.approx(d2), and the bin
 // coordinate as a fixed-point number in the mantissa of one more fma:
 //     bits(fma(s, scale, 1.5*2^(23-k) + off)) - bits(1.5*2^(23-k)) = slot * 2^k + frac
-// slot = bin + 1 (slot 0: below the range, slot n_bins + 1: above).  The coordinate is
+// slot = bin + 1 + lo (filter_plan: lo = ceil(r_lo * scale) when the histogram is sized
+// for the unclamped body, so that no coordinate is negative; else lo = 0).  The slots
+// outside [lo + 1, lo + n_bins] are scratch words, never read.  The coordinate is
 // additionally shifted up by the window half-width m, so that "within m of a bin
 // edge" reads "fraction bits <= 2m" (one AND + one MIN per pair on the ALU pipe).
+//
+// Three bodies, chosen per frame (one branch per block): half-box unclamped -- the block
+// histogram has a word for every slot the frame's fp32 arithmetic can reach
+// (rdf_device.cuh::filter_reach; cfg2: 353 slots), so a pair's word address is one SHF
+// and one LOP3 --, half-box clamped and rint clamped (one more MIN sends everything
+// beyond the histogram to its last slot).
 //
 // Error bound (rdf_filter_prepare_kernel, per frame, in bin units) -- see DESIGN.md
 // section 4.1b for the derivation.  With eps_b = |box*inv - 1| (the reference's
@@ -56,24 +64,27 @@ namespace {
 #endif
 
 constexpr int kListCap = 3072;           // deferred entries per block and tile
+constexpr int kTilePad = 4;              // rows behind each j-tile: the main loop fetches
+                                         // rows up to 4 ahead without a bound
 
-// shared memory of a block: histogram ((n_bins + 2) slots x 2^cb columns, first, so that
-// its address is the kernel's shared-memory base + an offset), thresholds, two j-tiles,
-// the deferred list
-__host__ __device__ inline size_t filter_hist_bytes(int n_bins, int cb)
+// shared memory of a block: histogram (hslots slots x 2^cb columns, first, so that its
+// address is the kernel's shared-memory base + an offset), thresholds, two j-tiles, the
+// deferred list
+__host__ __device__ inline size_t filter_hist_bytes(int hslots, int cb)
 {
-    return align16(sizeof(unsigned) * ((size_t)(n_bins + 2) << cb));
+    return align16(sizeof(unsigned) * ((size_t)hslots << cb));
 }
 template <int IPT>
-__host__ __device__ inline size_t filter_smem_bytes(int n_bins, int cb)
+__host__ __device__ inline size_t filter_smem_bytes(int n_bins, int hslots, int cb)
 {
-    return filter_hist_bytes(n_bins, cb) + align16(sizeof(double) * (n_bins + 1)) +
-           2 * kThreads * IPT * sizeof(float4) + sizeof(unsigned) * (kListCap + 4);
+    return filter_hist_bytes(hslots, cb) + align16(sizeof(double) * (n_bins + 1)) +
+           2 * (kThreads * IPT + kTilePad) * sizeof(float4) + sizeof(unsigned) * (kListCap + 4);
 }
 
 // Exact re-evaluation of the IPT pairs behind one deferred entry (thread te of the
 // block, tile row jj): every pair the main loop saw as uncertain has been added to
-// the slot the fp32 arithmetic suggested; move it if the fp64 arithmetic disagrees.
+// the slot the fp32 arithmetic suggested -- unclamped: its coordinate's slot, which
+// lies below fc.hslots --; move it if the fp64 arithmetic disagrees.
 template <bool EXCL, bool LOWER, int IPT, bool HALF>
 __device__ __noinline__ void filter_fix(const PairParams &P, int frame, int it, unsigned entry,
                                         const float4 *tile, const double *sT, unsigned hist32,
@@ -104,41 +115,45 @@ __device__ __noinline__ void filter_fix(const PairParams &P, int frame, int it, 
             if (!(u < span_l)) continue;
             if (!((u & ((1u << fc.k) - 1u)) < ff.wlim)) continue;
             if (EXCL && __float_as_int(a.w) == __float_as_int(pj.w)) continue;
-            // the main loop added the pair to (slot it saw, column of thread te's lane)
+            // the main loop added the pair to (slot it saw, column of thread te's lane);
+            // u < span_l: that slot is a word of the histogram, below fc.hslots
             const unsigned seen = (LOWER ? u : u - fc.cbits) >> fc.k;
             const unsigned col = (unsigned)te & ((1u << fc.cb) - 1u);
             const double d2 = pair_d2(a.x, a.y, a.z, pj, fb);
-            const int slot = P.fast_bins ? slot_fast(d2, sT, P.n_bins, P.guess)
-                                         : slot_search(d2, sT, P.n_bins);
+            const int slot = (P.fast_bins ? slot_fast(d2, sT, P.n_bins, P.guess)
+                                          : slot_search(d2, sT, P.n_bins)) + fc.lo;
             if (seen == (unsigned)slot) continue;
-            // slots 0 and n_bins + 1 are scratch words, so no range test is needed
+            // slots outside [lo + 1, lo + n_bins] are scratch words, so no range test is
+            // needed (a count may move between bin n_bins - 1 and a slot above lo + n_bins)
             red_shared(hist32 + 4u * ((seen << fc.cb) + col), 0u - weight);
             red_shared(hist32 + 4u * (((unsigned)slot << fc.cb) + col), weight);
         }
     }
 }
 
-// One block of rdf_filter_kernel with the frame's form of the minimum image.
-template <bool EXCL, bool LOWER, bool AUDIT, int IPT, bool HALF>
+// One block of rdf_filter_kernel with the frame's form of the minimum image; CLAMP =
+// false for frames whose every reachable slot is a histogram word (FrameFilter::unclamped).
+template <bool EXCL, bool LOWER, bool AUDIT, int IPT, bool HALF, bool CLAMP>
 __device__ __forceinline__ void filter_block(const PairParams &P, const FrameFilter &ff)
 {
     constexpr int TILE = kThreads * IPT;
+    constexpr int TSTRIDE = TILE + kTilePad;
     const int frame = blockIdx.y;
 
     extern __shared__ __align__(16) unsigned char smem[];
     const int n_bins = P.n_bins;
     const FilterConst fc = P.fc;
-    // ONE histogram per block: (n_bins + 2) slots x 2^cb columns, a lane updates column
-    // lane mod 2^cb -- with 32 columns the 32 updates of a warp instruction fall in 32
-    // different banks whatever the bins are (per-warp histograms with sub-bins took 3.8
-    // wavefronts per instruction on random bins).  Slot n_bins + 1 ("above the range") takes
-    // every pair beyond the range; it is never read.
-    const int hwords = (n_bins + 2) << fc.cb;
+    // ONE histogram per block: hslots slots x 2^cb columns, a lane updates column lane mod
+    // 2^cb -- with 32 columns the 32 updates of a warp instruction fall in 32 different
+    // banks whatever the bins are (per-warp histograms with sub-bins took 3.8 wavefronts
+    // per instruction on random bins).  Only slots lo + 1 .. lo + n_bins are read; the
+    // others take the pairs outside the range.
+    const int hwords = fc.hslots << fc.cb;
     unsigned *sH = reinterpret_cast<unsigned *>(smem);
-    double *sT = reinterpret_cast<double *>(smem + filter_hist_bytes(n_bins, fc.cb));
+    double *sT = reinterpret_cast<double *>(smem + filter_hist_bytes(fc.hslots, fc.cb));
     float4 *sJ = reinterpret_cast<float4 *>(reinterpret_cast<unsigned char *>(sT) +
                                             align16(sizeof(double) * (n_bins + 1)));
-    unsigned *sList = reinterpret_cast<unsigned *>(sJ + 2 * TILE);
+    unsigned *sList = reinterpret_cast<unsigned *>(sJ + 2 * TSTRIDE);
     unsigned *sCount = sList + kListCap;
 
     const int tid = threadIdx.x, lane = tid & 31;
@@ -181,13 +196,14 @@ __device__ __forceinline__ void filter_block(const PairParams &P, const FrameFil
     // Byte offset of a pair's word without touching the FMA pipe (an IMAD per pair there
     // costs as much as a packed FP32 instruction): t = u >> (k - cb - 2) holds the slot in
     // bits [cb + 2, cb + 2 + lg) -- above them, for !LOWER, the bits of 1.5*2^(23-k), which
-    // start at bit 24 - k + cb >= cb + 2 + lg --, fraction bits below.  One MIN clamps
-    // everything beyond the range to slot n_bins + 1, one LOP3 keeps the slot field and
-    // inserts the lane's column; the base is the kernel's shared-memory base, an immediate.
+    // start at bit 24 - k + cb >= cb + 2 + lg --, fraction bits below.  CLAMP: one MIN
+    // sends everything beyond the histogram to its last slot (a scratch word); without
+    // it the slot is below hslots already.  One LOP3 keeps the slot field and inserts the
+    // lane's column; the base is the kernel's shared-memory base, an immediate.
     const int tshift = fc.k - fc.cb - 2;
     const unsigned low = (4u << fc.cb) - 1u;
     const unsigned tmask = ((4u << (fc.cb + fc.lg)) - 1u) & ~low;
-    const unsigned tmax = ((((LOWER ? 0u : fc.cbits) >> fc.k) + (unsigned)(n_bins + 1))
+    const unsigned tmax = ((((LOWER ? 0u : fc.cbits) >> fc.k) + (unsigned)(fc.hslots - 1))
                            << (fc.cb + 2)) | low;
     const unsigned colbits = ((unsigned)lane & ((1u << fc.cb) - 1u)) << 2;
     const unsigned span_l = LOWER ? fc.span : fc.cbits + fc.span;
@@ -196,7 +212,7 @@ __device__ __forceinline__ void filter_block(const PairParams &P, const FrameFil
 
     auto stage_tile = [&](int jt, int buf) {
         const float4 *src = f2 + (int64_t)jt * TILE;
-        float4 *dst = sJ + buf * TILE;
+        float4 *dst = sJ + buf * TSTRIDE;
 #pragma unroll
         for (int q = 0; q < IPT; ++q)
             __pipeline_memcpy_async(dst + q * kThreads + tid, src + q * kThreads + tid,
@@ -221,7 +237,7 @@ __device__ __forceinline__ void filter_block(const PairParams &P, const FrameFil
 #pragma unroll
         for (int ii = 0; ii < IPT; ++ii) wi[ii] = vi[ii] ? weight : 0u;
         const int jn = min(TILE, P.n2 - jt * TILE);
-        const float4 *tile = sJ + buf * TILE;
+        const float4 *tile = sJ + buf * TSTRIDE;
 
         // Stage A1: packed squared distances of NR tile rows against the IPT particles of
         // this thread (FMA pipe only).
@@ -257,23 +273,29 @@ __device__ __forceinline__ void filter_block(const PairParams &P, const FrameFil
                     const unsigned u = uu[r][ii];
                     // uncertain iff the fraction bits are below wlim; keep the smallest
                     vmin[r] = min(vmin[r], u & fmask);
-                    unsigned t = min(u >> tshift, tmax);
+                    unsigned t = u >> tshift;
+                    if (CLAMP) t = min(t, tmax);
                     if (EXCL && gi[ii] == __float_as_int(pj[r].w)) t = tmax;
                     red_shared_hot(hist32 + lop3_and_or(t, tmask, colbits), wi[ii]);
                     if (AUDIT) {
                         const bool unc = (u & fmask) < ff.wlim;
                         const bool in = u < span_l;
+                        // an unclamped frame must never leave the histogram
+                        if (!CLAMP && !in) ++audit_bad;
                         const double d2 =
                             pair_d2(xi[ii], yi[ii], zi[ii], pj[r], P.boxes[frame]);
                         const int slot = slot_search(d2, sT, n_bins);
+                        // the slot the pair was added to, and the exact one
                         const unsigned fs = in ? ((LOWER ? u : u - fc.cbits) >> fc.k)
-                                               : (unsigned)(n_bins + 1);
+                                               : (unsigned)(fc.hslots - 1);
+                        const unsigned xs = (unsigned)(slot + fc.lo);
                         const bool counted = slot >= 1 && slot <= n_bins;
                         if (in && unc) ++audit_unc;
                         // certain pairs must agree with the exact arithmetic wherever
                         // a count is at stake
-                        if (!(in && unc) && (unsigned)slot != fs &&
-                            (counted || (fs >= 1u && fs <= (unsigned)n_bins)))
+                        if (!(in && unc) && xs != fs &&
+                            (counted || (fs >= (unsigned)fc.lo + 1u &&
+                                         fs <= (unsigned)(fc.lo + n_bins))))
                             ++audit_bad;
                     }
                 }
@@ -312,29 +334,27 @@ __device__ __forceinline__ void filter_block(const PairParams &P, const FrameFil
         // every warp offers both pipes work from its first to its last instruction; the
         // rows after those are fetched from shared memory one more iteration ahead.  Rows
         // up to TILE - 1 always exist (the packed arrays are padded), so the last
-        // iteration may evaluate two rows nobody uses.
+        // iteration may evaluate two rows nobody uses; the rows fetched past the end of the
+        // tile are its kTilePad padding rows.
         using two = std::integral_constant<int, 2>;
         const int jn2 = jn & ~1;
-        f32x2 da[2][IPT / 2];
+        f32x2 da[2][IPT / 2], db[2][IPT / 2];
         float4 cur[2] = {tile[0], tile[1]};
         float4 nxt[2] = {tile[2], tile[3]};
         if (jn2 > 0) stage_a1(cur, da, two());
-        // one step of the pipeline: rows (jj, jj+1) leave it, rows (jj+2, jj+3) enter
-        auto step = [&](int jj, unsigned *vmin) {
+        // one step of the pipeline: rows (jj, jj+1) leave it (their squared distances in
+        // din), rows (jj+2, jj+3) enter it (into dout).  The steps alternate da and db,
+        // so no register is copied from one step to the next.
+        auto step = [&](int jj, const f32x2 (*din)[IPT / 2], f32x2 (*dout)[IPT / 2],
+                        unsigned *vmin) {
             unsigned ua[2][IPT];
-            f32x2 db[2][IPT / 2];
             const float4 nn[2] = {nxt[0], nxt[1]};
-            const int jfetch = min(jj + 4, TILE - 2);
-            nxt[0] = tile[jfetch];
-            nxt[1] = tile[jfetch + 1];
-            stage_a2(da, ua, two());
-            stage_a1(nn, db, two());
+            nxt[0] = tile[jj + 4];
+            nxt[1] = tile[jj + 5];
+            stage_a2(din, ua, two());
+            stage_a1(nn, dout, two());
             stage_hist(cur, ua, vmin, two());
             cur[0] = nn[0]; cur[1] = nn[1];
-#pragma unroll
-            for (int r = 0; r < 2; ++r)
-#pragma unroll
-                for (int ip = 0; ip < IPT / 2; ++ip) da[r][ip] = db[r][ip];
         };
         int jj = 0;
 #if MDH_FILTER_ROWS == 4
@@ -342,14 +362,24 @@ __device__ __forceinline__ void filter_block(const PairParams &P, const FrameFil
         // the steps, so the second step's arithmetic overlaps the first step's updates
         for (; jj + 4 <= jn2; jj += 4) {
             unsigned vmin[4];
-            step(jj, vmin);
-            step(jj + 2, vmin + 2);
+            step(jj, da, db, vmin);
+            step(jj + 2, db, da, vmin + 2);
             stage_push(vmin, jj, std::integral_constant<int, 4>());
         }
-#endif
-        for (; jj < jn2; jj += 2) {
+#else
+        // two steps per trip, each with its own test for uncertain pairs: one loop
+        // counter, compare and branch per 2 steps, one row address per 2 steps
+        for (; jj + 4 <= jn2; jj += 4) {
             unsigned vmin[2];
-            step(jj, vmin);
+            step(jj, da, db, vmin);
+            stage_push(vmin, jj, two());
+            step(jj + 2, db, da, vmin);
+            stage_push(vmin, jj + 2, two());
+        }
+#endif
+        if (jj < jn2) {
+            unsigned vmin[2];
+            step(jj, da, db, vmin);
             stage_push(vmin, jj, two());
         }
         if (jn2 < jn) {
@@ -381,7 +411,7 @@ __device__ __forceinline__ void filter_block(const PairParams &P, const FrameFil
     for (int k = tid; k < n_bins; k += kThreads) {
         unsigned s = 0;
         for (int q = 0; q < (1 << fc.cb); ++q)
-            s += sH[((k + 1) << fc.cb) + ((q + tid) & ((1 << fc.cb) - 1))];
+            s += sH[((k + 1 + fc.lo) << fc.cb) + ((q + tid) & ((1 << fc.cb) - 1))];
         if (s) atomicAdd(&P.counts[k], (unsigned long long)s);
     }
     if (AUDIT) {
@@ -400,11 +430,19 @@ __global__ void __launch_bounds__(kThreads, OCC)
         return;
     }
     if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&P.fstats[ff.halfbox ? 5 : 6], 1ull);
-    // the frame's flag is uniform over the block: one branch, then straight-line code
-    if (ff.halfbox)
-        filter_block<EXCL, LOWER, AUDIT, IPT, true>(P, ff);
-    else
-        filter_block<EXCL, LOWER, AUDIT, IPT, false>(P, ff);
+    // the frame's flags are uniform over the block: one branch, then straight-line code.
+    // A launch whose coordinates may be negative (LOWER) never has unclamped frames.
+    if (ff.halfbox) {
+        if constexpr (!LOWER) {
+            if (ff.unclamped) {
+                filter_block<EXCL, LOWER, AUDIT, IPT, true, false>(P, ff);
+                return;
+            }
+        }
+        filter_block<EXCL, LOWER, AUDIT, IPT, true, true>(P, ff);
+    } else {
+        filter_block<EXCL, LOWER, AUDIT, IPT, false, true>(P, ff);
+    }
 }
 
 // Largest relative error of sqrt.approx.ftz.f32 over two binades [1, 4) -- all 2^24
@@ -427,6 +465,7 @@ struct PrepareParams {
     const FrameBox *boxes;
     const unsigned *ext1, *ext2;     // [F][6] keys
     FrameFilter *out;
+    unsigned long long *fstats;      // [7]: frames the filter kernel will run unclamped
     int n_frames;
     FilterPrep prep;
 };
@@ -435,13 +474,18 @@ __global__ void rdf_filter_prepare_kernel(const PrepareParams Q)
 {
     const int f = blockIdx.x * blockDim.x + threadIdx.x;
     if (f >= Q.n_frames) return;
-    Q.out[f] = filter_prepare_frame(Q.boxes[f], Q.ext1 + f * 6, Q.ext2 + f * 6, Q.prep);
+    const FrameFilter ff = filter_prepare_frame(Q.boxes[f], Q.ext1 + f * 6, Q.ext2 + f * 6, Q.prep);
+    Q.out[f] = ff;
+    // counted here rather than in the filter kernel, whose register allocation is at its
+    // limit; rdf_filter_kernel takes the unclamped body exactly for these frames (the
+    // flag is only set when the launch's layout has no negative coordinates, !LOWER)
+    if (ff.unclamped) atomicAdd(&Q.fstats[7], 1ull);
 }
 
 template <bool EXCL, bool LOWER, bool AUDIT, int IPT, int OCC>
 int launch_filter_o(mdh_ctx *c, const PairParams &P, dim3 grid)
 {
-    const size_t smem = filter_smem_bytes<IPT>(P.n_bins, P.fc.cb);
+    const size_t smem = filter_smem_bytes<IPT>(P.n_bins, P.fc.hslots, P.fc.cb);
     auto kern = rdf_filter_kernel<EXCL, LOWER, AUDIT, IPT, OCC>;
     MDH_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   (int)smem));
@@ -491,6 +535,23 @@ int rdf_filter_sqrt_error(mdh_ctx *c, double *err)
     return MDH_OK;
 }
 
+// shared memory of one block of the all-pairs filter kernel
+static size_t filter_need(const RdfState &R, int hslots, int cb)
+{
+    return R.ipt == 2 ? filter_smem_bytes<2>(R.n_bins, hslots, cb)
+                      : filter_smem_bytes<4>(R.n_bins, hslots, cb);
+}
+
+// histogram columns: as many (up to one per lane) as the shared memory of R.filter_occ
+// resident blocks allows
+static int filter_columns(const RdfState &R, int hslots, int k)
+{
+    const size_t budget = (size_t)(224 * 1024) / R.filter_occ - 1024;
+    int cb = 5;
+    while (cb > 0 && filter_need(R, hslots, cb) > budget) --cb;
+    return std::min(cb, k - 2);
+}
+
 // Decides whether a configuration can use the filter and fills R.fc.
 bool rdf_filter_configure(RdfState &R, const double *thr, double sqrt_err)
 {
@@ -523,16 +584,11 @@ bool rdf_filter_configure(RdfState &R, const double *thr, double sqrt_err)
     fc.span = (unsigned)(n_bins + 2) << k;
     fc.lower = R.r_lo > 0.0;
     fc.lg = lg;
-    // histogram columns: as many (up to one per lane) as the shared memory of
-    // R.filter_occ resident blocks allows
-    const size_t budget = (size_t)(224 * 1024) / R.filter_occ - 1024;
-    auto need = [&](int cb) {
-        return R.ipt == 2 ? filter_smem_bytes<2>(n_bins, cb) : filter_smem_bytes<4>(n_bins, cb);
-    };
-    int cb = 5;
-    while (cb > 0 && need(cb) > budget) --cb;
-    fc.cb = std::min(cb, k - 2);
-    if (need(fc.cb) > 200 * 1024) return false;
+    fc.lo = 0;
+    fc.hslots = n_bins + 2;
+    fc.unclamped = 0;
+    fc.cb = filter_columns(R, fc.hslots, k);
+    if (filter_need(R, fc.hslots, fc.cb) > 200 * 1024) return false;
     // the cell-pair kernel keeps one histogram per warp with 2^sb sub-bins per bin
     fc.sb = std::min(2, k);
     R.fc = fc;
@@ -549,22 +605,98 @@ FilterPrep rdf_filter_prep(const RdfState &R, double sqrt_err)
     q.d_max = R.r_hi + 2.0 / q.scale;
     q.sqrt_err = sqrt_err;
     q.offbase = R.fc.offbase;
+    q.fscale = (double)R.fc.scale;
+    q.hslots = 0;
     return q;
 }
 
-// Builds the per-frame filter parameters of a batch (device side, asynchronous).
+// The all-pairs filter kernel's histogram layout for a batch of frames.  Sized so that
+// every slot a half-box frame of the batch can reach is a word (rdf_device.cuh::
+// filter_reach with the largest |m| of the form, |m_k| <= box_k / 2), with the offset
+// shifted by lo = ceil(r_lo * scale) slots so that no coordinate is negative.  When that
+// histogram does not fit the shared memory of R.filter_occ blocks at the clamped layout's
+// column count, or would leave fewer than 9 fraction bits or more than one fewer than the
+// clamped layout (each lost bit about doubles the uncertain pairs; one bit is what the
+// measured trade covers: cfg2, 1.6x deferred entries for a 7 % faster kernel), it is the
+// clamped layout R.fc.
+static FilterConst filter_plan(const RdfState &R, const FrameBox *boxes, int n_frames,
+                               double sqrt_err)
+{
+    FilterConst fc = R.fc;
+    const int n_bins = R.n_bins;
+    const double scale = n_bins / (R.r_hi - R.r_lo);
+    const int lo = (int)ceil(R.r_lo * scale);
+    // offset coordinate: 1 + lo - r_lo * scale rounded to 2^-k, plus the window (< 1/16 by
+    // filter_prepare_frame's 2m + 1 < 2^k / 8)
+    auto top = [&](const FrameBox &b, int k) {
+        double mb[3];
+        for (int a = 0; a < 3; ++a) {
+            const double h = 0.5 * b.box[a];
+            mb[a] = filter_halfbox_mbound(a == R.drop_axis ? 0.0 : h, h);  // dropped: df = 0
+        }
+        const double c0 = 1.0 + lo - R.r_lo * scale + 1.0 / 16.0 + 1.0 / (double)(2u << k);
+        return floor(filter_reach(mb, (double)fc.scale, c0, sqrt_err, k));
+    };
+    // the frames' reachable slots at k = 9, the coarsest rounding; the histogram covers the
+    // largest of them that fits (frames beyond it keep the clamped body)
+    std::vector<double> t9(n_frames);
+    for (int f = 0; f < n_frames; ++f) t9[f] = top(boxes[f], 9);
+    std::sort(t9.begin(), t9.end());
+    t9.erase(std::unique(t9.begin(), t9.end()), t9.end());
+    int hslots = 0, k = 0, cb = 0;
+    for (int q = (int)t9.size() - 1; q >= 0 && hslots == 0; --q) {
+        if (!(t9[q] < 65536.0)) continue;
+        const int hs = std::max((int)t9[q] + 1, n_bins + lo + 2);
+        int lg = 0;
+        while ((1 << lg) < hs) ++lg;
+        k = std::min(16, 22 - lg);
+        if (k < 9 || k < R.fc.k - 1) continue;
+        cb = filter_columns(R, hs, k);
+        if (cb < R.fc.cb || filter_need(R, hs, cb) > 200 * 1024) continue;
+        hslots = hs;
+    }
+    if (hslots == 0) return fc;
+    int lg = 0;
+    while ((1 << lg) < hslots) ++lg;
+    const double two_k = (double)(1 << k);
+    const double magic = 1.5 * (double)(1 << (23 - k));
+    const double offbase = magic + nearbyint((1.0 + lo - R.r_lo * scale) * two_k) / two_k;
+    // representable with the largest shift added, and still below the next binade
+    if ((double)(float)offbase != offbase || (double)(float)(offbase + 0.125) != offbase + 0.125)
+        return fc;
+    fc.k = k;
+    fc.offbase = offbase;
+    const float mf = (float)magic;
+    memcpy(&fc.cbits, &mf, 4);
+    fc.span = (unsigned)hslots << k;
+    fc.lg = lg;
+    fc.cb = cb;
+    fc.lower = 0;
+    fc.lo = lo;
+    fc.hslots = hslots;
+    fc.unclamped = 1;
+    return fc;
+}
+
+// Builds the per-frame filter parameters of a batch (device side, asynchronous) and the
+// all-pairs kernel's layout for it (R.fca).
 int rdf_filter_prepare(mdh_ctx *c, int f0, int n_frames, double sqrt_err)
 {
     RdfState &R = c->rdf;
     if (int rc = R.filt.reserve(sizeof(FrameFilter) * n_frames)) return rc;
+    R.fca = filter_plan(R, R.h_boxes.data() + f0, n_frames, sqrt_err);
     PrepareParams Q;
     Q.boxes = R.boxes.as<FrameBox>() + f0;
     Q.ext1 = R.ext1.as<unsigned>();
     Q.ext2 = R.same ? Q.ext1 : R.ext2.as<unsigned>();
     Q.out = R.filt.as<FrameFilter>();
+    Q.fstats = R.fstats.as<unsigned long long>();
     Q.n_frames = n_frames;
     Q.prep = rdf_filter_prep(R, sqrt_err);
     Q.prep.halfbox = 1;            // the all-pairs kernel evaluates both forms
+    Q.prep.k = R.fca.k;
+    Q.prep.offbase = R.fca.offbase;
+    Q.prep.hslots = R.fca.unclamped ? R.fca.hslots : 0;
     rdf_filter_prepare_kernel<<<(n_frames + 127) / 128, 128, 0, c->stream>>>(Q);
     MDH_CUDA(cudaGetLastError());
     c->launches++;
