@@ -216,6 +216,29 @@ int mdh_rdf_triclinic_grid(const float *cell /* [9] */, double r_hi, int64_t n_m
 int mdh_rdf_cells_grid(const float *cell /* [9] */, double r_hi, int64_t n_max, int drop_axis,
                        int32_t *nc /* [3] */, double *margin);
 
+/*
+ * The fp32 filter's layout and per-frame windows for a configuration and a batch of frames,
+ * computed on the host as mdh_rdf_configure and mdh_rdf_accumulate would; device-free (the
+ * device measures sqrt_err, the relative error of sqrt.approx.ftz.f32; here the caller gives
+ * it, at most 2^-22).  n_bins, r_lo, r_hi, drop_axis as for mdh_rdf_configure (uniform bin
+ * edges); ipt (2 or 4) and filter_occ (2..4) as MDH_TUNE's ipt= and occ=.  box[n_frames][3]
+ * as for mdh_rdf_accumulate; ext1 / ext2 [n_frames][6]: {min x, y, z, max x, y, z} of the
+ * float32 coordinates of each group (the dropped coordinate 0; ext2 NULL: the same group).
+ * layout[2][12]: the configuration's clamped layout (what the cell-list kernels use), then
+ * the all-pairs kernel's layout for this batch, each {k, scale, offbase, cbits, span, lg,
+ * cb, hslots, lo, unclamped, sb, lower} (FilterConst).  frames[n_frames][2][5]: for the
+ * all-pairs kernel (half-box form allowed, batch layout), then for the cell-list kernels
+ * (rint form, clamped layout), each {offm, wlim, halfbox, unclamped, mu}: the FrameFilter
+ * and the error bound mu in bins (before the window's 1.25 margin).  MDH_EINVAL when the
+ * configuration is not eligible for the filter.
+ */
+int mdh_rdf_filter_window(int n_bins, double r_lo, double r_hi, int drop_axis, int ipt,
+                          int filter_occ, double sqrt_err, int n_frames,
+                          const float *box /* [n_frames][3] */,
+                          const float *ext1 /* [n_frames][6] */,
+                          const float *ext2 /* [n_frames][6] or NULL */,
+                          double *layout /* [2][12] */, double *frames /* [n_frames][2][5] */);
+
 int mdh_rdf_fetch(mdh_ctx *ctx, int64_t *counts /* [n_bins] host */);
 int mdh_rdf_reset(mdh_ctx *ctx);
 /* device address of the int64[n_bins] accumulator (for NCCL reductions) */

@@ -49,6 +49,8 @@ SIGNATURES = {
     "mdh_rdf_accumulate_triclinic": (_i32, [_p, _p, _i64, _p, _i64, _i32, _p, _i32]),
     "mdh_rdf_triclinic_grid": (_i32, [_p, _f64, _i64, _p, ctypes.POINTER(_f64)]),
     "mdh_rdf_cells_grid": (_i32, [_p, _f64, _i64, _i32, _p, ctypes.POINTER(_f64)]),
+    "mdh_rdf_filter_window": (_i32, [_i32, _f64, _f64, _i32, _i32, _i32, _f64, _i32, _p, _p,
+                                     _p, _p, _p]),
     "mdh_rdf_fetch": (_i32, [_p, _p]),
     "mdh_rdf_reset": (_i32, [_p]),
     "mdh_rdf_counts_device": (_i32, [_p, ctypes.POINTER(_p)]),
@@ -180,6 +182,42 @@ def cells_grid(cell, r_hi: float, n_max: int, drop_axis=None):
                                    -1 if drop_axis is None else int(drop_axis), nc.ctypes.data,
                                    ctypes.byref(margin)))
     return tuple(int(v) for v in nc), margin.value
+
+
+FILTER_LAYOUT_FIELDS = ("k", "scale", "offbase", "cbits", "span", "lg", "cb", "hslots", "lo",
+                        "unclamped", "sb", "lower")
+FILTER_FRAME_FIELDS = ("offm", "wlim", "halfbox", "unclamped", "mu")
+
+
+def filter_window(n_bins: int, r_lo: float, r_hi: float, box, ext1, ext2=None, *,
+                  drop_axis=None, ipt: int = 4, filter_occ: int = 2,
+                  sqrt_err: float = 2.0 ** -22) -> dict:
+    """Layout and per-frame windows of the fp32 RDF filter (``mdh_rdf_filter_window``; no
+    device needed).  ``box``: ``[n_frames, 3]``; ``ext1`` / ``ext2``: ``[n_frames, 6]``
+    float32 extents {min x, y, z, max x, y, z} of the two groups (``ext2=None``: one group).
+    Returns ``{"clamped": layout, "allpairs": layout, "frames": [{"allpairs": window,
+    "cells": window}, ...]}`` with the fields of ``FILTER_LAYOUT_FIELDS`` and
+    ``FILTER_FRAME_FIELDS`` (integers as ``int``; ``scale``, ``offbase``, ``offm``, ``mu`` as
+    ``float``).  Raises ``ValueError`` when the configuration is not eligible for the filter."""
+    b = np.ascontiguousarray(box, dtype=np.float32).reshape(-1, 3)
+    nf = len(b)
+    e1 = np.ascontiguousarray(ext1, dtype=np.float32).reshape(nf, 6)
+    e2 = None if ext2 is None else np.ascontiguousarray(ext2, dtype=np.float32).reshape(nf, 6)
+    lay = np.zeros((2, 12), np.float64)
+    fr = np.zeros((nf, 2, 5), np.float64)
+    check(lib().mdh_rdf_filter_window(int(n_bins), float(r_lo), float(r_hi),
+                                      -1 if drop_axis is None else int(drop_axis), int(ipt),
+                                      int(filter_occ), float(sqrt_err), nf, b.ctypes.data,
+                                      e1.ctypes.data, _ptr(e2), lay.ctypes.data,
+                                      fr.ctypes.data))
+
+    def typed(names, vals):
+        return {n: (float(v) if n in ("scale", "offbase", "offm", "mu") else int(v))
+                for n, v in zip(names, vals)}
+    return {"clamped": typed(FILTER_LAYOUT_FIELDS, lay[0]),
+            "allpairs": typed(FILTER_LAYOUT_FIELDS, lay[1]),
+            "frames": [{"allpairs": typed(FILTER_FRAME_FIELDS, fr[f, 0]),
+                        "cells": typed(FILTER_FRAME_FIELDS, fr[f, 1])} for f in range(nf)]}
 
 
 class Context:

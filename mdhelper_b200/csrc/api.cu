@@ -345,6 +345,14 @@ int mdh_rdf_cells_grid(const float *cell, double r_hi, int64_t n_max, int drop_a
     return rdf_cells_grid_impl(cell, r_hi, n_max, drop_axis, nc, margin);
 }
 
+int mdh_rdf_filter_window(int n_bins, double r_lo, double r_hi, int drop_axis, int ipt,
+                          int filter_occ, double sqrt_err, int n_frames, const float *box,
+                          const float *ext1, const float *ext2, double *layout, double *frames)
+{
+    return rdf_filter_window_impl(n_bins, r_lo, r_hi, drop_axis, ipt, filter_occ, sqrt_err,
+                                  n_frames, box, ext1, ext2, layout, frames);
+}
+
 int mdh_rdf_fetch(mdh_ctx *c, int64_t *counts)
 {
     CTX_GUARD(c);

@@ -303,6 +303,9 @@ int rdf_cells_grid_impl(const float *cell9, double r_hi, int64_t n_max, int drop
 int rdf_filter_sqrt_error(mdh_ctx *c, double *err);
 bool rdf_filter_configure(RdfState &R, const double *thr, double sqrt_err);
 int rdf_filter_prepare(mdh_ctx *c, int f0, int n_frames, double sqrt_err);
+int rdf_filter_window_impl(int n_bins, double r_lo, double r_hi, int drop_axis, int ipt,
+                           int filter_occ, double sqrt_err, int n_frames, const float *box,
+                           const float *ext1, const float *ext2, double *layout, double *frames);
 // sq.cu
 int sq_configure_impl(mdh_ctx *c, int64_t n_total, int n_groups, const int64_t *goff,
                       int n_q, const double *wv, const int32_t *lat_n, const double *lat_b,

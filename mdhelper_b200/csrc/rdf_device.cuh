@@ -471,8 +471,22 @@ __host__ __device__ inline double filter_halfbox_mbound(double D, double h)
     return fmin(D + h / 8388608.0, h) * (1.0 + 1.0 / 8388608.0);
 }
 
-__device__ inline FrameFilter filter_prepare_frame(const FrameBox &fb, const unsigned *e1,
-                                                   const unsigned *e2, const FilterPrep &Q)
+// bits of a float, on the host and on the device
+__host__ __device__ inline unsigned f32_bits(float f)
+{
+#ifdef __CUDA_ARCH__
+    return __float_as_uint(f);
+#else
+    unsigned b; memcpy(&b, &f, 4); return b;
+#endif
+}
+
+// Host and device: the preparation kernels run it per frame, mdh_rdf_filter_window on the
+// host (device-free tests of the window).  mu (optional): the bound in bins, before the
+// 1.25 margin of the window.
+__host__ __device__ inline FrameFilter filter_prepare_frame(const FrameBox &fb, const unsigned *e1,
+                                                            const unsigned *e2, const FilterPrep &Q,
+                                                            double *mu_out = nullptr)
 {
     const double e24 = 1.0 / 16777216.0;
     bool ok = true, half = Q.halfbox != 0;
@@ -483,7 +497,7 @@ __device__ inline FrameFilter filter_prepare_frame(const FrameBox &fb, const uns
                              ext_unkey(e2[3 + k])};
         // inf / NaN coordinates (all-ones exponent) make the bound meaningless
         for (int q = 0; q < 4; ++q)
-            if ((__float_as_uint(e4[q]) & 0x7f800000u) == 0x7f800000u) ok = false;
+            if ((f32_bits(e4[q]) & 0x7f800000u) == 0x7f800000u) ok = false;
         const double lo1 = (double)e4[0], hi1 = (double)e4[1];
         const double lo2 = (double)e4[2], hi2 = (double)e4[3];
         // D >= every |df| of the frame, the float32 rounding of df included
@@ -517,6 +531,7 @@ __device__ inline FrameFilter filter_prepare_frame(const FrameBox &fb, const uns
     const double two_k = (double)(1u << Q.k);
     const double mu = Q.scale * (sqrt(a2) + Q.d_max * (1.5 * e24 * 1.001 + Q.sqrt_err)) +
                       e24 * Q.scale * Q.d_max * 1.001 + 1.0 / two_k + 1e-9;
+    if (mu_out) *mu_out = mu;
     const double m = ceil(1.25 * mu * two_k) + 1.0;
     if (!(m >= 1.0) || !(2.0 * m + 1.0 < two_k / 8.0)) ok = false;
     if (ok) {

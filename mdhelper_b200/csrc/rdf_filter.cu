@@ -678,6 +678,17 @@ static FilterConst filter_plan(const RdfState &R, const FrameBox *boxes, int n_f
     return fc;
 }
 
+// The per-frame preparation of the all-pairs filter kernel for the batch layout fca
+static FilterPrep filter_prep_allpairs(const RdfState &R, const FilterConst &fca, double sqrt_err)
+{
+    FilterPrep q = rdf_filter_prep(R, sqrt_err);
+    q.halfbox = 1;                 // the all-pairs kernel evaluates both forms
+    q.k = fca.k;
+    q.offbase = fca.offbase;
+    q.hslots = fca.unclamped ? fca.hslots : 0;
+    return q;
+}
+
 // Builds the per-frame filter parameters of a batch (device side, asynchronous) and the
 // all-pairs kernel's layout for it (R.fca).
 int rdf_filter_prepare(mdh_ctx *c, int f0, int n_frames, double sqrt_err)
@@ -692,11 +703,7 @@ int rdf_filter_prepare(mdh_ctx *c, int f0, int n_frames, double sqrt_err)
     Q.out = R.filt.as<FrameFilter>();
     Q.fstats = R.fstats.as<unsigned long long>();
     Q.n_frames = n_frames;
-    Q.prep = rdf_filter_prep(R, sqrt_err);
-    Q.prep.halfbox = 1;            // the all-pairs kernel evaluates both forms
-    Q.prep.k = R.fca.k;
-    Q.prep.offbase = R.fca.offbase;
-    Q.prep.hslots = R.fca.unclamped ? R.fca.hslots : 0;
+    Q.prep = filter_prep_allpairs(R, R.fca, sqrt_err);
     rdf_filter_prepare_kernel<<<(n_frames + 127) / 128, 128, 0, c->stream>>>(Q);
     MDH_CUDA(cudaGetLastError());
     c->launches++;
@@ -710,4 +717,74 @@ int rdf_filter_launch(mdh_ctx *c, const PairParams &P, dim3 grid, bool excl, boo
                           : launch_filter_a<true, false>(c, P, grid, audit);
     return P.fc.lower ? launch_filter_a<false, true>(c, P, grid, audit)
                       : launch_filter_a<false, false>(c, P, grid, audit);
+}
+
+// Device-free: the layouts and per-frame windows the filter would use (mdh_rdf_filter_window).
+int rdf_filter_window_impl(int n_bins, double r_lo, double r_hi, int drop_axis, int ipt,
+                           int filter_occ, double sqrt_err, int n_frames, const float *box,
+                           const float *ext1, const float *ext2, double *layout, double *frames)
+{
+    MDH_REQUIRE(n_bins >= 1 && n_bins <= 65536, MDH_EINVAL, "filter_window: n_bins must be in [1, 65536]");
+    MDH_REQUIRE(r_hi > r_lo && r_lo >= 0, MDH_EINVAL, "filter_window: invalid range");
+    MDH_REQUIRE(drop_axis >= -1 && drop_axis <= 2, MDH_EINVAL, "filter_window: invalid drop_axis");
+    MDH_REQUIRE(ipt == 2 || ipt == 4, MDH_EINVAL, "filter_window: ipt must be 2 or 4");
+    MDH_REQUIRE(filter_occ >= 2 && filter_occ <= 4, MDH_EINVAL,
+                "filter_window: filter_occ must be in [2, 4]");
+    MDH_REQUIRE(n_frames >= 1 && box != nullptr && ext1 != nullptr && layout != nullptr &&
+                    frames != nullptr, MDH_EINVAL, "filter_window: NULL argument");
+    if (ext2 == nullptr) ext2 = ext1;
+    RdfState R;                    // host fields only: no device buffer is touched
+    R.n_bins = n_bins;
+    R.r_lo = r_lo;
+    R.r_hi = r_hi;
+    R.drop_axis = drop_axis;
+    R.ipt = ipt;
+    R.filter_occ = filter_occ;
+    // uniform edges (rdf_filter_configure only checks that the thresholds are these)
+    std::vector<double> thr(n_bins + 1);
+    for (int i = 0; i <= n_bins; ++i) {
+        const double e = r_lo + i * ((r_hi - r_lo) / n_bins);
+        thr[i] = e * e;
+    }
+    MDH_REQUIRE(rdf_filter_configure(R, thr.data(), sqrt_err), MDH_EINVAL,
+                "filter_window: the configuration is not eligible for the fp32 filter");
+    // per-frame boxes as mdh_rdf_accumulate builds them
+    std::vector<FrameBox> boxes(n_frames);
+    for (int f = 0; f < n_frames; ++f)
+        for (int k = 0; k < 3; ++k) {
+            const float b = box[3 * f + k];
+            MDH_REQUIRE(b > FLT_EPSILON && std::isfinite(b), MDH_EINVAL,
+                        "filter_window: box edge %d of frame %d is not a positive length", k, f);
+            boxes[f].box[k] = (double)b;
+            boxes[f].inv[k] = (double)(float)(1.0 / (double)b);
+        }
+    const FilterConst fca = filter_plan(R, boxes.data(), n_frames, sqrt_err);
+    for (int q = 0; q < 2; ++q) {
+        const FilterConst &fc = q ? fca : R.fc;
+        const double v[12] = {(double)fc.k,  (double)fc.scale, fc.offbase,          (double)fc.cbits,
+                              (double)fc.span, (double)fc.lg,  (double)fc.cb,       (double)fc.hslots,
+                              (double)fc.lo, (double)fc.unclamped, (double)fc.sb, (double)fc.lower};
+        for (int i = 0; i < 12; ++i) layout[12 * q + i] = v[i];
+    }
+    const FilterPrep qa = filter_prep_allpairs(R, fca, sqrt_err);
+    const FilterPrep qc = rdf_filter_prep(R, sqrt_err);     // cell lists: rint form, clamped
+    for (int f = 0; f < n_frames; ++f) {
+        unsigned k1[6], k2[6];
+        for (int i = 0; i < 6; ++i) {
+            const unsigned b1 = f32_bits(ext1[6 * f + i]), b2 = f32_bits(ext2[6 * f + i]);
+            k1[i] = (b1 & 0x80000000u) ? ~b1 : (b1 | 0x80000000u);   // rdf_device.cuh::ext_key
+            k2[i] = (b2 & 0x80000000u) ? ~b2 : (b2 | 0x80000000u);
+        }
+        for (int q = 0; q < 2; ++q) {
+            double mu = 0.0;
+            const FrameFilter ff = filter_prepare_frame(boxes[f], k1, k2, q ? qc : qa, &mu);
+            double *o = frames + 10 * f + 5 * q;
+            o[0] = (double)ff.offm;
+            o[1] = (double)ff.wlim;
+            o[2] = (double)ff.halfbox;
+            o[3] = (double)ff.unclamped;
+            o[4] = mu;
+        }
+    }
+    return MDH_OK;
 }
