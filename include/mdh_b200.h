@@ -324,6 +324,17 @@ int mdh_sq_tiling(mdh_ctx *ctx, int64_t *stats /* [4] host */);
  * wavevector set has columns without a compatible partner). */
 int mdh_sq_plan(int n_q, const int32_t *lattice_n /* [n_q][3] */, int64_t *stats /* [6] */,
                 int32_t *coverage /* [n_q] or NULL */, int32_t *pair_rule_violations);
+/* Per-warp report of the same planning (host only): counts[0] = warp items of the
+ * MDH_SQ_LATTICE_DMMA plan (padded to whole blocks of stats[4] warps), counts[1] = warps of
+ * the MDH_SQ_LATTICE_FP64 / _FP32 plan.  mma_items[i] (optional) = {nt0, nt1, t0, padding}
+ * of DMMA item i: the nz tiles of its two column groups (the kernel instance it runs), its
+ * first nz tile, 1 for an item without work.  lattice_warps[w] (optional) = the number of
+ * nz terms R (1..8, 0: padding) warp w of the scalar kernel runs.  At most cap entries of
+ * each array are written; counts are always complete. */
+int mdh_sq_plan_items(int n_q, const int32_t *lattice_n /* [n_q][3] */,
+                      int32_t *mma_items /* [cap][4] or NULL */,
+                      int32_t *lattice_warps /* [cap] or NULL */, int64_t cap,
+                      int64_t *counts /* [2] */);
 int mdh_sq_reset(mdh_ctx *ctx);
 int mdh_sq_accum_device(mdh_ctx *ctx, void **dptr);
 /* rho(q) of the LAST frame of the last batch: [n_rho][n_q][2] (re, im), n_rho =

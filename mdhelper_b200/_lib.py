@@ -67,6 +67,7 @@ SIGNATURES = {
     "mdh_sq_kernel": (_i32, [_p, _p]),
     "mdh_sq_tiling": (_i32, [_p, _p]),
     "mdh_sq_plan": (_i32, [_i32, _p, _p, _p, _p]),
+    "mdh_sq_plan_items": (_i32, [_i32, _p, _p, _p, _i64, _p]),
     "mdh_sq_reset": (_i32, [_p]),
     "mdh_sq_accum_device": (_i32, [_p, ctypes.POINTER(_p)]),
     "mdh_sq_fetch_rho": (_i32, [_p, _p]),
@@ -142,6 +143,22 @@ def sq_plan(lattice_n) -> dict:
     return {"items": stats[0], "tiles": stats[1], "max_scheduler_tiles": stats[2],
             "schedulers": stats[3], "warps_per_block": stats[4], "smem_bytes": stats[5],
             "coverage": cover, "pair_rule_violations": bad.value}
+
+
+def sq_plan_items(lattice_n) -> dict:
+    """Per-warp report of both lattice plans for ``lattice_n`` (``mdh_sq_plan_items``; no
+    device needed): ``mma`` is ``[items, 4]`` of ``(nt0, nt1, t0, padding)`` per warp item
+    of the DMMA kernel -- ``(nt0, nt1)`` names the ``sq_mma_consume`` instance it runs --,
+    ``lattice_r`` the number of nz terms ``R`` per warp of the scalar kernel (0: padding)."""
+    ln = np.ascontiguousarray(lattice_n, dtype=np.int32).reshape(-1, 3)
+    counts = np.zeros(2, dtype=np.int64)
+    check(lib().mdh_sq_plan_items(len(ln), ln.ctypes.data, None, None, 0, counts.ctypes.data))
+    cap = int(counts.max())
+    mma = np.zeros((cap, 4), dtype=np.int32)
+    r = np.zeros(cap, dtype=np.int32)
+    check(lib().mdh_sq_plan_items(len(ln), ln.ctypes.data, mma.ctypes.data, r.ctypes.data,
+                                  cap, counts.ctypes.data))
+    return {"mma": mma[:counts[0]], "lattice_r": r[:counts[1]]}
 
 
 def stage_plan(n_frames: int, bytes_per_frame: float, copy_over_kernel: float = 0.0) -> list:

@@ -506,6 +506,12 @@ int mdh_sq_plan(int n_q, const int32_t *lattice_n, int64_t *stats, int32_t *cove
     return sq_plan_impl(n_q, lattice_n, stats, coverage, pair_rule_violations);
 }
 
+int mdh_sq_plan_items(int n_q, const int32_t *lattice_n, int32_t *mma_items,
+                      int32_t *lattice_warps, int64_t cap, int64_t *counts)
+{
+    return sq_plan_items_impl(n_q, lattice_n, mma_items, lattice_warps, cap, counts);
+}
+
 int mdh_sq_tiling(mdh_ctx *c, int64_t *stats)
 {
     MDH_REQUIRE(c && stats, MDH_EINVAL, "NULL argument");

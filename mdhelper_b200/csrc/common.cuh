@@ -324,6 +324,8 @@ int com_reduce_f64_impl(mdh_ctx *c, int slot, const float *pos, int64_t stride, 
 int sq_configure_chains_impl(mdh_ctx *c, int64_t n_chains, int64_t n_monomers);
 int sq_plan_impl(int n_q, const int32_t *lat_n, int64_t *stats, int32_t *coverage,
                  int32_t *pair_rule_violations);
+int sq_plan_items_impl(int n_q, const int32_t *lat_n, int32_t *mma, int32_t *lattice_r,
+                       int64_t cap, int64_t *counts);
 int isf_configure_impl(mdh_ctx *c, int n_lags, int incoherent, int64_t max_frames);
 int isf_accumulate_f64_impl(mdh_ctx *c, const double *pos, int64_t stride, int location,
                             int n_frames);

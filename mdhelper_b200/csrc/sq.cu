@@ -1043,6 +1043,53 @@ static void mma_build_items(std::vector<Column> cols, const int (&nm)[3],
     (void)nm;
 }
 
+// Work items of sq_lattice_kernel: columns sorted by their number of wavevectors (cols is
+// reordered); thread tiles take two neighbouring columns (similar lengths) and one segment
+// of kSqTN nz values.  Items are padded to whole blocks of `block` consumer threads.
+static void lattice_build_items(std::vector<Column> &cols, const int (&nm)[3],
+                                std::vector<SqWorkItem> &items, std::vector<int> &qidx,
+                                int &block)
+{
+    std::stable_sort(cols.begin(), cols.end(), [](const Column &a, const Column &b) {
+        return column_top(a) > column_top(b);
+    });
+    const int n_seg = (nm[2] + kSqTN) / kSqTN;
+    for (int s = 0; s < n_seg; ++s)
+        for (size_t c0 = 0; c0 < cols.size(); c0 += kSqTM) {
+            SqWorkItem it{};
+            it.nz0 = s * kSqTN;
+            std::vector<int> qi(kSqTM * kSqTN, -1);
+            bool any = false;
+            for (int m = 0; m < kSqTM; ++m) {
+                if (c0 + m >= cols.size()) continue;
+                const Column &c = cols[c0 + m];
+                it.nx[m] = c.nx; it.ny[m] = c.ny;
+                for (int r = 0; r < kSqTN; ++r) {
+                    const int z = it.nz0 + r;
+                    if (z < (int)c.q.size() && c.q[z] >= 0) {
+                        qi[m * kSqTN + r] = c.q[z];
+                        it.len[m] = r + 1;
+                        any = true;
+                    }
+                }
+            }
+            if (!any) continue;
+            items.push_back(it);
+            qidx.insert(qidx.end(), qi.begin(), qi.end());
+        }
+    // consumer threads per block: whole warps, at most kSqThreads minus the
+    // producer warps; items padded to whole blocks
+    const int max_cons = kSqThreads - kSqProducers;
+    const int n_warps = (int)((items.size() + 31) / 32);
+    const int n_blocks = (n_warps * 32 + max_cons - 1) / max_cons;
+    block = ((n_warps + n_blocks - 1) / n_blocks) * 32;
+    block = std::max(block, 32);
+    while (items.size() % block) {
+        items.push_back(SqWorkItem{});
+        qidx.insert(qidx.end(), kSqTM * kSqTN, -1);
+    }
+}
+
 }  // namespace
 
 // Device-free planning of the DMMA kernel's work items (what mdh_sq_configure builds for
@@ -1081,6 +1128,47 @@ int sq_plan_impl(int n_q, const int32_t *lat_n, int64_t *stats, int32_t *coverag
             }
         *pair_rule_violations = bad;
     }
+    return MDH_OK;
+}
+
+// Per-warp report of both lattice plans (what mdh_sq_configure builds); see
+// mdh_sq_plan_items in the header.
+int sq_plan_items_impl(int n_q, const int32_t *lat_n, int32_t *mma, int32_t *lattice_r,
+                       int64_t cap, int64_t *counts)
+{
+    MDH_REQUIRE(n_q >= 1 && lat_n && counts && cap >= 0, MDH_EINVAL,
+                "sq plan items: missing argument");
+    int nm[3];
+    std::vector<Column> cols;
+    MDH_REQUIRE(build_columns(n_q, lat_n, nm, cols), MDH_EINVAL,
+                "sq plan items: wavevector indices are not usable by the lattice kernels");
+    std::vector<SqMmaItem> mitems;
+    std::vector<int> mqidx;
+    int warps = 0, st[4] = {0, 0, 0, 0};
+    mma_build_items(cols, nm, mitems, mqidx, warps, st);
+    std::vector<SqWorkItem> items;
+    std::vector<int> qidx;
+    int block = 0;
+    lattice_build_items(cols, nm, items, qidx, block);
+    counts[0] = (int64_t)mitems.size();
+    counts[1] = (int64_t)(items.size() / 32);
+    if (mma)
+        for (int64_t s = 0; s < std::min<int64_t>(cap, counts[0]); ++s) {
+            const SqMmaItem &it = mitems[s];
+            // the kernel dispatches on (nt[0], nt[kMmaG - 1]); no tiles: an idle warp
+            mma[4 * s + 0] = it.nt[0];
+            mma[4 * s + 1] = kMmaG > 1 ? it.nt[kMmaG - 1] : 0;
+            mma[4 * s + 2] = it.t0;
+            mma[4 * s + 3] = it.nt[0] == 0;
+        }
+    if (lattice_r)
+        for (int64_t w = 0; w < std::min<int64_t>(cap, counts[1]); ++w) {
+            // sq_lattice_kernel's warp-uniform R: the longest column segment of the warp
+            int r = 0;
+            for (int l = 0; l < 32; ++l)
+                for (int m = 0; m < kSqTM; ++m) r = std::max(r, items[32 * w + l].len[m]);
+            lattice_r[w] = r;
+        }
     return MDH_OK;
 }
 
@@ -1130,9 +1218,7 @@ int sq_configure_impl(mdh_ctx *c, int64_t n_total, int n_groups, const int64_t *
     S.rho_frames = 0;
     S.n_chains = S.n_monomers = 0;
 
-    // ---- lattice work items ----
-    // Columns (nx, ny) sorted by their number of wavevectors; thread tiles take two
-    // neighbouring columns (similar lengths) and one segment of kSqTN nz values.
+    // ---- lattice work items (lattice_build_items) ----
     bool lattice = lat_n && lat_b && mode != MDH_SQ_GENERAL_FP64;
     std::vector<SqWorkItem> items;
     std::vector<int> qidx;
@@ -1144,45 +1230,7 @@ int sq_configure_impl(mdh_ctx *c, int64_t n_total, int n_groups, const int64_t *
         std::vector<Column> cols;
         lattice = build_columns(n_q, lat_n, nm, cols);
         if (lattice) {
-            auto top = column_top;
-            std::stable_sort(cols.begin(), cols.end(),
-                             [&](const Column &a, const Column &b) { return top(a) > top(b); });
-            const int n_seg = (nm[2] + kSqTN) / kSqTN;
-            for (int s = 0; s < n_seg; ++s)
-                for (size_t c0 = 0; c0 < cols.size(); c0 += kSqTM) {
-                    SqWorkItem it{};
-                    it.nz0 = s * kSqTN;
-                    std::vector<int> qi(kSqTM * kSqTN, -1);
-                    bool any = false;
-                    for (int m = 0; m < kSqTM; ++m) {
-                        if (c0 + m >= cols.size()) continue;
-                        const Column &c = cols[c0 + m];
-                        it.nx[m] = c.nx; it.ny[m] = c.ny;
-                        for (int r = 0; r < kSqTN; ++r) {
-                            const int z = it.nz0 + r;
-                            if (z < (int)c.q.size() && c.q[z] >= 0) {
-                                qi[m * kSqTN + r] = c.q[z];
-                                it.len[m] = r + 1;
-                                any = true;
-                            }
-                        }
-                    }
-                    if (!any) continue;
-                    items.push_back(it);
-                    qidx.insert(qidx.end(), qi.begin(), qi.end());
-                }
-            // consumer threads per block: whole warps, at most kSqThreads minus the
-            // producer warps; items padded to whole blocks
-            const int max_cons = kSqThreads - kSqProducers;
-            const int n_warps = (int)((items.size() + 31) / 32);
-            const int n_blocks = (n_warps * 32 + max_cons - 1) / max_cons;
-            int block = ((n_warps + n_blocks - 1) / n_blocks) * 32;
-            block = std::max(block, 32);
-            S.block = block;
-            while (items.size() % block) {
-                items.push_back(SqWorkItem{});
-                qidx.insert(qidx.end(), kSqTM * kSqTN, -1);
-            }
+            lattice_build_items(cols, nm, items, qidx, S.block);
             for (int k = 0; k < 3; ++k) { S.nmax[k] = nm[k]; S.b[k] = lat_b[k]; }
 
             // ---- DMMA work items (sq_lattice_mma_kernel) ----
