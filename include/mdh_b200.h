@@ -261,6 +261,17 @@ int mdh_rdf_set_prewrap(mdh_ctx *ctx, int mode);
  * declined (left to the exact kernel), stats[5] 1 if the current configuration is
  * eligible for the filter.  Since the last configure / reset. */
 int mdh_rdf_filter_stats(mdh_ctx *ctx, int64_t *stats /* [6] host */);
+/* How the configured run bins its fp64 squared distances: out[0] 1 if the kernels use the
+ * branch-free bin guess (FAST instances), 0 if they use the binary search; out[1] the
+ * disagreements the configure-time self-check of the guess found (the guess is used only
+ * when there are none). */
+int mdh_rdf_bin_lookup(mdh_ctx *ctx, int64_t *out /* [2] host */);
+/* Checks the bin guess of the configured thresholds against the binary search for every
+ * double d2 >= 0, +inf and NaN, whether or not the run uses it (one kernel; synchronises).
+ * out[0] classes of d2 on which the guess is constant (each checked at both ends), out[1]
+ * disagreements (0: the guess is exact for this configuration), out[2] the bits of the
+ * smallest d2 that disagrees (-1: none), out[3] its fast slot minus its exact slot. */
+int mdh_rdf_bin_guess_audit(mdh_ctx *ctx, int64_t *out /* [4] host */);
 /* frames[0] frames the all-pairs filter kernel evaluated with the half-box minimum image
  * (every coordinate difference within 1.5 box lengths), frames[1] frames it evaluated
  * with the rint form.  Since the last configure / reset. */

@@ -58,6 +58,8 @@ SIGNATURES = {
     "mdh_rdf_set_filter": (_i32, [_p, _i32]),
     "mdh_rdf_set_prewrap": (_i32, [_p, _i32]),
     "mdh_rdf_filter_stats": (_i32, [_p, _p]),
+    "mdh_rdf_bin_lookup": (_i32, [_p, _p]),
+    "mdh_rdf_bin_guess_audit": (_i32, [_p, _p]),
     "mdh_rdf_filter_modes": (_i32, [_p, _p]),
     "mdh_rdf_filter_unclamped": (_i32, [_p, _p]),
     "mdh_sq_configure": (_i32, [_p, _i64, _i32, _p, _i32, _p, _p, _p, _i32, _p, _i32]),
@@ -355,6 +357,21 @@ class Context:
                          "audit_uncertain_pairs", "declined_frames", "eligible",
                          "halfbox_frames", "rint_frames", "unclamped_frames"),
                         (int(v) for v in out)))
+
+    def rdf_bin_lookup(self) -> dict:
+        """Which bin lookup the configured run uses (``fast``: the branch-free guess, else the
+        binary search) and the disagreements of its configure-time self-check."""
+        out = np.zeros(2, dtype=np.int64)
+        check(self._lib.mdh_rdf_bin_lookup(self._h, out.ctypes.data))
+        return {"fast": int(out[0]), "selfcheck_bad": int(out[1])}
+
+    def rdf_bin_guess_audit(self) -> dict:
+        """The bin guess of the configured thresholds checked for every d2 >= 0, inf and NaN
+        (``mdh_rdf_bin_guess_audit``): classes checked, disagreements, the bits of the
+        smallest bad d2 (-1: none) and its fast slot minus its exact slot."""
+        out = np.zeros(4, dtype=np.int64)
+        check(self._lib.mdh_rdf_bin_guess_audit(self._h, out.ctypes.data))
+        return dict(zip(("classes", "bad", "first_bits", "slot_diff"), (int(v) for v in out)))
 
     def rdf_pair_evaluations(self) -> int:
         n = _i64()

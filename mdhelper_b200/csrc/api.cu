@@ -430,6 +430,23 @@ int mdh_rdf_filter_stats(mdh_ctx *c, int64_t *stats)
     return MDH_OK;
 }
 
+int mdh_rdf_bin_lookup(mdh_ctx *c, int64_t *out)
+{
+    CTX_GUARD(c);
+    MDH_REQUIRE(out != nullptr, MDH_EINVAL, "out is NULL");
+    MDH_REQUIRE(c->rdf.configured, MDH_ESTATE, "rdf: not configured");
+    out[0] = c->rdf.fast_bins ? 1 : 0;
+    out[1] = c->rdf.selfcheck_bad;
+    return MDH_OK;
+}
+
+int mdh_rdf_bin_guess_audit(mdh_ctx *c, int64_t *out)
+{
+    CTX_GUARD(c);
+    MDH_REQUIRE(out != nullptr, MDH_EINVAL, "out is NULL");
+    return rdf_bin_guess_audit_impl(c, out);
+}
+
 int mdh_rdf_filter_modes(mdh_ctx *c, int64_t *frames)
 {
     CTX_GUARD(c);

@@ -125,6 +125,7 @@ struct RdfState {
     int64_t evals = 0;     // all-pairs evaluations (host-side count)
     int ipt = 2;           // i-particles per thread of the all-pairs kernel
     bool fast_bins = false;  // branch-free bin guess certified for this configuration
+    int selfcheck_bad = 0;   // disagreements rdf_selfcheck_kernel found at configure time
     // fp32 filter in front of the exact arithmetic (rdf_filter.cu)
     int prewrap_mode = MDH_WRAP_AUTO;    // survives configure
     int filter_mode = MDH_FILTER_AUTO;   // survives configure
@@ -292,6 +293,7 @@ int rdf_configure_impl(mdh_ctx *c, int64_t n1, int64_t n2, int same, int n_bins,
                        int drop_axis, int mode, int hist);
 int rdf_accumulate_impl(mdh_ctx *c, const float *pos1, int64_t s1, const float *pos2,
                         int64_t s2, int location, const float *box, int n_frames);
+int rdf_bin_guess_audit_impl(mdh_ctx *c, int64_t *out);
 // rdf_tri.cu
 int rdf_accumulate_triclinic_impl(mdh_ctx *c, const float *pos1, int64_t s1, const float *pos2,
                                   int64_t s2, int location, const float *box9, int n_frames);

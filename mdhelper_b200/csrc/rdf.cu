@@ -322,6 +322,7 @@ int rdf_configure_impl(mdh_ctx *c, int64_t n1, int64_t n2, int same, int n_bins,
     c->launches++;
     MDH_CUDA(cudaMemcpyAsync(&h_bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     MDH_CUDA(cudaStreamSynchronize(c->stream));   // also: t is a local
+    R.selfcheck_bad = h_bad;
     R.fast_bins = allow_fast && h_bad == 0;
 
     // fp32 filter: needs the 4-particle tile, the shared-atomic histogram layout and
@@ -332,6 +333,49 @@ int rdf_configure_impl(mdh_ctx *c, int64_t n1, int64_t n2, int same, int n_bins,
         rdf_filter_configure(R, thr, g_sqrt_err_cached);
     }
     R.configured = true;
+    return MDH_OK;
+}
+
+// Exhaustive check of the configured thresholds and bin guess (rdf_guess_audit_kernel):
+// out = {classes checked, disagreements, bits of the smallest bad d2 (-1: none), its fast
+// slot minus its exact slot}.
+int rdf_bin_guess_audit_impl(mdh_ctx *c, int64_t *out)
+{
+    RdfState &R = c->rdf;
+    MDH_REQUIRE(R.configured, MDH_ESTATE, "rdf: bin guess audit before configure");
+    DevBuf buf;
+    if (int rc = buf.reserve(2 * sizeof(unsigned long long) + sizeof(int))) return rc;
+    unsigned long long *d_out = buf.as<unsigned long long>();
+    const unsigned long long init[2] = {0ull, ~0ull};
+    MDH_CUDA(cudaMemcpyAsync(d_out, init, sizeof(init), cudaMemcpyHostToDevice, c->stream));
+    const BinGuess g = rdf_bin_guess(R);
+    const size_t smem = sizeof(double) * (R.n_bins + 1);
+    MDH_CUDA(cudaFuncSetAttribute(rdf_guess_audit_kernel,
+                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    rdf_guess_audit_kernel<<<c->sm_count * 8, 256, smem, c->stream>>>(R.thr.as<double>(),
+                                                                       R.n_bins, g, d_out);
+    MDH_CUDA(cudaGetLastError());
+    c->launches++;
+    unsigned long long h[2];
+    MDH_CUDA(cudaMemcpyAsync(h, d_out, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
+    MDH_CUDA(cudaStreamSynchronize(c->stream));
+    int diff = 0;
+    if (h[0]) {
+        int *d_diff = reinterpret_cast<int *>(d_out + 2);
+        double d2;
+        memcpy(&d2, &h[1], sizeof(d2));
+        rdf_guess_probe_kernel<<<1, 1, 0, c->stream>>>(R.thr.as<double>(), R.n_bins, g, d2,
+                                                       d_diff);
+        MDH_CUDA(cudaGetLastError());
+        c->launches++;
+        MDH_CUDA(cudaMemcpyAsync(&diff, d_diff, sizeof(int), cudaMemcpyDeviceToHost,
+                                 c->stream));
+        MDH_CUDA(cudaStreamSynchronize(c->stream));
+    }
+    out[0] = kGuessClasses;
+    out[1] = (int64_t)h[0];
+    out[2] = h[0] ? (int64_t)h[1] : -1;
+    out[3] = diff;
     return MDH_OK;
 }
 

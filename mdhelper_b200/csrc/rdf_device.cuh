@@ -270,6 +270,66 @@ static __global__ void rdf_selfcheck_kernel(const double *__restrict__ thr, int 
     if (wrong) atomicAdd(bad, wrong);
 }
 
+// Checks slot_fast for one configuration over EVERY double d2 >= 0 (certified or not).
+// slot_fast_parts builds its float from the clamped hi word and the top 3 bits of the lo
+// word, so the guess j is constant on each of kGuessClasses classes (hi in [kGuessHiMin,
+// kGuessHiMax], lo >> 29); slot_search is monotone in d2 and the compare against T[j] is
+// exact, so slot_fast is right on a whole class iff it is right at the class's smallest
+// and largest d2.  The clamped end classes absorb every d2 below 2^-127 (from 0 up) and
+// every finite d2 above 2^127; +inf and NaN (both signs, every lo >> 29) are checked
+// separately.  out[0] += disagreements, out[1] = min(out[1], bits of a bad d2).
+constexpr unsigned kGuessHiMin = 0x38000000u, kGuessHiMax = 0x47e00000u;
+constexpr long long kGuessClasses = ((long long)(kGuessHiMax - kGuessHiMin) + 1) * 8;
+
+static __global__ void __launch_bounds__(256)
+    rdf_guess_audit_kernel(const double *__restrict__ thr, int n_bins, BinGuess g,
+                           unsigned long long *out)
+{
+    extern __shared__ double sTa[];
+    for (int k = threadIdx.x; k <= n_bins; k += blockDim.x) sTa[k] = thr[k];
+    __syncthreads();
+    unsigned long long bad = 0, first = ~0ull;
+    auto check = [&](unsigned long long bits) {
+        const double d2 = __longlong_as_double((long long)bits);
+        if (slot_fast(d2, sTa, n_bins, g) != slot_search(d2, sTa, n_bins)) {
+            ++bad;
+            first = min(first, bits);
+        }
+    };
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x; c < kGuessClasses;
+         c += stride) {
+        const unsigned long long hi = kGuessHiMin + (unsigned long long)(c >> 3);
+        const unsigned long long t = (unsigned long long)(c & 7) << 29;
+        const unsigned long long hi_min = hi == kGuessHiMin ? 0ull : hi;
+        const unsigned long long hi_max = hi == kGuessHiMax ? 0x7fefffffull : hi;
+        check((hi_min << 32) | t);
+        check((hi_max << 32) | t | 0x1fffffffull);
+    }
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        check(0x7ff0000000000000ull);                                  // +inf
+        for (unsigned long long t = 0; t < 8; ++t) {
+            check(0x7ff8000000000000ull | (t << 29));                  // NaN
+            check(0xfff8000000000000ull | (t << 29));
+        }
+    }
+    for (int o = 16; o; o >>= 1) {
+        bad += __shfl_xor_sync(0xffffffffu, bad, o);
+        first = min(first, __shfl_xor_sync(0xffffffffu, first, o));
+    }
+    if ((threadIdx.x & 31) == 0 && bad) {
+        atomicAdd(&out[0], bad);
+        atomicMin(&out[1], first);
+    }
+}
+
+// fast slot minus exact slot of one d2 (the audit's first disagreement)
+static __global__ void rdf_guess_probe_kernel(const double *__restrict__ thr, int n_bins,
+                                              BinGuess g, double d2, int *diff)
+{
+    *diff = slot_fast(d2, thr, n_bins, g) - slot_search(d2, thr, n_bins);
+}
+
 // ---- shared-memory layout and histogram privatisation ------------------------------
 
 // Per-warp u32 histogram for the shared-atomic scheme: one pad word (receives the

@@ -6,6 +6,8 @@ minimum bit for bit."""
 import numpy as np
 import pytest
 
+from _threshold_pairs import image_d2 as _image_d2, wrap as _wrap
+
 U8 = 60          # kTriShiftMax
 
 
@@ -27,19 +29,6 @@ def _widths(h):
                      vol / np.linalg.norm(np.cross(a, b))])
 
 
-def _wrap(p, h):
-    """tri_wrap_kernel: along c, then b, then a, in double, rounded to float32."""
-    ax, bx, by, cx, cy, cz = (float(h[0, 0]), float(h[1, 0]), float(h[1, 1]), float(h[2, 0]),
-                              float(h[2, 1]), float(h[2, 2]))
-    x, y, z = (p[:, k].astype(np.float64) for k in range(3))
-    s = np.floor(z / cz)
-    x, y, z = x - s * cx, y - s * cy, z - s * cz
-    s = np.floor(y / by)
-    x, y = x - s * bx, y - s * by
-    x = x - np.floor(x / ax) * ax
-    return np.stack([x, y, z], 1).astype(np.float32)
-
-
 def _tri_cell(p, h, nc):
     """tri_cell: fractional coordinates, cell per axis, lattice shift k = -floor(s)."""
     ax, bx, by, cx, cy, cz = (float(h[0, 0]), float(h[1, 0]), float(h[1, 1]), float(h[2, 0]),
@@ -54,16 +43,6 @@ def _tri_cell(p, h, nc):
         c.append(np.clip(((s - f) * float(n)).astype(np.int64), 0, n - 1))
         k.append(np.clip(-f, -U8, U8).astype(np.int64))
     return np.stack(c, 1), np.stack(k, 1)
-
-
-def _image_d2(dx, h, m):
-    """tri_image_d2 with the shift terms h_k * i."""
-    h = h.astype(np.float64)
-    ix, iy, iz = (m[..., k].astype(np.float64) for k in range(3))
-    rx = ((dx[..., 0] + h[0, 0] * ix) + h[1, 0] * iy) + h[2, 0] * iz
-    ry = (dx[..., 1] + h[1, 1] * iy) + h[2, 1] * iz
-    rz = dx[..., 2] + h[2, 2] * iz
-    return (rx * rx + ry * ry) + rz * rz
 
 
 def _check(h, r_hi, p):
