@@ -280,6 +280,11 @@ int mdh_rdf_filter_modes(mdh_ctx *ctx, int64_t *frames /* [2] host */);
  * (its block histogram has a word for every slot the frame can reach; a subset of
  * mdh_rdf_filter_modes' frames[0]).  Since the last configure / reset. */
 int mdh_rdf_filter_unclamped(mdh_ctx *ctx, int64_t *frames /* [1] host */);
+/* pairs[0] pairs the all-pairs filter kernel evaluated in x-clean tile pairs: the groups are
+ * sorted by x, and a tile pair whose x differences all share one periodic image takes the
+ * x component of the minimum image as one subtraction (unclamped half-box frames only).
+ * Since the last configure / reset. */
+int mdh_rdf_filter_cleanx(mdh_ctx *ctx, int64_t *pairs /* [1] host */);
 
 /* ---- seam #2: direct-sum structure factor ------------------------------------ */
 

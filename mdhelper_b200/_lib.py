@@ -62,6 +62,7 @@ SIGNATURES = {
     "mdh_rdf_bin_guess_audit": (_i32, [_p, _p]),
     "mdh_rdf_filter_modes": (_i32, [_p, _p]),
     "mdh_rdf_filter_unclamped": (_i32, [_p, _p]),
+    "mdh_rdf_filter_cleanx": (_i32, [_p, _p]),
     "mdh_sq_configure": (_i32, [_p, _i64, _i32, _p, _i32, _p, _p, _p, _i32, _p, _i32]),
     "mdh_sq_accumulate": (_i32, [_p, _p, _i64, _i32, _i32]),
     "mdh_sq_accumulate_f64": (_i32, [_p, _p, _i64, _i32, _i32]),
@@ -349,13 +350,15 @@ class Context:
         check(self._lib.mdh_rdf_set_prewrap(self._h, WRAP_MODES[mode]))
 
     def rdf_filter_stats(self) -> dict:
-        out = np.zeros(9, dtype=np.int64)
+        out = np.zeros(10, dtype=np.int64)
         check(self._lib.mdh_rdf_filter_stats(self._h, out[:6].ctypes.data))
         check(self._lib.mdh_rdf_filter_modes(self._h, out[6:8].ctypes.data))
-        check(self._lib.mdh_rdf_filter_unclamped(self._h, out[8:].ctypes.data))
+        check(self._lib.mdh_rdf_filter_unclamped(self._h, out[8:9].ctypes.data))
+        check(self._lib.mdh_rdf_filter_cleanx(self._h, out[9:].ctypes.data))
         return dict(zip(("deferred_entries", "inline_entries", "audit_violations",
                          "audit_uncertain_pairs", "declined_frames", "eligible",
-                         "halfbox_frames", "rint_frames", "unclamped_frames"),
+                         "halfbox_frames", "rint_frames", "unclamped_frames",
+                         "cleanx_pairs"),
                         (int(v) for v in out)))
 
     def rdf_bin_lookup(self) -> dict:

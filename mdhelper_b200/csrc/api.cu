@@ -372,7 +372,7 @@ int mdh_rdf_reset(mdh_ctx *c)
     if (c->rdf.evals_dev_init)
         MDH_CUDA(cudaMemsetAsync(c->rdf.cell[9].p, 0, sizeof(unsigned long long), c->stream));
     if (c->rdf.fstats.p)
-        MDH_CUDA(cudaMemsetAsync(c->rdf.fstats.p, 0, sizeof(unsigned long long) * 8, c->stream));
+        MDH_CUDA(cudaMemsetAsync(c->rdf.fstats.p, 0, sizeof(unsigned long long) * 9, c->stream));
     c->rdf.evals = 0;
     return MDH_OK;
 }
@@ -469,6 +469,18 @@ int mdh_rdf_filter_unclamped(mdh_ctx *c, int64_t *frames)
     MDH_CUDA(cudaMemcpyAsync(h, c->rdf.fstats.p, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
     MDH_CUDA(cudaStreamSynchronize(c->stream));
     frames[0] = (int64_t)h[7];
+    return MDH_OK;
+}
+
+int mdh_rdf_filter_cleanx(mdh_ctx *c, int64_t *pairs)
+{
+    CTX_GUARD(c);
+    MDH_REQUIRE(pairs != nullptr, MDH_EINVAL, "pairs is NULL");
+    MDH_REQUIRE(c->rdf.configured, MDH_ESTATE, "rdf: not configured");
+    unsigned long long h[9] = {0};
+    MDH_CUDA(cudaMemcpyAsync(h, c->rdf.fstats.p, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
+    MDH_CUDA(cudaStreamSynchronize(c->stream));
+    pairs[0] = (int64_t)h[8];
     return MDH_OK;
 }
 

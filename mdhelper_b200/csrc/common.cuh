@@ -135,7 +135,10 @@ struct RdfState {
     FilterConst fca;       // the all-pairs filter kernel's layout for the current batch
     DevBuf ext1, ext2;     // unsigned[F][6]: coordinate extents of each frame (keys)
     DevBuf filt;           // FrameFilter[F]
-    DevBuf fstats;         // unsigned long long[8], see PairParams::fstats
+    DevBuf fstats;         // unsigned long long[9], see PairParams::fstats
+    DevBuf xsort;          // float4[F][npad]: packed rows before the x-sort (rdf_xsort_kernel)
+    DevBuf tx1, tx2;       // float2[F][tiles]: x extents of the tiles of the x-sorted groups
+    DevBuf xform;          // unsigned char[F][i-tiles][j-tiles]: x form of every tile pair
 };
 
 struct SqWorkItem {        // one thread's tile of the lattice kernels: two (nx, ny)

@@ -47,6 +47,94 @@ __host__ __device__ inline size_t pair_smem_bytes(int n_bins)
            hist_smem_bytes<HIST>(n_bins);
 }
 
+// ---- x-sorted groups for the all-pairs filter kernel -------------------------------
+// One block per frame: a counting sort of the frame's packed rows by an x-slab key
+// (kXSlabs slabs over the frame's x extent), then the x extent of every tile of `tile`
+// rows.  Rows keep their tags (.w), so exclusions and same-group runs see the same pairs;
+// the order within a slab is whatever the shared-memory atomics give (the counts do not
+// depend on the order of the rows).  Padding rows are copied as they are.
+constexpr int kXSlabs = 1024;
+
+__global__ void __launch_bounds__(1024)
+    rdf_xsort_kernel(const float4 *__restrict__ in, float4 *__restrict__ out, int64_t n,
+                     int64_t npad, const unsigned *__restrict__ ext, int tile,
+                     float2 *__restrict__ tx)
+{
+    __shared__ unsigned cnt[kXSlabs];
+    __shared__ unsigned wsum[32];
+    const int frame = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const float4 *src = in + (int64_t)frame * npad;
+    float4 *dst = out + (int64_t)frame * npad;
+    const float x0 = ext_unkey(ext[frame * 6]), x1 = ext_unkey(ext[frame * 6 + 3]);
+    // slab of x: NaN and a frame of width 0 (or inf) fall into slab 0 or the last one
+    const float inv = (float)kXSlabs / (x1 - x0);
+    auto slab = [&](float x) {
+        const float s = fminf(fmaxf((x - x0) * inv, 0.f), (float)(kXSlabs - 1));
+        return (int)s;
+    };
+    static_assert(kXSlabs == 1024, "one slab per thread in the scan");
+    cnt[tid] = 0;
+    __syncthreads();
+    for (int64_t i = tid; i < n; i += 1024) atomicAdd(&cnt[slab(src[i].x)], 1u);
+    __syncthreads();
+    // exclusive scan of the 1024 counts
+    const unsigned c = cnt[tid];
+    unsigned v = c;
+    for (int o = 1; o < 32; o <<= 1) {
+        const unsigned t = __shfl_up_sync(0xffffffffu, v, o);
+        if (lane >= o) v += t;
+    }
+    if (lane == 31) wsum[warp] = v;
+    __syncthreads();
+    if (warp == 0) {
+        unsigned w = wsum[lane];
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned t = __shfl_up_sync(0xffffffffu, w, o);
+            if (lane >= o) w += t;
+        }
+        wsum[lane] = w;
+    }
+    __syncthreads();
+    cnt[tid] = v - c + (warp ? wsum[warp - 1] : 0u);
+    __syncthreads();
+    for (int64_t i = tid; i < n; i += 1024) {
+        const float4 p = src[i];
+        dst[atomicAdd(&cnt[slab(p.x)], 1u)] = p;
+    }
+    for (int64_t i = n + tid; i < npad; i += 1024) dst[i] = src[i];
+    __syncthreads();          // the block's global writes are visible to the block
+    // x extent of every tile (rows below n), one warp per tile
+    const int n_tiles = (int)(npad / tile);
+    for (int t = warp; t < n_tiles; t += 32) {
+        unsigned lo = 0xffffffffu, hi = 0u;
+        const int64_t r1 = min((int64_t)(t + 1) * tile, n);
+        for (int64_t r = (int64_t)t * tile + lane; r < r1; r += 32) {
+            const unsigned k = ext_key(dst[r].x);
+            lo = min(lo, k);
+            hi = max(hi, k);
+        }
+        lo = __reduce_min_sync(0xffffffffu, lo);
+        hi = __reduce_max_sync(0xffffffffu, hi);
+        if (lane == 0) tx[(int64_t)frame * n_tiles + t] = make_float2(ext_unkey(lo), ext_unkey(hi));
+    }
+}
+
+// filter_cleanx_form of every tile pair (i-tile, j-tile) of every frame from the tile
+// extents tx1 [F][ni], tx2 [F][nj] of the sorted groups: out [F][ni][nj]
+__global__ void rdf_cleanx_forms_kernel(const float2 *__restrict__ tx1,
+                                               const float2 *__restrict__ tx2, int ni, int nj,
+                                               const FrameBox *__restrict__ boxes,
+                                               unsigned char *__restrict__ out)
+{
+    const int frame = blockIdx.y;
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= ni * nj) return;
+    const int a = q / nj, b = q - a * nj;
+    const float2 ti = tx1[(int64_t)frame * ni + a], tj = tx2[(int64_t)frame * nj + b];
+    out[(int64_t)frame * ni * nj + q] =
+        (unsigned char)filter_cleanx_form(ti.x, ti.y, tj.x, tj.y, (float)boxes[frame].box[0]);
+}
+
 template <int HIST, bool EXCL, bool FAST, int IPT>
 __global__ void __launch_bounds__(kThreads, 2) rdf_allpairs_kernel(const PairParams P)
 {
@@ -302,8 +390,8 @@ int rdf_configure_impl(mdh_ctx *c, int64_t n1, int64_t n2, int same, int n_bins,
     if (int rc = R.thr.reserve(sizeof(double) * (n_bins + 2))) return rc;
     if (int rc = R.counts.reserve(sizeof(unsigned long long) * n_bins)) return rc;
     if (int rc = R.cell[9].reserve(sizeof(unsigned long long) + sizeof(int))) return rc;
-    if (int rc = R.fstats.reserve(sizeof(unsigned long long) * 8)) return rc;
-    MDH_CUDA(cudaMemsetAsync(R.fstats.p, 0, sizeof(unsigned long long) * 8, c->stream));
+    if (int rc = R.fstats.reserve(sizeof(unsigned long long) * 9)) return rc;
+    MDH_CUDA(cudaMemsetAsync(R.fstats.p, 0, sizeof(unsigned long long) * 9, c->stream));
     std::vector<double> t(thr, thr + n_bins + 1);
     t.push_back(INFINITY);
     MDH_CUDA(cudaMemcpyAsync(R.thr.p, t.data(), sizeof(double) * t.size(),
@@ -380,10 +468,13 @@ int rdf_bin_guess_audit_impl(mdh_ctx *c, int64_t *out)
 }
 
 // host input: the copy into `raw` is queued on the stager's copy stream (the caller
-// brackets the group copies of a piece with stager.acquire / publish)
+// brackets the group copies of a piece with stager.acquire / publish).  tx (with ext): the
+// packed rows are sorted by x and tx receives the x extents of their tiles of `tile` rows
+// (rdf_xsort_kernel), for the x-clean tile pairs of the all-pairs filter kernel.
 static int rdf_upload_group(mdh_ctx *c, const float *pos, int64_t stride, int location,
                             int64_t n, int64_t npad, int64_t excl, int n_frames,
-                            DevBuf &raw, DevBuf &pk, DevBuf *ext, bool copy_only, int f0)
+                            DevBuf &raw, DevBuf &pk, DevBuf *ext, bool copy_only, int f0,
+                            DevBuf *tx = nullptr, int tile = 0)
 {
     RdfState &R = c->rdf;
     MDH_REQUIRE(pos != nullptr, MDH_EINVAL, "rdf: coordinate pointer is NULL");
@@ -413,12 +504,25 @@ static int rdf_upload_group(mdh_ctx *c, const float *pos, int64_t stride, int lo
         MDH_CUDA(cudaGetLastError());
         c->launches++;
     }
+    const bool sort = tx != nullptr && d_ext != nullptr;
+    if (sort) {
+        if (int rc = R.xsort.reserve(sizeof(float4) * npad * n_frames)) return rc;
+        if (int rc = tx->reserve(sizeof(float2) * (npad / tile) * n_frames)) return rc;
+    }
     dim3 grid((unsigned)std::min<int64_t>((npad + 255) / 256, 2048), n_frames);
-    rdf_pack_kernel<<<grid, 256, 0, c->stream>>>(dsrc, dstride, pk.as<float4>(), n, npad, excl,
-                                                 R.drop_axis, d_ext,
+    rdf_pack_kernel<<<grid, 256, 0, c->stream>>>(dsrc, dstride,
+                                                 (sort ? R.xsort : pk).as<float4>(), n, npad,
+                                                 excl, R.drop_axis, d_ext,
                                                  R.boxes.as<FrameBox>() + f0);
     MDH_CUDA(cudaGetLastError());
     c->launches++;
+    if (sort) {
+        rdf_xsort_kernel<<<n_frames, 1024, 0, c->stream>>>(R.xsort.as<float4>(), pk.as<float4>(),
+                                                           n, npad, d_ext, tile,
+                                                           tx->as<float2>());
+        MDH_CUDA(cudaGetLastError());
+        c->launches++;
+    }
     return MDH_OK;
 }
 
@@ -545,14 +649,16 @@ static int rdf_accumulate_piece(mdh_ctx *c, const float *pos1, int64_t s1, const
             if (int rc = c->stager.retire(c->stream, slot)) return rc;
         return MDH_OK;
     }
+    // the filter kernel's groups are sorted by x (x-clean tile pairs); the exact kernel
+    // reads the same sorted rows
     if (int rc = rdf_upload_group(c, pos1, s1, location, R.n1, pad1, R.excl1, n_frames,
                                   R.raw1[slot], R.pk1, use_filter ? &R.ext1 : nullptr, false,
-                                  f0))
+                                  f0, use_filter ? &R.tx1 : nullptr, tile))
         return rc;
     if (!R.same)
         if (int rc = rdf_upload_group(c, pos2, s2, location, R.n2, pad2, R.excl2, n_frames,
                                       R.raw2[slot], R.pk2, use_filter ? &R.ext2 : nullptr,
-                                      false, f0)) return rc;
+                                      false, f0, use_filter ? &R.tx2 : nullptr, tile)) return rc;
     // the raw staging slot has been consumed by the pack kernels
     if (location == MDH_HOST)
         if (int rc = c->stager.retire(c->stream, slot)) return rc;
@@ -589,6 +695,18 @@ static int rdf_accumulate_piece(mdh_ctx *c, const float *pos1, int64_t s1, const
         P.fc = use_filter ? R.fca : R.fc;       // R.fca: set by rdf_filter_prepare
         P.fast_bins = R.fast_bins ? 1 : 0;
         P.fstats = R.fstats.as<unsigned long long>();
+        P.xform = nullptr;
+        if (use_filter) {
+            const int64_t n_pairs = (int64_t)n_itiles * P.n_jtiles;
+            if (int rc = R.xform.reserve(n_pairs * n_frames)) return rc;
+            const float2 *tx1 = R.tx1.as<float2>(), *tx2 = R.same ? tx1 : R.tx2.as<float2>();
+            rdf_cleanx_forms_kernel<<<dim3((unsigned)((n_pairs + 127) / 128), n_frames), 128, 0,
+                                      c->stream>>>(tx1, tx2, n_itiles, P.n_jtiles, P.boxes,
+                                                   R.xform.as<unsigned char>());
+            MDH_CUDA(cudaGetLastError());
+            c->launches++;
+            P.xform = R.xform.as<unsigned char>();
+        }
         if (use_filter) {
             // the filter kernel takes every frame whose error bound is small against a
             // bin; the exact kernel below then only runs the frames it declined

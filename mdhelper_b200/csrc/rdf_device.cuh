@@ -439,10 +439,13 @@ __device__ __forceinline__ f32x2 abs2(f32x2 v)
 //   HALF = false  m = fma(-box, rint(df * inv), df)        4 packed instructions per axis
 //   HALF = true   m = ||df| - box/2| - box/2               2 packed instructions per axis,
 //                 |m| is the minimum image for |df| <= 1.5 box (only |m| matters for m^2)
-template <bool HALF>
+//   CX (HALF only, x axis): m_x = bx + ax, no fold -- the all-pairs kernel's x-clean tile
+//                 pairs (filter_cleanx_form), whose operands already carry the shift S
+template <bool HALF, bool CX = false>
 __device__ __forceinline__ f32x2 filter_d2(f32x2 ax, f32x2 ay, f32x2 az, f32x2 bx, f32x2 by,
                                            f32x2 bz, const FrameFilter &ff)
 {
+    static_assert(HALF || !CX, "the x-clean form is a variant of the half-box form");
     const f32x2 dx = add2(bx, ax);
     const f32x2 dy = add2(by, ay);
     const f32x2 dz = add2(bz, az);
@@ -451,7 +454,7 @@ __device__ __forceinline__ f32x2 filter_d2(f32x2 ax, f32x2 ay, f32x2 az, f32x2 b
         const f32x2 hx = pk2(ff.nhalf[0], ff.nhalf[0]);
         const f32x2 hy = pk2(ff.nhalf[1], ff.nhalf[1]);
         const f32x2 hz = pk2(ff.nhalf[2], ff.nhalf[2]);
-        mx = add2(abs2(add2(abs2(dx), hx)), hx);
+        mx = CX ? dx : add2(abs2(add2(abs2(dx), hx)), hx);
         my = add2(abs2(add2(abs2(dy), hy)), hy);
         mz = add2(abs2(add2(abs2(dz), hz)), hz);
     } else {
@@ -481,13 +484,41 @@ __device__ __forceinline__ void filter_bin2(f32x2 d2, float scale, float offm, u
     u1 = __float_as_uint(b) - (LOWER ? cbits : 0u);
 }
 
-template <bool LOWER, bool HALF = false>
+template <bool LOWER, bool HALF = false, bool CX = false>
 __device__ __forceinline__ void filter_eval2(f32x2 ax, f32x2 ay, f32x2 az, f32x2 bx, f32x2 by,
                                              f32x2 bz, const FrameFilter &ff, float scale,
                                              float offm, unsigned cbits, unsigned &u0,
                                              unsigned &u1)
 {
-    filter_bin2<LOWER>(filter_d2<HALF>(ax, ay, az, bx, by, bz, ff), scale, offm, cbits, u0, u1);
+    filter_bin2<LOWER>(filter_d2<HALF, CX>(ax, ay, az, bx, by, bz, ff), scale, offm, cbits, u0,
+                       u1);
+}
+
+// The x form of one tile pair of the all-pairs filter kernel, from the x extents of its
+// i-tile [lo_i, hi_i] and j-tile [lo_j, hi_j] (float32 values) and the box edge L (a
+// float32 value); every x difference xj - xi of the pair lies in [lo_j - hi_i, hi_j - lo_i]
+// (exact in fp64).  If that interval shifted by S in {0, +L, -L} lies inside (-h + delta,
+// h - delta), h = L/2, every pair has the same x image and m_x = (xj - S) - xi is ONE
+// rounded FADD (DESIGN.md section 4.1b):
+//   0  dirty: the half-box fold, as for every other body
+//   1  S = 0
+//   2  S = +L, applied to the j-tile: xj - L is exact (Sterbenz) for xj in [L/2, 2L]
+//   3  S = -L, applied to the negated i-coordinates: L - xi is exact for xi in [L/2, 2L],
+//      and (L - xi) - L gives -xi back exactly
+// delta = 2^-20 L > 2^-23 * 1.5 L: the float32 difference df = fl(xj - xi) of the
+// reference then also has |df - S| < h, so |df - S| is df's minimum image.  NaN extents
+// compare false: dirty.
+__host__ __device__ inline int filter_cleanx_form(float lo_i, float hi_i, float lo_j, float hi_j,
+                                                  float L)
+{
+    const double l = (double)L, h = 0.5 * l, dl = l * (1.0 / 1048576.0);
+    const double lo = (double)lo_j - (double)hi_i, hi = (double)hi_j - (double)lo_i;
+    const bool sterbenz_j = (double)lo_j >= h && (double)hi_j <= 2.0 * l;
+    const bool sterbenz_i = (double)lo_i >= h && (double)hi_i <= 2.0 * l;
+    if (lo > -h + dl && hi < h - dl) return 1;
+    if (sterbenz_j && lo - l > -h + dl && hi - l < h - dl) return 2;
+    if (sterbenz_i && lo + l > -h + dl && hi + l < h - dl) return 3;
+    return 0;
 }
 
 // Per-frame parameters of the fp32 filter from the frame's box and coordinate extents
@@ -543,7 +574,9 @@ __host__ __device__ inline unsigned f32_bits(float f)
 
 // Host and device: the preparation kernels run it per frame, mdh_rdf_filter_window on the
 // host (device-free tests of the window).  mu (optional): the bound in bins, before the
-// 1.25 margin of the window.
+// 1.25 margin of the window.  CLEANX: the all-pairs filter kernel, whose x-clean tile pairs
+// (filter_cleanx_form) widen the half-box term of the x axis.
+template <bool CLEANX = false>
 __host__ __device__ inline FrameFilter filter_prepare_frame(const FrameBox &fb, const unsigned *e1,
                                                             const unsigned *e2, const FilterPrep &Q,
                                                             double *mu_out = nullptr)
@@ -579,8 +612,14 @@ __host__ __device__ inline FrameFilter filter_prepare_frame(const FrameBox &fb, 
         // By Sterbenz at most one of the two rounds, and the rounded result lies in
         // [h/2, h] (|df| < h/2: e; h/2 <= |df| <= box: m) or in [h, 2h] (|df| > box: e).
         if (!(D <= 1.5 * box)) half = false;
-        const double ah = e24 * (D <= box ? 0.5 * box : box) * (1.0 + 1e-6) + eps_b * D +
-                          D / 2251799813685248.0 + 1e-30;
+        double ah = e24 * (D <= box ? 0.5 * box : box) * (1.0 + 1e-6) + eps_b * D +
+                    D / 2251799813685248.0 + 1e-30;
+        // x axis of the all-pairs kernel, x-clean tile pairs (filter_cleanx_form): m_x =
+        // fl(xj - xi - S) with |xj - xi - S| < h rounds once (2^-24 h) from the exact
+        // difference, which is within 2^-24 D of the reference's df - S
+        if (CLEANX && k == 0)
+            ah = fmax(ah, e24 * (0.5 * box + D) * (1.0 + 1e-6) + eps_b * D +
+                              D / 2251799813685248.0 + 1e-30);
         h2 += ah * ah;
         mb[k] = filter_halfbox_mbound(D, 0.5 * box);
         ff.nbox[k] = -(float)box;                          // box is a float32 value
@@ -648,7 +687,11 @@ struct PairParams {
                                    // declined by the filter, [5] / [6] frames the all-pairs
                                    // filter evaluated in the half-box / rint form,
                                    // [7] half-box frames it evaluated unclamped
-                                   // (counted by rdf_filter_prepare_kernel)
+                                   // (counted by rdf_filter_prepare_kernel), [8] pairs it
+                                   // evaluated in x-clean tile pairs
+    // x form of every tile pair of the x-sorted groups (rdf_cleanx_forms_kernel),
+    // [F][pad1 / tile][n_jtiles]; nullptr: the groups are not sorted, every pair is dirty
+    const unsigned char *xform;
 };
 
 }  // namespace rdfdev

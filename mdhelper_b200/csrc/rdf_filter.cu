@@ -84,11 +84,13 @@ __host__ __device__ inline size_t filter_smem_bytes(int n_bins, int hslots, int 
 // Exact re-evaluation of the IPT pairs behind one deferred entry (thread te of the
 // block, tile row jj): every pair the main loop saw as uncertain has been added to
 // the slot the fp32 arithmetic suggested -- unclamped: its coordinate's slot, which
-// lies below fc.hslots --; move it if the fp64 arithmetic disagrees.
-template <bool EXCL, bool LOWER, int IPT, bool HALF>
+// lies below fc.hslots --; move it if the fp64 arithmetic disagrees.  CX: the tile pair is
+// x-clean with the shift of form (filter_cleanx_form): the i-coordinates take the same
+// shift as in the main loop, and the j-row's x is restored for the fp64 arithmetic.
+template <bool EXCL, bool LOWER, int IPT, bool HALF, bool CX = false>
 __device__ __noinline__ void filter_fix(const PairParams &P, int frame, int it, unsigned entry,
                                         const float4 *tile, const double *sT, unsigned hist32,
-                                        unsigned weight)
+                                        unsigned weight, int form = 0)
 {
     constexpr int TILE = kThreads * IPT;
     const FrameFilter ff = P.filt[frame];
@@ -98,15 +100,20 @@ __device__ __noinline__ void filter_fix(const PairParams &P, int frame, int it, 
     const float4 pj = tile[jj];
     const float4 *f1 = P.p1 + (int64_t)frame * P.pad1;
     const unsigned span_l = LOWER ? fc.span : fc.cbits + fc.span;
+    const float L = -ff.nbox[0];
+    float4 pjx = pj;                      // the j-row as the reference sees it
+    if (CX && form == 2) pjx.x = __fadd_rn(pj.x, L);
     for (int ip = 0; ip < IPT; ip += 2) {
         // the same particle pairing as the main loop (rows past the end of the group
         // repeat the last particle there; they carry weight 0 and are skipped here)
         const int i0 = it * TILE + ip * kThreads + te, i1 = i0 + kThreads;
         const float4 a0 = f1[min(i0, P.n1 - 1)], a1 = f1[min(i1, P.n1 - 1)];
+        f32x2 ax = pk2(-a0.x, -a1.x);
+        if (CX && form == 3) ax = add2(ax, pk2(L, L));
         unsigned uu[2];
-        filter_eval2<LOWER, HALF>(pk2(-a0.x, -a1.x), pk2(-a0.y, -a1.y), pk2(-a0.z, -a1.z),
-                            pk2(pj.x, pj.x), pk2(pj.y, pj.y), pk2(pj.z, pj.z), ff, fc.scale,
-                            ff.offm, fc.cbits, uu[0], uu[1]);
+        filter_eval2<LOWER, HALF, CX>(ax, pk2(-a0.y, -a1.y), pk2(-a0.z, -a1.z),
+                                      pk2(pj.x, pj.x), pk2(pj.y, pj.y), pk2(pj.z, pj.z), ff,
+                                      fc.scale, ff.offm, fc.cbits, uu[0], uu[1]);
         for (int h = 0; h < 2; ++h) {
             const int i = h ? i1 : i0;
             const float4 a = h ? a1 : a0;
@@ -119,7 +126,7 @@ __device__ __noinline__ void filter_fix(const PairParams &P, int frame, int it, 
             // u < span_l: that slot is a word of the histogram, below fc.hslots
             const unsigned seen = (LOWER ? u : u - fc.cbits) >> fc.k;
             const unsigned col = (unsigned)te & ((1u << fc.cb) - 1u);
-            const double d2 = pair_d2(a.x, a.y, a.z, pj, fb);
+            const double d2 = pair_d2(a.x, a.y, a.z, pjx, fb);
             const int slot = (P.fast_bins ? slot_fast(d2, sT, P.n_bins, P.guess)
                                           : slot_search(d2, sT, P.n_bins)) + fc.lo;
             if (seen == (unsigned)slot) continue;
@@ -174,11 +181,12 @@ __device__ __forceinline__ void filter_block(const PairParams &P, const FrameFil
     static_assert(IPT % 2 == 0, "particles are processed in packed pairs");
     float xi[IPT], yi[IPT], zi[IPT];
     int gi[IPT];
-    bool vi[IPT];
+    // rows of this thread below the end of the group: ii * kThreads < nv (one register
+    // across the tile loop rather than one per row)
+    const int nv = P.n1 - it * TILE - tid;
 #pragma unroll
     for (int ii = 0; ii < IPT; ++ii) {
         const int i = it * TILE + ii * kThreads + tid;
-        vi[ii] = i < P.n1;
         // rows past the end of the group repeat the last particle with weight 0
         const float4 a = f1[min(i, P.n1 - 1)];
         xi[ii] = a.x; yi[ii] = a.y; zi[ii] = a.z; gi[ii] = __float_as_int(a.w);
@@ -221,6 +229,14 @@ __device__ __forceinline__ void filter_block(const PairParams &P, const FrameFil
     };
     stage_tile(jt0, 0);
 
+    // x-clean tile pairs (filter_cleanx_form) in the half-box unclamped body of x-sorted
+    // groups.  The tile pair's form is kept in a shared word (sCount[1]) and the box edge
+    // L is reread where it is needed: no register stays live across the hot loop for them.
+    // Not with exclusions: the tag compare leaves no room for a second body without
+    // spills in the hot loop (ptxas -v; those launches keep the dirty form).
+    constexpr bool CXOK = HALF && !CLAMP && !EXCL;
+    unsigned *sForm = sCount + 1;
+
     unsigned long long audit_bad = 0, audit_unc = 0;
     int buf = 0;
     for (int jt = jt0; jt < jt1; ++jt) {
@@ -230,15 +246,40 @@ __device__ __forceinline__ void filter_block(const PairParams &P, const FrameFil
         } else {
             __pipeline_wait_prior(0);
         }
+        // the tile pair's x form (uniform over the block); S = +L moves this thread's own
+        // rows of the j-tile (their copies have landed), S = -L the thread's i-coordinates
+        if constexpr (CXOK) {
+            if (P.xform != nullptr) {
+                const float L = -ff.nbox[0];
+                const int form =
+                    P.xform[((int64_t)frame * (P.pad1 / TILE) + it) * P.n_jtiles + jt];
+                if (tid == 0) *sForm = (unsigned)form;
+                if (form == 2) {
+                    float4 *rows = sJ + buf * TSTRIDE;
+#pragma unroll
+                    for (int q = 0; q < IPT; ++q)
+                        rows[q * kThreads + tid].x = __fsub_rn(rows[q * kThreads + tid].x, L);
+                }
+                if (form == 3) {
+#pragma unroll
+                    for (int ip = 0; ip < IPT / 2; ++ip) nx[ip] = add2(nx[ip], pk2(L, L));
+                }
+            } else if (tid == 0) {
+                *sForm = 0u;
+            }
+        }
         __syncthreads();
 
         const unsigned weight = (P.same && jt > it) ? 2u : 1u;
         unsigned wi[IPT];
 #pragma unroll
-        for (int ii = 0; ii < IPT; ++ii) wi[ii] = vi[ii] ? weight : 0u;
+        for (int ii = 0; ii < IPT; ++ii) wi[ii] = ii * kThreads < nv ? weight : 0u;
         const int jn = min(TILE, P.n2 - jt * TILE);
         const float4 *tile = sJ + buf * TSTRIDE;
 
+        // the tile's pipeline and deferred entries, in the x-clean form (CX) or not
+        auto body = [&](auto cx_tag) {
+        constexpr bool CX = decltype(cx_tag)::value;
         // Stage A1: packed squared distances of NR tile rows against the IPT particles of
         // this thread (FMA pipe only).
         auto stage_a1 = [&](const float4 *pj, f32x2 (*dd)[IPT / 2], auto nr_tag) {
@@ -247,7 +288,7 @@ __device__ __forceinline__ void filter_block(const PairParams &P, const FrameFil
             for (int r = 0; r < NR; ++r)
 #pragma unroll
                 for (int ip = 0; ip < IPT / 2; ++ip)
-                    dd[r][ip] = filter_d2<HALF>(nx[ip], ny[ip], nz[ip], pk2(pj[r].x, pj[r].x),
+                    dd[r][ip] = filter_d2<HALF, CX>(nx[ip], ny[ip], nz[ip], pk2(pj[r].x, pj[r].x),
                                           pk2(pj[r].y, pj[r].y), pk2(pj[r].z, pj[r].z), ff);
         };
         // Stage A2: square roots (MUFU) and fixed-point bin coordinates.
@@ -282,8 +323,9 @@ __device__ __forceinline__ void filter_block(const PairParams &P, const FrameFil
                         const bool in = u < span_l;
                         // an unclamped frame must never leave the histogram
                         if (!CLAMP && !in) ++audit_bad;
-                        const double d2 =
-                            pair_d2(xi[ii], yi[ii], zi[ii], pj[r], P.boxes[frame]);
+                        float4 pr = pj[r];       // the j-row as the reference sees it
+                        if (CX && *sForm == 2u) pr.x = __fadd_rn(pr.x, -ff.nbox[0]);
+                        const double d2 = pair_d2(xi[ii], yi[ii], zi[ii], pr, P.boxes[frame]);
                         const int slot = slot_search(d2, sT, n_bins);
                         // the slot the pair was added to, and the exact one
                         const unsigned fs = in ? ((LOWER ? u : u - fc.cbits) >> fc.k)
@@ -315,8 +357,9 @@ __device__ __forceinline__ void filter_block(const PairParams &P, const FrameFil
                         const unsigned idx = atomicAdd(sCount, 1u);
                         if (idx < (unsigned)kListCap) sList[idx] = entry;
                         else
-                            filter_fix<EXCL, LOWER, IPT, HALF>(P, frame, it, entry, tile, sT, hist32,
-                                                         weight);
+                            filter_fix<EXCL, LOWER, IPT, HALF, CX>(P, frame, it, entry, tile,
+                                                                   sT, hist32, weight,
+                                                                   CX ? (int)*sForm : 0);
                     }
                 }
             }
@@ -395,10 +438,29 @@ __device__ __forceinline__ void filter_block(const PairParams &P, const FrameFil
         const unsigned n_push = *sCount;
         const unsigned n_list = min(n_push, (unsigned)kListCap);
         for (unsigned e = tid; e < n_list; e += kThreads)
-            filter_fix<EXCL, LOWER, IPT, HALF>(P, frame, it, sList[e], tile, sT, hist32, weight);
+            filter_fix<EXCL, LOWER, IPT, HALF, CX>(P, frame, it, sList[e], tile, sT, hist32,
+                                                   weight, CX ? (int)*sForm : 0);
         if (tid == 0 && n_push) {
             atomicAdd(&P.fstats[0], (unsigned long long)n_list);
             if (n_push > n_list) atomicAdd(&P.fstats[1], (unsigned long long)(n_push - n_list));
+        }
+        };
+        if constexpr (CXOK) {
+            if (*sForm) {
+                body(std::true_type());
+                if (tid == 0)     // nv of thread 0: the rows of the i-tile below n1
+                    atomicAdd(&P.fstats[8], (unsigned long long)min(TILE, nv) *
+                                                (unsigned long long)jn);
+                if (*sForm == 3u) {
+                    const float L = -ff.nbox[0];
+#pragma unroll
+                    for (int ip = 0; ip < IPT / 2; ++ip) nx[ip] = add2(nx[ip], pk2(-L, -L));
+                }
+            } else {
+                body(std::false_type());
+            }
+        } else {
+            body(std::false_type());
         }
         __syncthreads();
         if (tid == 0) *sCount = 0;
@@ -474,7 +536,8 @@ __global__ void rdf_filter_prepare_kernel(const PrepareParams Q)
 {
     const int f = blockIdx.x * blockDim.x + threadIdx.x;
     if (f >= Q.n_frames) return;
-    const FrameFilter ff = filter_prepare_frame(Q.boxes[f], Q.ext1 + f * 6, Q.ext2 + f * 6, Q.prep);
+    const FrameFilter ff =
+        filter_prepare_frame<true>(Q.boxes[f], Q.ext1 + f * 6, Q.ext2 + f * 6, Q.prep);
     Q.out[f] = ff;
     // counted here rather than in the filter kernel, whose register allocation is at its
     // limit; rdf_filter_kernel takes the unclamped body exactly for these frames (the
@@ -777,7 +840,8 @@ int rdf_filter_window_impl(int n_bins, double r_lo, double r_hi, int drop_axis, 
         }
         for (int q = 0; q < 2; ++q) {
             double mu = 0.0;
-            const FrameFilter ff = filter_prepare_frame(boxes[f], k1, k2, q ? qc : qa, &mu);
+            const FrameFilter ff = q ? filter_prepare_frame(boxes[f], k1, k2, qc, &mu)
+                                     : filter_prepare_frame<true>(boxes[f], k1, k2, qa, &mu);
             double *o = frames + 10 * f + 5 * q;
             o[0] = (double)ff.offm;
             o[1] = (double)ff.wlim;
