@@ -239,6 +239,24 @@ int mdh_rdf_filter_window(int n_bins, double r_lo, double r_hi, int drop_axis, i
                           const float *ext2 /* [n_frames][6] or NULL */,
                           double *layout /* [2][12] */, double *frames /* [n_frames][2][5] */);
 
+/*
+ * The triclinic fp32 filter's per-frame parameters, computed on the host as
+ * mdh_rdf_accumulate_triclinic would (all-pairs path); device-free.  n_bins, r_lo, r_hi and
+ * sqrt_err as for mdh_rdf_filter_window; cell[n_frames][9] as for
+ * mdh_rdf_accumulate_triclinic; ext1 / ext2 [n_frames][6]: {min x, y, z, max x, y, z} of
+ * each group's coordinates AFTER the wrap into the cell (ext2 NULL: the same group).
+ * frames[n_frames][8]: {eligible (1: filtered, 0: declined), R = min(a_x, b_y, c_z) / 2,
+ * delta (how far the exact folded image can lie outside the brick), mu (error bound in
+ * bins, before the window's 1.25 margin), reach (the frame is filtered iff reach < R and the
+ * window fits), offm, wlim, k}.  MDH_EINVAL when the configuration is not eligible for the
+ * filter or a cell is invalid.
+ */
+int mdh_rdf_triclinic_filter_window(int n_bins, double r_lo, double r_hi, double sqrt_err,
+                                    int n_frames, const float *cell /* [n_frames][9] */,
+                                    const float *ext1 /* [n_frames][6] */,
+                                    const float *ext2 /* [n_frames][6] or NULL */,
+                                    double *frames /* [n_frames][8] */);
+
 int mdh_rdf_fetch(mdh_ctx *ctx, int64_t *counts /* [n_bins] host */);
 int mdh_rdf_reset(mdh_ctx *ctx);
 /* device address of the int64[n_bins] accumulator (for NCCL reductions) */
@@ -249,8 +267,11 @@ int mdh_rdf_pair_evaluations(mdh_ctx *ctx, int64_t *evals);
 /*
  * The all-pairs kernel bins a pair from fp32 arithmetic when a rigorous error bound
  * proves the reference's fp64 distance lies in the same bin, and re-evaluates every
- * other pair with the fp64 arithmetic (rdf_filter.cu).  mode is an MDH_FILTER_*
- * value; it persists across mdh_rdf_configure calls of the context.
+ * other pair with the fp64 arithmetic (rdf_filter.cu).  This covers triclinic cells on
+ * the all-pairs path too (rdf_tri.cu): frames whose r_max plus the bound does not fit
+ * inside half the shortest of a_x, b_y, c_z, or with non-finite coordinates, are declined
+ * and take the 27-image arithmetic; the triclinic cell list is fp64 whatever the mode.
+ * mode is an MDH_FILTER_* value; it persists across mdh_rdf_configure calls of the context.
  */
 int mdh_rdf_set_filter(mdh_ctx *ctx, int mode);
 /* MDH_WRAP_* selector; persists across mdh_rdf_configure calls of the context. */
@@ -285,6 +306,10 @@ int mdh_rdf_filter_unclamped(mdh_ctx *ctx, int64_t *frames /* [1] host */);
  * x component of the minimum image as one subtraction (unclamped half-box frames only).
  * Since the last configure / reset. */
 int mdh_rdf_filter_cleanx(mdh_ctx *ctx, int64_t *pairs /* [1] host */);
+/* out[0] triclinic frames the all-pairs filter evaluated (the declined ones are counted in
+ * mdh_rdf_filter_stats' stats[4]), out[1] pairs of those frames it re-evaluated with the
+ * 27-image fp64 arithmetic (inside the window).  Since the last configure / reset. */
+int mdh_rdf_filter_triclinic(mdh_ctx *ctx, int64_t *out /* [2] host */);
 
 /* ---- seam #2: direct-sum structure factor ------------------------------------ */
 

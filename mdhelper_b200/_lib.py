@@ -51,6 +51,7 @@ SIGNATURES = {
     "mdh_rdf_cells_grid": (_i32, [_p, _f64, _i64, _i32, _p, ctypes.POINTER(_f64)]),
     "mdh_rdf_filter_window": (_i32, [_i32, _f64, _f64, _i32, _i32, _i32, _f64, _i32, _p, _p,
                                      _p, _p, _p]),
+    "mdh_rdf_triclinic_filter_window": (_i32, [_i32, _f64, _f64, _f64, _i32, _p, _p, _p, _p]),
     "mdh_rdf_fetch": (_i32, [_p, _p]),
     "mdh_rdf_reset": (_i32, [_p]),
     "mdh_rdf_counts_device": (_i32, [_p, ctypes.POINTER(_p)]),
@@ -63,6 +64,7 @@ SIGNATURES = {
     "mdh_rdf_filter_modes": (_i32, [_p, _p]),
     "mdh_rdf_filter_unclamped": (_i32, [_p, _p]),
     "mdh_rdf_filter_cleanx": (_i32, [_p, _p]),
+    "mdh_rdf_filter_triclinic": (_i32, [_p, _p]),
     "mdh_sq_configure": (_i32, [_p, _i64, _i32, _p, _i32, _p, _p, _p, _i32, _p, _i32]),
     "mdh_sq_accumulate": (_i32, [_p, _p, _i64, _i32, _i32]),
     "mdh_sq_accumulate_f64": (_i32, [_p, _p, _i64, _i32, _i32]),
@@ -240,6 +242,30 @@ def filter_window(n_bins: int, r_lo: float, r_hi: float, box, ext1, ext2=None, *
                         "cells": typed(FILTER_FRAME_FIELDS, fr[f, 1])} for f in range(nf)]}
 
 
+TRI_FILTER_FIELDS = ("eligible", "R", "delta", "mu", "reach", "offm", "wlim", "k")
+
+
+def triclinic_filter_window(n_bins: int, r_lo: float, r_hi: float, cell, ext1, ext2=None, *,
+                            sqrt_err: float = 2.0 ** -22) -> list:
+    """Per-frame parameters of the triclinic fp32 RDF filter
+    (``mdh_rdf_triclinic_filter_window``; no device needed).  ``cell``: ``[n_frames, 3, 3]``
+    lower-triangular cell matrices; ``ext1`` / ``ext2``: ``[n_frames, 6]`` float32 extents
+    {min x, y, z, max x, y, z} of the two groups after the wrap into the cell (``ext2=None``:
+    one group).  Returns one dict per frame with the fields of ``TRI_FILTER_FIELDS``
+    (``eligible``, ``wlim``, ``k`` as ``int``, the others as ``float``).  Raises ``ValueError``
+    when the configuration is not eligible for the filter or a cell is invalid."""
+    c = np.ascontiguousarray(cell, dtype=np.float32).reshape(-1, 9)
+    nf = len(c)
+    e1 = np.ascontiguousarray(ext1, dtype=np.float32).reshape(nf, 6)
+    e2 = None if ext2 is None else np.ascontiguousarray(ext2, dtype=np.float32).reshape(nf, 6)
+    fr = np.zeros((nf, 8), np.float64)
+    check(lib().mdh_rdf_triclinic_filter_window(int(n_bins), float(r_lo), float(r_hi),
+                                                float(sqrt_err), nf, c.ctypes.data,
+                                                e1.ctypes.data, _ptr(e2), fr.ctypes.data))
+    return [{n: (int(v) if n in ("eligible", "wlim", "k") else float(v))
+             for n, v in zip(TRI_FILTER_FIELDS, fr[f])} for f in range(nf)]
+
+
 class Context:
     """
     One device, one stream (``mdh_ctx``).  ``stream=None`` uses torch's current
@@ -341,7 +367,11 @@ class Context:
         check(self._lib.mdh_rdf_reset(self._h))
 
     def rdf_set_filter(self, mode: str = "auto"):
-        """fp32 filter of the all-pairs kernel: ``auto``, ``off``, ``on``, ``audit``."""
+        """fp32 filter of the all-pairs kernel: ``auto``, ``off``, ``on``, ``audit``.  It
+        covers triclinic cells on the all-pairs path as well; frames whose ``r_max`` plus the
+        error bound does not fit inside half the shortest of a_x, b_y, c_z (or with
+        non-finite coordinates) are declined and take the 27-image fp64 arithmetic.  The
+        triclinic cell list is fp64 whatever the mode."""
         check(self._lib.mdh_rdf_set_filter(self._h, FILTER_MODES[mode]))
 
     def rdf_set_prewrap(self, mode: str = "auto"):
@@ -350,15 +380,16 @@ class Context:
         check(self._lib.mdh_rdf_set_prewrap(self._h, WRAP_MODES[mode]))
 
     def rdf_filter_stats(self) -> dict:
-        out = np.zeros(10, dtype=np.int64)
+        out = np.zeros(12, dtype=np.int64)
         check(self._lib.mdh_rdf_filter_stats(self._h, out[:6].ctypes.data))
         check(self._lib.mdh_rdf_filter_modes(self._h, out[6:8].ctypes.data))
         check(self._lib.mdh_rdf_filter_unclamped(self._h, out[8:9].ctypes.data))
-        check(self._lib.mdh_rdf_filter_cleanx(self._h, out[9:].ctypes.data))
+        check(self._lib.mdh_rdf_filter_cleanx(self._h, out[9:10].ctypes.data))
+        check(self._lib.mdh_rdf_filter_triclinic(self._h, out[10:].ctypes.data))
         return dict(zip(("deferred_entries", "inline_entries", "audit_violations",
                          "audit_uncertain_pairs", "declined_frames", "eligible",
                          "halfbox_frames", "rint_frames", "unclamped_frames",
-                         "cleanx_pairs"),
+                         "cleanx_pairs", "triclinic_frames", "triclinic_exact_pairs"),
                         (int(v) for v in out)))
 
     def rdf_bin_lookup(self) -> dict:

@@ -128,7 +128,11 @@ def radial_histogram(
         (pairs provably inside a bin are binned from fp32, all others are
         re-evaluated exactly); ``"off"``: fp64 for every pair; ``"audit"``:
         filter plus a full exact comparison (test aid).  Counts do not depend
-        on it either.
+        on it either.  On triclinic cells it applies to the all-pairs kernel;
+        frames whose ``range[1]`` plus the error bound does not fit inside half
+        the shortest of a_x, b_y, c_z (or with non-finite coordinates) are
+        declined and take the 27-image fp64 arithmetic, and the triclinic cell
+        list is fp64 whatever ``arith`` says.
     wrap : `str`, keyword-only
         Coordinates outside the cell: ``"auto"`` follows the reference --
         ``capped_distance`` moves both coordinate sets into the cell in float32 before

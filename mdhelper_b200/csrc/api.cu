@@ -353,6 +353,14 @@ int mdh_rdf_filter_window(int n_bins, double r_lo, double r_hi, int drop_axis, i
                                   n_frames, box, ext1, ext2, layout, frames);
 }
 
+int mdh_rdf_triclinic_filter_window(int n_bins, double r_lo, double r_hi, double sqrt_err,
+                                    int n_frames, const float *cell, const float *ext1,
+                                    const float *ext2, double *frames)
+{
+    return rdf_triclinic_filter_window_impl(n_bins, r_lo, r_hi, sqrt_err, n_frames, cell, ext1,
+                                            ext2, frames);
+}
+
 int mdh_rdf_fetch(mdh_ctx *c, int64_t *counts)
 {
     CTX_GUARD(c);
@@ -372,7 +380,7 @@ int mdh_rdf_reset(mdh_ctx *c)
     if (c->rdf.evals_dev_init)
         MDH_CUDA(cudaMemsetAsync(c->rdf.cell[9].p, 0, sizeof(unsigned long long), c->stream));
     if (c->rdf.fstats.p)
-        MDH_CUDA(cudaMemsetAsync(c->rdf.fstats.p, 0, sizeof(unsigned long long) * 9, c->stream));
+        MDH_CUDA(cudaMemsetAsync(c->rdf.fstats.p, 0, sizeof(unsigned long long) * 11, c->stream));
     c->rdf.evals = 0;
     return MDH_OK;
 }
@@ -481,6 +489,19 @@ int mdh_rdf_filter_cleanx(mdh_ctx *c, int64_t *pairs)
     MDH_CUDA(cudaMemcpyAsync(h, c->rdf.fstats.p, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
     MDH_CUDA(cudaStreamSynchronize(c->stream));
     pairs[0] = (int64_t)h[8];
+    return MDH_OK;
+}
+
+int mdh_rdf_filter_triclinic(mdh_ctx *c, int64_t *out)
+{
+    CTX_GUARD(c);
+    MDH_REQUIRE(out != nullptr, MDH_EINVAL, "out is NULL");
+    MDH_REQUIRE(c->rdf.configured, MDH_ESTATE, "rdf: not configured");
+    unsigned long long h[11] = {0};
+    MDH_CUDA(cudaMemcpyAsync(h, c->rdf.fstats.p, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
+    MDH_CUDA(cudaStreamSynchronize(c->stream));
+    out[0] = (int64_t)h[9];
+    out[1] = (int64_t)h[10];
     return MDH_OK;
 }
 

@@ -134,8 +134,9 @@ struct RdfState {
     FilterConst fc;
     FilterConst fca;       // the all-pairs filter kernel's layout for the current batch
     DevBuf ext1, ext2;     // unsigned[F][6]: coordinate extents of each frame (keys)
-    DevBuf filt;           // FrameFilter[F]
-    DevBuf fstats;         // unsigned long long[9], see PairParams::fstats
+    DevBuf filt;           // FrameFilter[F] (triclinic frames: TriFilter[F], rdf_tri.cu)
+    DevBuf fstats;         // unsigned long long[11], see PairParams::fstats and
+                           // rdf_tri.cu::TriFilterParams::fstats
     DevBuf xsort;          // float4[F][npad]: packed rows before the x-sort (rdf_xsort_kernel)
     DevBuf tx1, tx2;       // float2[F][tiles]: x extents of the tiles of the x-sorted groups
     DevBuf xform;          // unsigned char[F][i-tiles][j-tiles]: x form of every tile pair
@@ -304,6 +305,9 @@ int rdf_triclinic_grid_impl(const float *cell9, double r_hi, int64_t n_max, int3
                             double *margin);
 int rdf_cells_grid_impl(const float *cell9, double r_hi, int64_t n_max, int drop_axis,
                         int32_t *nc, double *margin);
+int rdf_triclinic_filter_window_impl(int n_bins, double r_lo, double r_hi, double sqrt_err,
+                                     int n_frames, const float *cell, const float *ext1,
+                                     const float *ext2, double *frames);
 // rdf_filter.cu
 int rdf_filter_sqrt_error(mdh_ctx *c, double *err);
 bool rdf_filter_configure(RdfState &R, const double *thr, double sqrt_err);

@@ -390,8 +390,8 @@ int rdf_configure_impl(mdh_ctx *c, int64_t n1, int64_t n2, int same, int n_bins,
     if (int rc = R.thr.reserve(sizeof(double) * (n_bins + 2))) return rc;
     if (int rc = R.counts.reserve(sizeof(unsigned long long) * n_bins)) return rc;
     if (int rc = R.cell[9].reserve(sizeof(unsigned long long) + sizeof(int))) return rc;
-    if (int rc = R.fstats.reserve(sizeof(unsigned long long) * 9)) return rc;
-    MDH_CUDA(cudaMemsetAsync(R.fstats.p, 0, sizeof(unsigned long long) * 9, c->stream));
+    if (int rc = R.fstats.reserve(sizeof(unsigned long long) * 11)) return rc;
+    MDH_CUDA(cudaMemsetAsync(R.fstats.p, 0, sizeof(unsigned long long) * 11, c->stream));
     std::vector<double> t(thr, thr + n_bins + 1);
     t.push_back(INFINITY);
     MDH_CUDA(cudaMemcpyAsync(R.thr.p, t.data(), sizeof(double) * t.size(),

@@ -16,8 +16,10 @@
 //      and d^2 = (rx rx + ry ry) + rz rz.
 // Binning is the squared-threshold comparison of the orthorhombic kernels (rdf.cu).
 //
-// Two pair kernels give the same counts:
+// Three pair kernels give the same counts:
 //   rdf_triclinic_kernel   all pairs, every pair evaluates the 27 images (fp64);
+//   rdf_tri_filter_kernel  all pairs, ONE image per pair in fp32 behind an error bound,
+//                          the 27 images for pairs near a bin edge (DESIGN.md 4.8b);
 //   rdf_tri_cells_kernel   cut-off runs: a cell list in fractional coordinates, and for
 //                          every candidate only the ONE image that can be in range
 //                          (argument and margin: tri_grid_plan below, DESIGN.md 4.8).
@@ -145,6 +147,436 @@ __global__ void __launch_bounds__(256) rdf_triclinic_kernel(const TriParams P)
         for (int w = 0; w < kWarps; ++w) s += sH[w * n_bins + k];
         if (s) atomicAdd(&P.counts[k], s);
     }
+}
+
+// ---- fp32 filter of the all-pairs path (DESIGN.md 4.8b) -------------------------------
+//
+// Per pair ONE image in fp32, from the sequential fold the lower-triangular cell allows
+// (tri_fold2): n_c = rint(df_z / c_z), then n_b from the remaining y, then n_a from the
+// remaining x, u = df - n_c c - n_b b - n_a a.  Let B be the open brick of half-widths
+// a_x / 2, b_y / 2, c_z / 2 and R = min(a_x, b_y, c_z) / 2.  Two points of B never differ by
+// a lattice vector (compare z, then y, then x), so if the exact value of u has |u| < R it
+// lies in B and every other image is at least R long.  The computed n are rint of rounded
+// arguments, so the exact u lies within delta of B (tri_filter_prepare_frame bounds delta)
+// and the true minimum is at least min(|u|, R - delta).  A frame is filtered when every
+// pair the filter can bin lies well inside R - delta; then
+//   - n in {-1, 0, 1}^3 (u is one of the reference's 27 images): the reference's minimum
+//     is its fp64 d^2 of u, and the window of 4.1b decides the bin from the fp32 d^2;
+//   - some |n_k| >= 2: u is not among the reference's images, its minimum is at least
+//     R - delta - (fp64 error) > r_hi, and the pair goes to the above-range slot.  This is
+//     the reference's quirk (its 27 images miss the shortest one), reproduced.
+// Pairs inside the window are re-evaluated with tri_d2 (rdf_triclinic_kernel's bits).
+
+struct TriFilter {         // per frame (tri_filter_prepare_frame)
+    float nh[6];           // -a_x, -b_x, -b_y, -c_x, -c_y, -c_z
+    float inv[3];          // (float)(1 / a_x), (float)(1 / b_y), (float)(1 / c_z)
+    float offm;            // as FrameFilter::offm
+    unsigned wlim;         // as FrameFilter::wlim; 0 = declined (rdf_triclinic_kernel's arithmetic)
+};
+
+// The fold of two pairs, d = b + a per axis (a: the negated group-1 coordinates).  Returns
+// the packed fp32 |u|^2; w0 / w1 are the bits of n_a | n_b | n_c of each pair, whose bit
+// 30 is set iff some |n_k| >= 2 (the n are small integers in float32).  Odd-symmetric bit
+// for bit: (j, i) gives -df, -n, -u.
+__device__ __forceinline__ f32x2 tri_fold2(f32x2 ax, f32x2 ay, f32x2 az, f32x2 bx, f32x2 by,
+                                           f32x2 bz, const TriFilter &tf, unsigned &w0,
+                                           unsigned &w1)
+{
+    const f32x2 magic = pk2(kMagicF, kMagicF), nmagic = pk2(-kMagicF, -kMagicF);
+    const f32x2 dx = add2(bx, ax), dy = add2(by, ay), dz = add2(bz, az);
+    const f32x2 nc = add2(fma2(dz, pk2(tf.inv[2], tf.inv[2]), magic), nmagic);
+    const f32x2 uz = fma2(nc, pk2(tf.nh[5], tf.nh[5]), dz);
+    const f32x2 y1 = fma2(nc, pk2(tf.nh[4], tf.nh[4]), dy);
+    const f32x2 x1 = fma2(nc, pk2(tf.nh[3], tf.nh[3]), dx);
+    const f32x2 nb = add2(fma2(y1, pk2(tf.inv[1], tf.inv[1]), magic), nmagic);
+    const f32x2 uy = fma2(nb, pk2(tf.nh[2], tf.nh[2]), y1);
+    const f32x2 x2 = fma2(nb, pk2(tf.nh[1], tf.nh[1]), x1);
+    const f32x2 na = add2(fma2(x2, pk2(tf.inv[0], tf.inv[0]), magic), nmagic);
+    const f32x2 ux = fma2(na, pk2(tf.nh[0], tf.nh[0]), x2);
+    float a0, a1, b0, b1, c0, c1;
+    upk2(na, a0, a1);
+    upk2(nb, b0, b1);
+    upk2(nc, c0, c1);
+    w0 = __float_as_uint(a0) | __float_as_uint(b0) | __float_as_uint(c0);
+    w1 = __float_as_uint(a1) | __float_as_uint(b1) | __float_as_uint(c1);
+    return fma2(uz, uz, fma2(uy, uy, mul2(ux, ux)));
+}
+
+// Per-frame parameters from the cell and the extent keys of the WRAPPED coordinates
+// (e1 / e2: {min x, y, z, max x, y, z} of the two groups).  info (optional): {R, delta, mu
+// (the bound in bins, before the 1.25 margin of the window), reach}.  Bound, per axis, of
+// the fp32 |u| against the reference's fp64 d of the same image:
+//   fold: one rounding per FMA, on results bounded by the extents D and the tilts:
+//         x: 2^-24 (X1 + X2 + H_x), y: 2^-24 (Y1 + H_y), z: 2^-24 H_z (H_k = half-width
+//         + delta_k bounds |u_k|; X1, X2, Y1 bound the intermediate x', x'', y');
+//   reference: its image sums in fp64, 3 / 2 / 1 roundings of terms below D_k + the
+//         row of the cell (no eps_b term: the triclinic reference has no float32 inverse);
+// then, as filter_prepare_frame: the 2-norm of those, the fp32 sum of squares, the measured
+// sqrt.approx error, scale / offset / fma roundings, and the fp64 squares of the reference.
+// delta_k: the rint argument's rounding, |arg| |inv_k h_kk - 1| h_kk, plus the fold's
+// roundings before it.  The frame is filtered when reach = d_max + 1.25 mu / scale + 2 (fp64
+// error of any image) + delta < R.
+__host__ __device__ inline TriFilter tri_filter_prepare_frame(const TriBox &h, const unsigned *e1,
+                                                              const unsigned *e2,
+                                                              const FilterPrep &Q,
+                                                              double *info = nullptr)
+{
+    const double e24 = 1.0 / 16777216.0, u53 = 1.0 / 9007199254740992.0;
+    bool ok = true;
+    double D[3];
+    for (int k = 0; k < 3; ++k) {
+        const float e4[4] = {ext_unkey(e1[k]), ext_unkey(e1[3 + k]), ext_unkey(e2[k]),
+                             ext_unkey(e2[3 + k])};
+        for (int q = 0; q < 4; ++q)
+            if ((f32_bits(e4[q]) & 0x7f800000u) == 0x7f800000u) ok = false;
+        D[k] = fmax(fmax((double)e4[3] - (double)e4[0], (double)e4[1] - (double)e4[2]), 0.0) *
+               (1.0 + 2.0 * e24);
+    }
+    TriFilter tf;
+    const float ia = (float)(1.0 / h.ax), ib = (float)(1.0 / h.by), ic = (float)(1.0 / h.cz);
+    const double ea = fabs((double)ia * h.ax - 1.0), eb = fabs((double)ib * h.by - 1.0),
+                 ec = fabs((double)ic * h.cz - 1.0);              // exact: 24 x 24 bits
+    const double Nc = floor(D[2] * ic * (1.0 + 1e-12) + 0.5);
+    const double Y1 = (D[1] + Nc * fabs(h.cy)) * (1.0 + e24);
+    const double Nb = floor(Y1 * ib * (1.0 + 1e-12) + 0.5);
+    const double X1 = (D[0] + Nc * fabs(h.cx)) * (1.0 + e24);
+    const double X2 = (X1 + Nb * fabs(h.bx)) * (1.0 + e24);
+    // the magic-number rint needs its arguments well inside 2^22
+    if (!(D[2] * ic < 1048576.0 && Y1 * ib < 1048576.0 && X2 * ia < 1048576.0)) ok = false;
+    const double dz = D[2] * ec, dy = Y1 * (eb + e24), dx = X2 * ea + e24 * (X1 + X2);
+    const double delta = fmax(dx, fmax(dy, dz)) * (1.0 + 1e-6);
+    const double Hx = 0.5 * h.ax + dx, Hy = 0.5 * h.by + dy, Hz = 0.5 * h.cz + dz;
+    const double fx = e24 * (X1 + X2 + Hx) * (1.0 + 1e-6), fy = e24 * (Y1 + Hy) * (1.0 + 1e-6),
+                 fz = e24 * Hz * (1.0 + 1e-6);
+    const double rx = 3.0 * u53 * (D[0] + h.ax + fabs(h.bx) + fabs(h.cx)),
+                 ry = 2.0 * u53 * (D[1] + h.by + fabs(h.cy)), rz = u53 * (D[2] + h.cz);
+    const double a = sqrt((fx + rx) * (fx + rx) + (fy + ry) * (fy + ry) + (fz + rz) * (fz + rz));
+    const double e_ref = sqrt(rx * rx + ry * ry + rz * rz);
+    const double R = 0.5 * fmin(h.ax, fmin(h.by, h.cz));
+    const double two_k = (double)(1u << Q.k);
+    const double mu = Q.scale * (a + Q.d_max * (1.5 * e24 * 1.001 + Q.sqrt_err + 4.0 * u53)) +
+                      e24 * Q.scale * Q.d_max * 1.001 + 1.0 / two_k + 1e-9;
+    const double m = ceil(1.25 * mu * two_k) + 1.0;
+    if (!(m >= 1.0) || !(2.0 * m + 1.0 < two_k / 8.0)) ok = false;
+    const double reach = Q.d_max + 1.25 * mu / Q.scale + 2.0 * (e_ref + 4.0 * u53 * R) + delta;
+    if (!(reach * (1.0 + 1e-9) < R)) ok = false;
+    if (info) { info[0] = R; info[1] = delta; info[2] = mu; info[3] = reach; }
+    tf.nh[0] = -(float)h.ax; tf.nh[1] = -(float)h.bx; tf.nh[2] = -(float)h.by;
+    tf.nh[3] = -(float)h.cx; tf.nh[4] = -(float)h.cy; tf.nh[5] = -(float)h.cz;
+    tf.inv[0] = ia; tf.inv[1] = ib; tf.inv[2] = ic;
+    tf.offm = ok ? (float)(Q.offbase + m / two_k) : 0.f;
+    tf.wlim = ok ? 2u * (unsigned)m + 1u : 0u;
+    return tf;
+}
+
+// per frame {min x, y, z, max x, y, z} keys of the wrapped packed coordinates (ext set
+// up by rdf_ext_init_kernel)
+__global__ void __launch_bounds__(256)
+    tri_extent_kernel(const float4 *__restrict__ p, int64_t npad, int n, unsigned *__restrict__ ext)
+{
+    __shared__ unsigned red[8][6];
+    const int frame = blockIdx.y, tid = threadIdx.x;
+    unsigned lo[3] = {0xffffffffu, 0xffffffffu, 0xffffffffu}, hi[3] = {0u, 0u, 0u};
+    for (int i = blockIdx.x * 256 + tid; i < n; i += gridDim.x * 256) {
+        const float4 v = p[(int64_t)frame * npad + i];
+        const unsigned k[3] = {ext_key(v.x), ext_key(v.y), ext_key(v.z)};
+        for (int a = 0; a < 3; ++a) { lo[a] = min(lo[a], k[a]); hi[a] = max(hi[a], k[a]); }
+    }
+    for (int a = 0; a < 3; ++a) {
+        const unsigned l = __reduce_min_sync(0xffffffffu, lo[a]);
+        const unsigned h = __reduce_max_sync(0xffffffffu, hi[a]);
+        if ((tid & 31) == 0) { red[tid >> 5][a] = l; red[tid >> 5][3 + a] = h; }
+    }
+    __syncthreads();
+    if (tid < 6) {
+        unsigned v = red[0][tid];
+        for (int w = 1; w < 8; ++w) v = tid < 3 ? min(v, red[w][tid]) : max(v, red[w][tid]);
+        if (tid < 3) { if (v != 0xffffffffu) atomicMin(&ext[frame * 6 + tid], v); }
+        else if (v != 0u) atomicMax(&ext[frame * 6 + tid], v);
+    }
+}
+
+constexpr int kTriIpt = 4;                       // i-particles per thread
+constexpr int kTriTile = kThreads * kTriIpt;     // rows of an i-tile and of a j-tile
+constexpr int kTriListCap = 2048;                // deferred rows per block and tile
+
+struct TriFilterParams {
+    const float4 *p1, *p2;
+    int64_t pad1, pad2;            // multiples of kTriTile
+    int n1, n2;
+    const TriBox *boxes;
+    const TriFilter *filt;
+    const double *thr;
+    int n_bins;
+    BinGuess guess;
+    int fast_bins;
+    int same;
+    int n_jchunks, jtiles_per_chunk, n_jtiles;
+    FilterConst fc;                // the clamped layout (rdf_filter_configure)
+    unsigned long long *counts;
+    unsigned long long *fstats;    // PairParams::fstats; [9] frames filtered, [10] pairs
+                                   // re-evaluated with the 27-image arithmetic
+    unsigned long long *evals;
+};
+
+__host__ __device__ inline size_t tri_filter_smem_bytes(int n_bins, int hslots, int cb)
+{
+    return align16(sizeof(unsigned) * ((size_t)hslots << cb)) +
+           align16(sizeof(double) * (n_bins + 1)) + 2 * kTriTile * sizeof(float4) +
+           sizeof(unsigned) * (kTriListCap + 4);
+}
+
+// Exact re-evaluation of the kTriIpt pairs of one deferred row (thread te, tile row jj):
+// every in-window pair of the row was added to the slot its fp32 coordinate gave; move it
+// where tri_d2 puts it.  Pairs that are not one of the reference's images (|n_k| >= 2) went
+// to the above-range slot, which is where the reference puts them too.  *n_exact (shared)
+// counts the pairs evaluated with tri_d2.
+template <bool EXCL, bool LOWER>
+__device__ __noinline__ void tri_filter_fix(const TriFilterParams &P, int frame, int it,
+                                                unsigned entry, const float4 *tile,
+                                            const double *sT, unsigned hist32, unsigned weight,
+                                            unsigned *n_exact)
+{
+    const TriFilter tf = P.filt[frame];
+    const TriBox h = P.boxes[frame];
+    const FilterConst fc = P.fc;
+    const int te = (int)(entry >> 16), jj = (int)(entry & 0xffffu);
+    const float4 pj = tile[jj];
+    const float4 *f1 = P.p1 + (int64_t)frame * P.pad1;
+    const unsigned span_l = LOWER ? fc.span : fc.cbits + fc.span;
+    for (int ip = 0; ip < kTriIpt; ip += 2) {
+        const int i0 = it * kTriTile + ip * kThreads + te, i1 = i0 + kThreads;
+        const float4 a0 = f1[min(i0, P.n1 - 1)], a1 = f1[min(i1, P.n1 - 1)];
+        unsigned w[2], uu[2];
+        const f32x2 d2 = tri_fold2(pk2(-a0.x, -a1.x), pk2(-a0.y, -a1.y), pk2(-a0.z, -a1.z),
+                                   pk2(pj.x, pj.x), pk2(pj.y, pj.y), pk2(pj.z, pj.z), tf, w[0],
+                                   w[1]);
+        filter_bin2<LOWER>(d2, fc.scale, tf.offm, fc.cbits, uu[0], uu[1]);
+        for (int q = 0; q < 2; ++q) {
+            const int i = q ? i1 : i0;
+            const float4 a = q ? a1 : a0;
+            const unsigned u = uu[q];
+            if (i >= P.n1 || (w[q] & 0x40000000u)) continue;
+            if (!(u < span_l) || !((u & ((1u << fc.k) - 1u)) < tf.wlim)) continue;
+            if (EXCL && __float_as_int(a.w) == __float_as_int(pj.w)) continue;
+            const unsigned seen = (LOWER ? u : u - fc.cbits) >> fc.k;
+            const unsigned col = (unsigned)te & ((1u << fc.cb) - 1u);
+            const double d2r = tri_d2(a.x, a.y, a.z, pj, h);
+            const int slot = P.fast_bins ? slot_fast(d2r, sT, P.n_bins, P.guess)
+                                         : slot_search(d2r, sT, P.n_bins);
+            atomicAdd(n_exact, 1u);
+            if (seen == (unsigned)slot) continue;
+            red_shared(hist32 + 4u * ((seen << fc.cb) + col), 0u - weight);
+            red_shared(hist32 + 4u * (((unsigned)slot << fc.cb) + col), weight);
+        }
+    }
+}
+
+// All pairs of tile pairs (i-tile, j-tile) in the fp32 fold; same group: the upper triangle
+// of tile pairs, weight 2 off the diagonal (fold and reference are odd-symmetric), the
+// diagonal tiles with every ordered pair, the self pairs included.  Tiles are staged with
+// cp.async into two buffers; one block histogram of hslots x 2^cb columns (as
+// rdf_filter_kernel); rows with an in-window pair go on the block's list, drained after each
+// tile by tri_filter_fix (all rows of the tile if the list overflowed).  AUDIT: every pair also through tri_d2, disagreements among the
+// certified pairs counted in fstats[2].
+// (exclusion tags and the audit do not fit 128 registers: those instances take one block
+// per SM's register file share, 255 registers)
+template <bool EXCL, bool LOWER, bool AUDIT>
+__global__ void __launch_bounds__(kThreads, EXCL || AUDIT ? 1 : 2)
+    rdf_tri_filter_kernel(const __grid_constant__ TriFilterParams P)
+{
+    const int frame = blockIdx.y, tid = threadIdx.x, lane = tid & 31;
+    const TriFilter tf = P.filt[frame];
+    if (tf.wlim == 0u) {                  // declined: rdf_triclinic_kernel takes the frame
+        if (blockIdx.x == 0 && tid == 0) atomicAdd(&P.fstats[4], 1ull);
+        return;
+    }
+    if (blockIdx.x == 0 && tid == 0) atomicAdd(&P.fstats[9], 1ull);
+    const int it = blockIdx.x / P.n_jchunks;
+    const int jc = blockIdx.x - it * P.n_jchunks;
+    int jt0 = jc * P.jtiles_per_chunk;
+    const int jt1 = min(P.n_jtiles, jt0 + P.jtiles_per_chunk);
+    if (P.same) jt0 = max(jt0, it);
+    if (jt0 >= jt1) return;
+
+    extern __shared__ __align__(16) unsigned char smem[];
+    const int n_bins = P.n_bins;
+    const FilterConst fc = P.fc;
+    const int hwords = fc.hslots << fc.cb;
+    unsigned *sH = reinterpret_cast<unsigned *>(smem);
+    double *sT = reinterpret_cast<double *>(smem + align16(sizeof(unsigned) * hwords));
+    float4 *sJ = reinterpret_cast<float4 *>(reinterpret_cast<unsigned char *>(sT) +
+                                            align16(sizeof(double) * (n_bins + 1)));
+    unsigned *sList = reinterpret_cast<unsigned *>(sJ + 2 * kTriTile);
+    unsigned *sCount = sList + kTriListCap;
+    for (int k = tid; k <= n_bins; k += kThreads) sT[k] = P.thr[k];
+    for (int k = tid; k < hwords; k += kThreads) sH[k] = 0;
+    if (tid == 0) { sCount[0] = 0; sCount[1] = 0; }
+
+    const float4 *f1 = P.p1 + (int64_t)frame * P.pad1;
+    const float4 *f2 = P.same ? f1 : P.p2 + (int64_t)frame * P.pad2;
+    float xi[kTriIpt], yi[kTriIpt], zi[kTriIpt];
+    int gi[kTriIpt];
+    const int nv = P.n1 - it * kTriTile - tid;
+#pragma unroll
+    for (int ii = 0; ii < kTriIpt; ++ii) {
+        // rows past the end of the group repeat the last particle with weight 0
+        const float4 a = f1[min(it * kTriTile + ii * kThreads + tid, P.n1 - 1)];
+        xi[ii] = a.x; yi[ii] = a.y; zi[ii] = a.z; gi[ii] = __float_as_int(a.w);
+    }
+    f32x2 nx[kTriIpt / 2], ny[kTriIpt / 2], nz[kTriIpt / 2];
+#pragma unroll
+    for (int ip = 0; ip < kTriIpt / 2; ++ip) {
+        nx[ip] = pk2(-xi[2 * ip], -xi[2 * ip + 1]);
+        ny[ip] = pk2(-yi[2 * ip], -yi[2 * ip + 1]);
+        nz[ip] = pk2(-zi[2 * ip], -zi[2 * ip + 1]);
+    }
+
+    // word address of a slot as in rdf_filter_kernel (clamped body); a pair that is not one
+    // of the reference's images gets bit 30 in t, which the clamp sends to the last slot
+    const unsigned hist32 = (unsigned)__cvta_generic_to_shared(sH);
+    const int tshift = fc.k - fc.cb - 2;
+    const unsigned low = (4u << fc.cb) - 1u;
+    const unsigned tmask = ((4u << (fc.cb + fc.lg)) - 1u) & ~low;
+    const unsigned tmax = ((((LOWER ? 0u : fc.cbits) >> fc.k) + (unsigned)(fc.hslots - 1))
+                           << (fc.cb + 2)) | low;
+    const unsigned colbits = ((unsigned)lane & ((1u << fc.cb) - 1u)) << 2;
+    const unsigned span_l = LOWER ? fc.span : fc.cbits + fc.span;
+    const unsigned fmask = (1u << fc.k) - 1u;
+    const float scale = fc.scale, offm = tf.offm;
+    const unsigned wlim = tf.wlim;
+
+    auto stage_tile = [&](int jt, int buf) {
+        const float4 *src = f2 + (int64_t)jt * kTriTile;
+        float4 *dst = sJ + buf * kTriTile;
+#pragma unroll
+        for (int q = 0; q < kTriIpt; ++q)
+            __pipeline_memcpy_async(dst + q * kThreads + tid, src + q * kThreads + tid,
+                                    sizeof(float4));
+        __pipeline_commit();
+    };
+    stage_tile(jt0, 0);
+
+    unsigned long long audit_bad = 0, audit_unc = 0;
+    int buf = 0;
+    for (int jt = jt0; jt < jt1; ++jt) {
+        if (jt + 1 < jt1) {
+            stage_tile(jt + 1, buf ^ 1);
+            __pipeline_wait_prior(1);
+        } else {
+            __pipeline_wait_prior(0);
+        }
+        __syncthreads();
+        const unsigned weight = (P.same && jt > it) ? 2u : 1u;
+        unsigned wi[kTriIpt];
+#pragma unroll
+        for (int ii = 0; ii < kTriIpt; ++ii) wi[ii] = ii * kThreads < nv ? weight : 0u;
+        const int jn = min(kTriTile, P.n2 - jt * kTriTile);
+        const float4 *tile = sJ + buf * kTriTile;
+
+        // two rows per trip where the registers allow it (ptxas -v: no spills)
+        constexpr int kRows = 2;
+#pragma unroll kRows
+        for (int jj = 0; jj < jn; ++jj) {
+            const float4 pj = tile[jj];
+            unsigned vmin = 0xffffffffu;
+#pragma unroll
+            for (int ip = 0; ip < kTriIpt / 2; ++ip) {
+                unsigned w[2], uu[2];
+                const f32x2 d2 = tri_fold2(nx[ip], ny[ip], nz[ip], pk2(pj.x, pj.x),
+                                           pk2(pj.y, pj.y), pk2(pj.z, pj.z), tf, w[0], w[1]);
+                filter_bin2<LOWER>(d2, scale, offm, fc.cbits, uu[0], uu[1]);
+#pragma unroll
+                for (int q = 0; q < 2; ++q) {
+                    const int ii = 2 * ip + q;
+                    const unsigned u = uu[q];
+                    vmin = min(vmin, u & fmask);
+                    unsigned t = min(lop3_and_or(w[q], 0x40000000u, u >> tshift), tmax);
+                    if (EXCL && gi[ii] == __float_as_int(pj.w)) t = tmax;
+                    red_shared_hot(hist32 + lop3_and_or(t, tmask, colbits), wi[ii]);
+                    if (AUDIT && wi[ii] && !(EXCL && gi[ii] == __float_as_int(pj.w))) {
+                        const bool bad = (w[q] & 0x40000000u) != 0u;
+                        const bool in = u < span_l && !bad;
+                        const bool unc = in && (u & fmask) < wlim;
+                        const double d2r = tri_d2(xi[ii], yi[ii], zi[ii], pj, P.boxes[frame]);
+                        const int slot = slot_search(d2r, sT, n_bins);
+                        // the slot the pair was added to, and the exact one
+                        const unsigned fs = in ? ((LOWER ? u : u - fc.cbits) >> fc.k)
+                                               : (unsigned)(fc.hslots - 1);
+                        const bool counted = slot >= 1 && slot <= n_bins;
+                        const bool fcounted = fs >= 1u && fs <= (unsigned)n_bins;
+                        if (unc) ++audit_unc;
+                        else if (fs != (unsigned)slot && (counted || fcounted)) ++audit_bad;
+                    }
+                }
+            }
+            if (vmin < wlim) {
+                const unsigned entry = ((unsigned)tid << 16) | (unsigned)jj;
+                const unsigned idx = atomicAdd(sCount, 1u);
+                if (idx < (unsigned)kTriListCap) sList[idx] = entry;
+            }
+        }
+        __syncthreads();
+        const unsigned n_push = *sCount;
+        const unsigned n_list = min(n_push, (unsigned)kTriListCap);
+        if (n_push <= (unsigned)kTriListCap) {
+            for (unsigned e = tid; e < n_list; e += kThreads)
+                tri_filter_fix<EXCL, LOWER>(P, frame, it, sList[e], tile, sT, hist32, weight,
+                                            sCount + 1);
+        } else {
+            // the list overflowed (rare): every thread re-evaluates all its rows of the tile,
+            // tri_filter_fix acts on the in-window pairs only
+            for (int jj = 0; jj < jn; ++jj)
+                tri_filter_fix<EXCL, LOWER>(P, frame, it, ((unsigned)tid << 16) | (unsigned)jj,
+                                            tile, sT, hist32, weight, sCount + 1);
+        }
+        if (tid == 0) {
+            if (n_push) {
+                atomicAdd(&P.fstats[0], (unsigned long long)n_list);
+                if (n_push > n_list)
+                    atomicAdd(&P.fstats[1], (unsigned long long)(n_push - n_list));
+            }
+            // pairs evaluated: the rows of the i-tile below n1 (nv of thread 0) x jn
+            atomicAdd(P.evals, (unsigned long long)min(kTriTile, nv) * (unsigned long long)jn);
+        }
+        __syncthreads();
+        if (tid == 0) *sCount = 0;
+        buf ^= 1;
+    }
+
+    for (int k = tid; k < n_bins; k += kThreads) {
+        unsigned s = 0;
+        for (int q = 0; q < (1 << fc.cb); ++q)
+            s += sH[((k + 1) << fc.cb) + ((q + tid) & ((1 << fc.cb) - 1))];
+        if (s) atomicAdd(&P.counts[k], (unsigned long long)s);
+    }
+    if (tid == 0 && sCount[1]) atomicAdd(&P.fstats[10], (unsigned long long)sCount[1]);
+    if (AUDIT) {
+        if (audit_bad) atomicAdd(&P.fstats[2], audit_bad);
+        if (audit_unc) atomicAdd(&P.fstats[3], audit_unc);
+    }
+}
+
+template <bool EXCL, bool LOWER, bool AUDIT>
+int launch_tri_filter(mdh_ctx *c, const TriFilterParams &P, dim3 grid)
+{
+    const size_t smem = tri_filter_smem_bytes(P.n_bins, P.fc.hslots, P.fc.cb);
+    auto kern = rdf_tri_filter_kernel<EXCL, LOWER, AUDIT>;
+    MDH_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<grid, kThreads, smem, c->stream>>>(P);
+    MDH_CUDA(cudaGetLastError());
+    c->launches++;
+    return MDH_OK;
+}
+
+template <bool EXCL>
+int launch_tri_filter_e(mdh_ctx *c, const TriFilterParams &P, dim3 grid, bool audit)
+{
+    if (P.fc.lower)
+        return audit ? launch_tri_filter<EXCL, true, true>(c, P, grid)
+                     : launch_tri_filter<EXCL, true, false>(c, P, grid);
+    return audit ? launch_tri_filter<EXCL, false, true>(c, P, grid)
+                 : launch_tri_filter<EXCL, false, false>(c, P, grid);
 }
 
 // ---- cell list in fractional coordinates ---------------------------------------------
@@ -753,6 +1185,55 @@ int tri_cells_accumulate(mdh_ctx *c, const std::vector<TriGrid> &grids, int64_t 
 
 }  // namespace
 
+int rdf_filter_sqrt_error(mdh_ctx *c, double *err);        // rdf_filter.cu
+
+// Device-free: the per-frame parameters of the triclinic filter (mdh_rdf_triclinic_filter_window)
+int rdf_triclinic_filter_window_impl(int n_bins, double r_lo, double r_hi, double sqrt_err,
+                                     int n_frames, const float *cell, const float *ext1,
+                                     const float *ext2, double *frames)
+{
+    MDH_REQUIRE(n_bins >= 1 && n_bins <= 65536, MDH_EINVAL,
+                "triclinic_filter_window: n_bins must be in [1, 65536]");
+    MDH_REQUIRE(r_hi > r_lo && r_lo >= 0, MDH_EINVAL, "triclinic_filter_window: invalid range");
+    MDH_REQUIRE(n_frames >= 1 && cell != nullptr && ext1 != nullptr && frames != nullptr,
+                MDH_EINVAL, "triclinic_filter_window: NULL argument");
+    if (ext2 == nullptr) ext2 = ext1;
+    RdfState R;                    // host fields only: no device buffer is touched
+    R.n_bins = n_bins;
+    R.r_lo = r_lo;
+    R.r_hi = r_hi;
+    R.ipt = 4;
+    std::vector<double> thr(n_bins + 1);
+    for (int i = 0; i <= n_bins; ++i) {
+        const double e = r_lo + i * ((r_hi - r_lo) / n_bins);
+        thr[i] = e * e;
+    }
+    MDH_REQUIRE(rdf_filter_configure(R, thr.data(), sqrt_err), MDH_EINVAL,
+                "triclinic_filter_window: the configuration is not eligible for the fp32 filter");
+    const FilterPrep Q = rdf_filter_prep(R, sqrt_err);
+    for (int f = 0; f < n_frames; ++f) {
+        if (int rc = tri_check_matrix(cell + 9 * f, r_hi)) return rc;
+        const float *m = cell + 9 * f;
+        const TriBox h{(double)m[0], (double)m[3], (double)m[4], (double)m[6], (double)m[7],
+                       (double)m[8]};
+        unsigned k1[6], k2[6];
+        for (int i = 0; i < 6; ++i) {
+            const unsigned b1 = f32_bits(ext1[6 * f + i]), b2 = f32_bits(ext2[6 * f + i]);
+            k1[i] = (b1 & 0x80000000u) ? ~b1 : (b1 | 0x80000000u);   // ext_key
+            k2[i] = (b2 & 0x80000000u) ? ~b2 : (b2 | 0x80000000u);
+        }
+        double info[4];
+        const TriFilter tf = tri_filter_prepare_frame(h, k1, k2, Q, info);
+        double *o = frames + 8 * f;
+        o[0] = tf.wlim != 0u ? 1.0 : 0.0;
+        for (int i = 0; i < 4; ++i) o[1 + i] = info[i];
+        o[5] = (double)tf.offm;
+        o[6] = (double)tf.wlim;
+        o[7] = (double)Q.k;
+    }
+    return MDH_OK;
+}
+
 // pack kernel of rdf_device.cuh is instantiated in this translation unit as well
 int rdf_accumulate_triclinic_impl(mdh_ctx *c, const float *pos1, int64_t s1, const float *pos2,
                                   int64_t s2, int location, const float *box9, int n_frames)
@@ -842,7 +1323,15 @@ int rdf_accumulate_triclinic_impl(mdh_ctx *c, const float *pos1, int64_t s1, con
                              cudaMemcpyHostToDevice, c->stream));
     MDH_CUDA(cudaStreamSynchronize(c->stream));        // hb is a local
 
-    const int64_t pad1 = (R.n1 + 255) / 256 * 256, pad2 = (R.n2 + 255) / 256 * 256;
+    // fp32 filter of the all-pairs path (arith auto / on / audit); the cell list stays fp64
+    const bool use_filter = mode == MDH_RDF_ALLPAIRS && R.filter_ok &&
+                            R.filter_mode != MDH_FILTER_OFF &&
+                            tri_filter_smem_bytes(R.n_bins, R.fc.hslots, R.fc.cb) <= kMaxSmem;
+    double sqrt_err = 0.0;         // measured once per process (rdf_filter.cu)
+    if (use_filter)
+        if (int rc = rdf_filter_sqrt_error(c, &sqrt_err)) return rc;
+    const int64_t pq = use_filter ? kTriTile : 256;
+    const int64_t pad1 = (R.n1 + pq - 1) / pq * pq, pad2 = (R.n2 + pq - 1) / pq * pq;
     const int n_groups = R.same ? 1 : 2;
     // the cell-list path times its whole pipeline (pack and wrap included)
     if (mode == MDH_RDF_CELLS)
@@ -874,6 +1363,17 @@ int rdf_accumulate_triclinic_impl(mdh_ctx *c, const float *pos1, int64_t s1, con
                                                      d_box.as<TriBox>());
         MDH_CUDA(cudaGetLastError());
         c->launches += 2;
+        if (use_filter) {
+            // the filter's bound takes the extents of the wrapped coordinates
+            DevBuf &ext = g ? R.ext2 : R.ext1;
+            if (int rc = ext.reserve(sizeof(unsigned) * 6 * n_frames)) return rc;
+            rdf_ext_init_kernel<<<(6 * n_frames + 255) / 256, 256, 0, c->stream>>>(
+                ext.as<unsigned>(), 6 * n_frames);
+            tri_extent_kernel<<<grid, 256, 0, c->stream>>>(pk.as<float4>(), npad, (int)n,
+                                                           ext.as<unsigned>());
+            MDH_CUDA(cudaGetLastError());
+            c->launches += 2;
+        }
     }
     if (mode == MDH_RDF_CELLS) {
         if (int rc = tri_cells_accumulate(c, grids, pad1, pad2)) return rc;
@@ -899,6 +1399,79 @@ int rdf_accumulate_triclinic_impl(mdh_ctx *c, const float *pos1, int64_t s1, con
     dim3 grid((unsigned)iblocks, (unsigned)((R.n2 + jchunk - 1) / jchunk), (unsigned)n_frames);
     MDH_REQUIRE(grid.y <= 65535, MDH_EINVAL, "rdf: group 2 is too large for the triclinic kernel");
     if (int rc = c->t_rdf.begin(c->stream)) return rc;
+    if (use_filter) {
+        // per-frame parameters on the host from the extents of the wrapped coordinates;
+        // the declined frames then go to rdf_triclinic_kernel, run by run
+        std::vector<unsigned> he(6 * (size_t)n_frames * n_groups);
+        for (int g = 0; g < n_groups; ++g)
+            MDH_CUDA(cudaMemcpyAsync(he.data() + 6 * (size_t)n_frames * g,
+                                     (g ? R.ext2 : R.ext1).p, sizeof(unsigned) * 6 * n_frames,
+                                     cudaMemcpyDeviceToHost, c->stream));
+        MDH_CUDA(cudaStreamSynchronize(c->stream));
+        const unsigned *he2 = he.data() + (R.same ? 0 : 6 * (size_t)n_frames);
+        const FilterPrep fq = rdf_filter_prep(R, sqrt_err);
+        std::vector<TriFilter> hf(n_frames);
+        for (int f = 0; f < n_frames; ++f)
+            hf[f] = tri_filter_prepare_frame(hb[f], he.data() + 6 * f, he2 + 6 * f, fq);
+        if (int rc = R.filt.reserve(sizeof(TriFilter) * n_frames)) return rc;
+        // pageable source: the runtime stages it before returning
+        MDH_CUDA(cudaMemcpyAsync(R.filt.p, hf.data(), sizeof(TriFilter) * n_frames,
+                                 cudaMemcpyHostToDevice, c->stream));
+        TriFilterParams Q;
+        Q.p1 = P.p1; Q.p2 = P.p2;
+        Q.pad1 = P.pad1; Q.pad2 = P.pad2;
+        Q.n1 = P.n1; Q.n2 = P.n2;
+        Q.boxes = P.boxes;
+        Q.filt = R.filt.as<TriFilter>();
+        Q.thr = P.thr;
+        Q.n_bins = P.n_bins;
+        Q.guess = rdf_bin_guess(R);
+        Q.fast_bins = R.fast_bins ? 1 : 0;
+        Q.same = R.same;
+        Q.fc = R.fc;
+        Q.counts = P.counts;
+        Q.fstats = R.fstats.as<unsigned long long>();
+        Q.evals = R.cell[9].as<unsigned long long>();
+        // tile pairs as the orthorhombic all-pairs launch (rdf.cu): about 12 blocks per SM,
+        // and a block's u32 histogram below 2^31 weighted pairs
+        const int n_itiles = (int)(pad1 / kTriTile);
+        Q.n_jtiles = (int)(Q.pad2 / kTriTile);
+        const int64_t target = (int64_t)c->sm_count * 2 * 6;
+        int64_t n_jchunks = (target + (int64_t)n_itiles * n_frames - 1) /
+                            ((int64_t)n_itiles * n_frames);
+        n_jchunks = std::max<int64_t>(1, std::min<int64_t>(n_jchunks, Q.n_jtiles));
+        n_jchunks = std::max<int64_t>(n_jchunks, (Q.n_jtiles + 1023) / 1024);
+        Q.jtiles_per_chunk = (int)((Q.n_jtiles + n_jchunks - 1) / n_jchunks);
+        Q.n_jchunks = (int)((Q.n_jtiles + Q.jtiles_per_chunk - 1) / Q.jtiles_per_chunk);
+        const dim3 fgrid((unsigned)(n_itiles * Q.n_jchunks), (unsigned)n_frames);
+        const bool audit = R.filter_mode == MDH_FILTER_AUDIT;
+        if (int rc = R.excl1 > 0 ? launch_tri_filter_e<true>(c, Q, fgrid, audit)
+                                 : launch_tri_filter_e<false>(c, Q, fgrid, audit))
+            return rc;
+        if (R.excl1 > 0)
+            MDH_CUDA(cudaFuncSetAttribute(rdf_triclinic_kernel<true>,
+                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        else
+            MDH_CUDA(cudaFuncSetAttribute(rdf_triclinic_kernel<false>,
+                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        for (int f0 = 0; f0 < n_frames;) {
+            if (hf[f0].wlim != 0u) { ++f0; continue; }
+            int f1 = f0 + 1;
+            while (f1 < n_frames && hf[f1].wlim == 0u) ++f1;
+            TriParams Pd = P;
+            Pd.p1 = P.p1 + f0 * P.pad1;
+            Pd.p2 = P.p2 + f0 * P.pad2;
+            Pd.boxes = P.boxes + f0;
+            const dim3 dgrid(grid.x, grid.y, (unsigned)(f1 - f0));
+            if (R.excl1 > 0) rdf_triclinic_kernel<true><<<dgrid, 256, smem, c->stream>>>(Pd);
+            else rdf_triclinic_kernel<false><<<dgrid, 256, smem, c->stream>>>(Pd);
+            MDH_CUDA(cudaGetLastError());
+            c->launches++;
+            R.evals += R.n1 * R.n2 * (int64_t)(f1 - f0);
+            f0 = f1;
+        }
+        return c->t_rdf.end(c->stream);
+    }
     if (R.excl1 > 0) {
         MDH_CUDA(cudaFuncSetAttribute(rdf_triclinic_kernel<true>,
                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
