@@ -257,6 +257,20 @@ int mdh_rdf_triclinic_filter_window(int n_bins, double r_lo, double r_hi, double
                                     const float *ext2 /* [n_frames][6] or NULL */,
                                     double *frames /* [n_frames][8] */);
 
+/*
+ * The per-frame parameters of the triclinic CELL LIST's fp32 filter, computed on the host as
+ * mdh_rdf_accumulate_triclinic would; device-free.  The bound depends on the cell matrix
+ * alone (it holds for every frame whose coordinates are finite and not "far"; the device
+ * declines the others).  Arguments as for mdh_rdf_triclinic_filter_window.
+ * frames[n_frames][7]: {eligible (1: filtered, 0: declined), A (absolute error of the fp32
+ * image), a (A plus the reference's float32-dx and fp64 image-sum errors), mu (error bound
+ * in bins, before the window's 1.25 margin), offm, wlim, k}.  MDH_EINVAL when the
+ * configuration is not eligible for the filter or a cell is invalid.
+ */
+int mdh_rdf_triclinic_cells_filter_window(int n_bins, double r_lo, double r_hi, double sqrt_err,
+                                          int n_frames, const float *cell /* [n_frames][9] */,
+                                          double *frames /* [n_frames][7] */);
+
 int mdh_rdf_fetch(mdh_ctx *ctx, int64_t *counts /* [n_bins] host */);
 int mdh_rdf_reset(mdh_ctx *ctx);
 /* device address of the int64[n_bins] accumulator (for NCCL reductions) */

@@ -52,6 +52,7 @@ SIGNATURES = {
     "mdh_rdf_filter_window": (_i32, [_i32, _f64, _f64, _i32, _i32, _i32, _f64, _i32, _p, _p,
                                      _p, _p, _p]),
     "mdh_rdf_triclinic_filter_window": (_i32, [_i32, _f64, _f64, _f64, _i32, _p, _p, _p, _p]),
+    "mdh_rdf_triclinic_cells_filter_window": (_i32, [_i32, _f64, _f64, _f64, _i32, _p, _p]),
     "mdh_rdf_fetch": (_i32, [_p, _p]),
     "mdh_rdf_reset": (_i32, [_p]),
     "mdh_rdf_counts_device": (_i32, [_p, ctypes.POINTER(_p)]),
@@ -266,6 +267,27 @@ def triclinic_filter_window(n_bins: int, r_lo: float, r_hi: float, cell, ext1, e
              for n, v in zip(TRI_FILTER_FIELDS, fr[f])} for f in range(nf)]
 
 
+TRI_CELLS_FILTER_FIELDS = ("eligible", "A", "a", "mu", "offm", "wlim", "k")
+
+
+def triclinic_cells_filter_window(n_bins: int, r_lo: float, r_hi: float, cell, *,
+                                  sqrt_err: float = 2.0 ** -22) -> list:
+    """Per-frame parameters of the fp32 filter of the triclinic cell list
+    (``mdh_rdf_triclinic_cells_filter_window``; no device needed).  ``cell``:
+    ``[n_frames, 3, 3]`` lower-triangular cell matrices; the bound depends on the cell alone.
+    Returns one dict per frame with the fields of ``TRI_CELLS_FILTER_FIELDS`` (``eligible``,
+    ``wlim``, ``k`` as ``int``, the others as ``float``).  Raises ``ValueError`` when the
+    configuration is not eligible for the filter or a cell is invalid."""
+    c = np.ascontiguousarray(cell, dtype=np.float32).reshape(-1, 9)
+    nf = len(c)
+    fr = np.zeros((nf, 7), np.float64)
+    check(lib().mdh_rdf_triclinic_cells_filter_window(int(n_bins), float(r_lo), float(r_hi),
+                                                      float(sqrt_err), nf, c.ctypes.data,
+                                                      fr.ctypes.data))
+    return [{n: (int(v) if n in ("eligible", "wlim", "k") else float(v))
+             for n, v in zip(TRI_CELLS_FILTER_FIELDS, fr[f])} for f in range(nf)]
+
+
 class Context:
     """
     One device, one stream (``mdh_ctx``).  ``stream=None`` uses torch's current
@@ -370,8 +392,10 @@ class Context:
         """fp32 filter of the all-pairs kernel: ``auto``, ``off``, ``on``, ``audit``.  It
         covers triclinic cells on the all-pairs path as well; frames whose ``r_max`` plus the
         error bound does not fit inside half the shortest of a_x, b_y, c_z (or with
-        non-finite coordinates) are declined and take the 27-image fp64 arithmetic.  The
-        triclinic cell list is fp64 whatever the mode."""
+        non-finite coordinates) are declined and take the 27-image fp64 arithmetic.  On the
+        triclinic cell list, frames with a "far" coordinate, non-finite coordinates or a bound
+        that is not small against a bin are declined and take the fp64 arithmetic of the
+        cell list."""
         check(self._lib.mdh_rdf_set_filter(self._h, FILTER_MODES[mode]))
 
     def rdf_set_prewrap(self, mode: str = "auto"):

@@ -128,11 +128,14 @@ def radial_histogram(
         (pairs provably inside a bin are binned from fp32, all others are
         re-evaluated exactly); ``"off"``: fp64 for every pair; ``"audit"``:
         filter plus a full exact comparison (test aid).  Counts do not depend
-        on it either.  On triclinic cells it applies to the all-pairs kernel;
-        frames whose ``range[1]`` plus the error bound does not fit inside half
-        the shortest of a_x, b_y, c_z (or with non-finite coordinates) are
-        declined and take the 27-image fp64 arithmetic, and the triclinic cell
-        list is fp64 whatever ``arith`` says.
+        on it either.  On triclinic cells it applies to the all-pairs kernel and
+        to the cell list.  All pairs: frames whose ``range[1]`` plus the error
+        bound does not fit inside half the shortest of a_x, b_y, c_z (or with
+        non-finite coordinates) are declined and take the 27-image fp64
+        arithmetic.  Cell list: frames with a coordinate far outside the cell,
+        with non-finite coordinates, or whose cell gives a bound that is not
+        small against a bin are declined and take the cell list's fp64
+        arithmetic.
     wrap : `str`, keyword-only
         Coordinates outside the cell: ``"auto"`` follows the reference --
         ``capped_distance`` moves both coordinate sets into the cell in float32 before

@@ -361,6 +361,13 @@ int mdh_rdf_triclinic_filter_window(int n_bins, double r_lo, double r_hi, double
                                             ext2, frames);
 }
 
+int mdh_rdf_triclinic_cells_filter_window(int n_bins, double r_lo, double r_hi, double sqrt_err,
+                                          int n_frames, const float *cell, double *frames)
+{
+    return rdf_triclinic_cells_filter_window_impl(n_bins, r_lo, r_hi, sqrt_err, n_frames, cell,
+                                                  frames);
+}
+
 int mdh_rdf_fetch(mdh_ctx *c, int64_t *counts)
 {
     CTX_GUARD(c);

@@ -112,7 +112,7 @@ struct RdfState {
     DevBuf raw1[2], raw2[2];  // float[F][n][3] staging for host input, one per stager slot
     DevBuf pk1, pk2;       // float4[F][npad]
     DevBuf boxes;          // FrameBox[F]
-    DevBuf cell[10];       // cell-list scratch, layout in rdf_cells.cu
+    DevBuf cell[12];       // cell-list scratch, layout in rdf_cells.cu and rdf_tri.cu
     double cells_ws_mb = 192.0;   // working set of one group of frames (sort + pair kernel)
     int cells_chunk = 4;         // cells per work item of the cell-pair kernel
     int cells_ipt = 4;           // particles per lane of the cell-pair kernel (2 or 4)
@@ -308,6 +308,8 @@ int rdf_cells_grid_impl(const float *cell9, double r_hi, int64_t n_max, int drop
 int rdf_triclinic_filter_window_impl(int n_bins, double r_lo, double r_hi, double sqrt_err,
                                      int n_frames, const float *cell, const float *ext1,
                                      const float *ext2, double *frames);
+int rdf_triclinic_cells_filter_window_impl(int n_bins, double r_lo, double r_hi, double sqrt_err,
+                                           int n_frames, const float *cell, double *frames);
 // rdf_filter.cu
 int rdf_filter_sqrt_error(mdh_ctx *c, double *err);
 bool rdf_filter_configure(RdfState &R, const double *thr, double sqrt_err);

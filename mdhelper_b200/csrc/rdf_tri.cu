@@ -859,6 +859,290 @@ int launch_tri_cells(mdh_ctx *c, const TriCellParams &P, dim3 grid)
     return MDH_OK;
 }
 
+// ---- fp32 filter of the cell list (DESIGN.md 4.8c) -------------------------------------
+//
+// The cell list evaluates one image per candidate, m' = k_j - k_i + w (tri_grid_plan).
+// With q = r + k H, the particle's position inside its cell (tri_cellq_kernel stores it
+// rounded to float32), that image is q_j + (w H - q_i) exactly.  Per run the thread holds
+// v = (float)(w H - q_i), so a candidate costs u = q_j + v (3 FADD), the fp32 sum of
+// squares, sqrt.approx and the fixed-point bin coordinate of 4.1b.  A candidate with its
+// coordinate inside the window (tri_cells_filter_prepare bounds its error against the
+// reference's fp64 d^2 of the same image) is re-evaluated on the spot with the bits of
+// rdf_tri_cells_kernel: tri_image_d2 of m' from the wrapped r, and the same slot lookup.
+
+struct TriCellFilter {     // per frame, from the cell matrix alone (tri_cells_filter_prepare)
+    float offm;            // as FrameFilter::offm
+    unsigned wlim;         // as FrameFilter::wlim; 0 = declined
+};
+
+// q = r + k H of every cell-sorted particle, (q_x, q_y, q_z, shift code); bad[frame] = 1 if
+// a q is not finite.  The sums in fp64 (the products k h are exact), one float32 rounding.
+__global__ void __launch_bounds__(256)
+    tri_cellq_kernel(const float4 *__restrict__ sorted, const int *__restrict__ kcode, int n,
+                     const TriGrid *__restrict__ grids, float4 *__restrict__ q,
+                     int *__restrict__ bad)
+{
+    const int frame = blockIdx.y;
+    const TriBox h = grids[frame].h;
+    bool nonfinite = false;
+    for (int64_t i0 = (int64_t)blockIdx.x * 256; i0 < n; i0 += (int64_t)gridDim.x * 256) {
+        const int64_t i = i0 + threadIdx.x;
+        if (i < n) {
+            const int64_t o = (int64_t)frame * n + i;
+            const float4 p = sorted[o];
+            const unsigned kc = (unsigned)kcode[o];
+            const double ka = (signed char)(kc & 0xffu), kb = (signed char)((kc >> 8) & 0xffu),
+                         kk = (signed char)((kc >> 16) & 0xffu);
+            const float qx = (float)__dadd_rn(__dadd_rn(__dadd_rn((double)p.x, ka * h.ax),
+                                                        kb * h.bx), kk * h.cx);
+            const float qy = (float)__dadd_rn(__dadd_rn((double)p.y, kb * h.by), kk * h.cy);
+            const float qz = (float)__dadd_rn((double)p.z, kk * h.cz);
+            nonfinite = nonfinite || !isfinite(qx) || !isfinite(qy) || !isfinite(qz);
+            q[o] = make_float4(qx, qy, qz, __uint_as_float(kc));
+        }
+    }
+    if (__syncthreads_or(nonfinite) && threadIdx.x == 0) bad[frame] = 1;
+}
+
+struct TriCellFilterParams {
+    TriCellParams c;              // the fp64 kernel's parameters (s1, s2: the wrapped r)
+    const float4 *q1, *q2;        // (q, shift code) of the cell-sorted groups
+    const int *bad;               // [G] (tri_cellq_kernel)
+    const TriCellFilter *filt;    // [G]
+    FilterConst fc;
+    int fast_bins;
+    unsigned long long *fstats;   // [4] declined frames, [9] frames filtered, [10] candidates
+                                  // re-evaluated exactly, [2] / [3] audit
+};
+
+// rdf_tri_cells_kernel with the fp32 filter: one thread per particle i of the cell-sorted
+// group 1, the same runs in the same order.  A frame the filter cannot certify (TriCellFilter
+// wlim 0, a "far" coordinate, a non-finite q) is declined: every candidate then takes the
+// exact arithmetic (far: every ordered pair with all 27 images), as in rdf_tri_cells_kernel.
+// AUDIT: every certain candidate of a filtered frame is also evaluated exactly;
+// disagreements in fstats[2], uncertain candidates in fstats[3].
+template <bool EXCL, bool LOWER, bool AUDIT>
+__global__ void __launch_bounds__(kThreads, 2)
+    rdf_tri_cells_filter_kernel(const __grid_constant__ TriCellFilterParams F)
+{
+    const TriCellParams &P = F.c;
+    extern __shared__ __align__(16) unsigned char smem[];
+    double *sT = reinterpret_cast<double *>(smem);
+    unsigned *sH =
+        reinterpret_cast<unsigned *>(smem + align16(sizeof(double) * (P.n_bins + 1)));
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int frame = blockIdx.y;
+    const int n_bins = P.n_bins;
+    for (int k = tid; k <= n_bins; k += kThreads) sT[k] = P.thr[k];
+    for (int k = tid; k < kWarps * warp_hist_words(n_bins); k += kThreads) sH[k] = 0;
+    __syncthreads();
+
+    // word 0 of the warp's histogram: slot 0 (below the range); slot s: word s; words from
+    // n_bins + 1 on: scratch, one per lane
+    unsigned *myhist = sH + warp * warp_hist_words(n_bins) + 1;
+    const unsigned hist32 = (unsigned)__cvta_generic_to_shared(myhist);
+    const unsigned slot32 = hist32 - 4u;
+    const unsigned trash32 = hist32 + 4u * (unsigned)(n_bins + lane);
+    const BinGuess guess = P.guess;
+    const bool fast = F.fast_bins != 0;
+
+    const TriGrid g = P.grids[frame];
+    const TriBox h = g.h;
+    const TriCellFilter tf = F.filt[frame];
+    const bool far = P.far[frame] != 0;
+    const bool filtered = tf.wlim != 0u && !far && !F.bad[frame];
+    if (blockIdx.x == 0 && tid == 0) atomicAdd(&F.fstats[filtered ? 9 : 4], 1ull);
+    const float4 *s1 = P.s1 + (int64_t)frame * P.n1;
+    const float4 *s2 = P.s2 + (int64_t)frame * P.n2;
+    const float4 *q2 = F.q2 + (int64_t)frame * P.n2;
+    const int *start = P.start2 + (int64_t)frame * P.cstride;
+
+    const int i = blockIdx.x * kThreads + tid;
+    const bool valid = i < P.n1;
+    const int ic = min(i, P.n1 - 1);
+    const float4 pi = s1[ic];
+    const float4 qi = F.q1[(int64_t)frame * P.n1 + ic];
+    const int gi = __float_as_int(pi.w);
+    unsigned ki;
+    const int my_cell = tri_cell(pi, g, ki);
+    const int cx = my_cell % g.nc[0], cy = (my_cell / g.nc[0]) % g.nc[1],
+              cz = my_cell / (g.nc[0] * g.nc[1]);
+    const unsigned kneg = __vsub4(0u, ki);          // -k_i per byte
+    unsigned long long my_evals = 0;
+    unsigned n_exact = 0;
+    unsigned long long audit_bad = 0, audit_unc = 0;
+
+    const FilterConst fc = F.fc;
+    const unsigned span_l = LOWER ? fc.span : fc.cbits + fc.span;
+    const unsigned fmask = (1u << fc.k) - 1u;
+    const float scale = fc.scale, offm = tf.offm;
+    const unsigned wlim = tf.wlim;
+
+    // the slot of an exact d^2 and its histogram word, as rdf_tri_cells_kernel bins
+    auto exact_word = [&](double d2, bool keep, int &slot) -> unsigned {
+        if (fast) {
+            bool below;
+            const int j = slot_fast_parts(d2, sT, n_bins, guess, below);
+            slot = below ? j : j + 1;
+            return ((!below && j == n_bins) || !keep) ? trash32 : slot32 + 4u * (unsigned)slot;
+        }
+        slot = slot_search(d2, sT, n_bins);
+        return (keep && (unsigned)(slot - 1) < (unsigned)n_bins) ? slot32 + 4u * (unsigned)slot
+                                                                  : trash32;
+    };
+
+    if (far) {
+        // the margin does not hold for this frame: every ordered pair, all 27 images
+        if (valid) {
+            for (int j = 0; j < P.n2; ++j) {
+                const float4 pj = s2[j];
+                int slot;
+                red_shared(exact_word(tri_d2(pi.x, pi.y, pi.z, pj, h), !(EXCL && gi ==
+                                      __float_as_int(pj.w)), slot), 1u);
+            }
+            my_evals += P.n2;
+        }
+    } else {
+        // candidates [b, b + len) of a run with wrap code wc; base = (w - k_i) per byte
+        auto sweep = [&](int b, int len, unsigned wc, unsigned w_first, unsigned w_rest) {
+            if (!valid) return;
+            my_evals += len;
+            const unsigned base = __vadd4(wc, kneg);
+            const double wa = (signed char)(wc & 0xffu), wb = (signed char)((wc >> 8) & 0xffu),
+                         ww = (signed char)((wc >> 16) & 0xffu);
+            // v = (float)(w H - q_i): the lattice vector w H in fp64, one float32 rounding
+            const float vx = (float)__dsub_rn(
+                __dadd_rn(__dadd_rn(wa * h.ax, wb * h.bx), ww * h.cx), (double)qi.x);
+            const float vy = (float)__dsub_rn(__dadd_rn(wb * h.by, ww * h.cy), (double)qi.y);
+            const float vz = (float)__dsub_rn(ww * h.cz, (double)qi.z);
+            for (int t = 0; t < len; ++t) {
+                const float4 qj = __ldg(q2 + b + t);
+                const unsigned m = __vadd4(__float_as_uint(qj.w), base);
+                // every byte in {-1, 0, 1} (byte 3 is 0)
+                const bool ref_image = __vcmpleu4(__vadd4(m, 0x00010101u), 0x00020202u) ==
+                                       0xffffffffu;
+                const bool keep =
+                    ref_image &&
+                    !(EXCL && gi == __ldg(reinterpret_cast<const int *>(s2 + b + t) + 3));
+                const float ux = __fadd_rn(qj.x, vx), uy = __fadd_rn(qj.y, vy),
+                            uz = __fadd_rn(qj.z, vz);
+                const float d2 = __fmaf_rn(uz, uz, __fmaf_rn(uy, uy, __fmul_rn(ux, ux)));
+                float s;
+                asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(s) : "f"(d2));
+                const unsigned u = __float_as_uint(__fmaf_rn(s, scale, offm)) -
+                                   (LOWER ? fc.cbits : 0u);
+                const bool in = u < span_l && keep;
+                const unsigned fs = (LOWER ? u : u - fc.cbits) >> fc.k;
+                const unsigned wgt = t == 0 ? w_first : w_rest;
+                // declined frame: every candidate exact
+                const bool unc = !filtered || (in && (u & fmask) < wlim);
+                if (unc || (AUDIT && filtered && keep)) {
+                    // exact: the image m' of the reference's dx, rdf_tri_cells_kernel's bits
+                    const float4 pj = __ldg(s2 + b + t);
+                    const int ix = (int)(signed char)(m & 0xffu);
+                    const int iy = (int)(signed char)((m >> 8) & 0xffu);
+                    const int iz = (int)(signed char)((m >> 16) & 0xffu);
+                    auto sh = [](double v, int q) { return q == 0 ? 0.0 : (q > 0 ? v : -v); };
+                    const double d2r = tri_image_d2(
+                        (double)__fsub_rn(pj.x, pi.x), (double)__fsub_rn(pj.y, pi.y),
+                        (double)__fsub_rn(pj.z, pi.z), sh(h.ax, ix), sh(h.bx, iy),
+                        sh(h.by, iy), sh(h.cx, iz), sh(h.cy, iz), sh(h.cz, iz));
+                    int slot;
+                    const unsigned a = exact_word(d2r, keep, slot);
+                    if (unc) {
+                        red_shared(a, wgt);
+                        ++n_exact;
+                        if (AUDIT && filtered) ++audit_unc;
+                        continue;
+                    }
+                    if (AUDIT) {
+                        const bool counted = keep && slot >= 1 && slot <= n_bins;
+                        const bool fcounted = in && fs >= 1u && fs <= (unsigned)n_bins;
+                        if ((counted || fcounted) && (!counted || !fcounted || fs != (unsigned)slot))
+                            ++audit_bad;
+                    }
+                }
+                red_shared(in && fs <= (unsigned)n_bins ? slot32 + 4u * fs : trash32, wgt);
+            }
+        };
+        auto wrap = [](int v, int n, int &w) {
+            w = v < 0 ? -1 : (v >= n ? 1 : 0);
+            return v - w * n;
+        };
+        auto code = [](int wa, int wb, int wc) {
+            return ((unsigned)wa & 0xffu) | (((unsigned)wb & 0xffu) << 8) |
+                   (((unsigned)wc & 0xffu) << 16);
+        };
+        auto sweep_row = [&](int dy, int dz, unsigned w) {
+            int wb, wc;
+            const int y = wrap(cy + dy, g.nc[1], wb), z = wrap(cz + dz, g.nc[2], wc);
+            const int row = (z * g.nc[1] + y) * g.nc[0];
+            const int xa = max(cx - 1, 0), xb = min(cx + 1, g.nc[0] - 1);
+            const int b0 = start[row + xa];
+            sweep(b0, start[row + xb + 1] - b0, code(0, wb, wc), w, w);
+            if (cx == 0 || cx == g.nc[0] - 1) {
+                const int wa = cx == 0 ? -1 : 1, xw = cx == 0 ? g.nc[0] - 1 : 0;
+                const int bw = start[row + xw];
+                sweep(bw, start[row + xw + 1] - bw, code(wa, wb, wc), w, w);
+            }
+        };
+        const int dz_max = g.nc[2] > 1 ? 1 : 0;
+        if (!P.half) {
+            for (int dz = -dz_max; dz <= dz_max; ++dz)
+                for (int dy = -1; dy <= 1; ++dy) sweep_row(dy, dz, 1u);
+        } else {
+            if (dz_max)
+                for (int dy = -1; dy <= 1; ++dy) sweep_row(dy, 1, 2u);
+            sweep_row(1, 0, 2u);
+            const int row = (cz * g.nc[1] + cy) * g.nc[0];
+            int wa;
+            const int xr = wrap(cx + 1, g.nc[0], wa);
+            const int br = start[row + xr];
+            sweep(br, start[row + xr + 1] - br, code(wa, 0, 0), 2u, 2u);
+            sweep(i, start[row + cx + 1] - i, 0u, 1u, 2u);
+        }
+    }
+    __syncthreads();
+    for (int k = tid; k < n_bins; k += kThreads) {
+        unsigned long long s = 0;
+#pragma unroll
+        for (int w = 0; w < kWarps; ++w) s += sH[w * warp_hist_words(n_bins) + 1 + k];
+        if (s) atomicAdd(&P.counts[k], s);
+    }
+    for (int o = 16; o; o >>= 1) my_evals += __shfl_xor_sync(0xffffffffu, my_evals, o);
+    if (lane == 0 && my_evals) atomicAdd(P.evals, my_evals);
+    if (filtered) {
+        n_exact = __reduce_add_sync(0xffffffffu, n_exact);
+        if (lane == 0 && n_exact) atomicAdd(&F.fstats[10], (unsigned long long)n_exact);
+    }
+    if (AUDIT) {
+        if (audit_bad) atomicAdd(&F.fstats[2], audit_bad);
+        if (audit_unc) atomicAdd(&F.fstats[3], audit_unc);
+    }
+}
+
+template <bool EXCL, bool LOWER, bool AUDIT>
+int launch_tri_cells_filter(mdh_ctx *c, const TriCellFilterParams &F, dim3 grid)
+{
+    const size_t smem = tri_cells_smem_bytes(F.c.n_bins);
+    auto kern = rdf_tri_cells_filter_kernel<EXCL, LOWER, AUDIT>;
+    MDH_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<grid, kThreads, smem, c->stream>>>(F);
+    MDH_CUDA(cudaGetLastError());
+    c->launches++;
+    return MDH_OK;
+}
+
+template <bool EXCL>
+int launch_tri_cells_filter_e(mdh_ctx *c, const TriCellFilterParams &F, dim3 grid, bool audit)
+{
+    if (F.fc.lower)
+        return audit ? launch_tri_cells_filter<EXCL, true, true>(c, F, grid)
+                     : launch_tri_cells_filter<EXCL, true, false>(c, F, grid);
+    return audit ? launch_tri_cells_filter<EXCL, false, true>(c, F, grid)
+                 : launch_tri_cells_filter<EXCL, false, false>(c, F, grid);
+}
+
 // ---- grid planner (host, no device) ------------------------------------------------------
 //
 // Why one image per candidate gives the reference's counts.  Cells are cut in fractional
@@ -1036,6 +1320,60 @@ int tri_grid_plan_flat(const float *m9, double r_hi, int64_t n_max, TriPlan &out
     return MDH_OK;
 }
 
+// Per-frame parameters of the cell-list filter (rdf_tri_cells_filter_kernel) from the cell
+// matrix alone: no extent pass, valid for every frame that is not "far" (tri_far; those
+// are declined on the device).  info (optional): {A, a, mu} (A: the fp32 evaluation's
+// absolute error, a: A + e_f + e_d, mu: the bound in bins before the 1.25 margin).
+//
+// Rows of the cell: R_x = a_x + |b_x| + |c_x|, R_y = b_y + |c_y|, R_z = c_z.  The fractional
+// coordinates of q = r + k H are s + k = s - floor(s~) in [-eps, 1 + eps] (s~ the computed
+// s, eps < 1e-12 whenever the plan gives a grid), so |q_k| <= Q_k = R_k (1 + 1e-9).  Per
+// axis, against the exact image dx + m' H = q_j + w H - q_i:
+//   q      tri_cellq_kernel: three fp64 sums of terms below 1.5 E_k + 60 R_k (non-far r,
+//          |k| <= kTriShiftMax), one float32 rounding: e_q = 2^-24 Q_k + 3 u (1.5 E_k + 60 R_k);
+//   v      (float)(w H - q~_i): three fp64 sums below R_k + Q_k, one float32 rounding of a
+//          result below R_k + Q_k (1 + 2^-24): e_v = 2^-24 (R_k + Q_k) (1 + 2^-23) +
+//          3 u (R_k + Q_k);
+//   A_k = 2 e_q + e_v (q_i and q_j are both rounded);
+//   u      the FADD q~_j + v~ rounds once: 2^-24 |u_k|, relative, in the d_max term below.
+// Reference side (as tri_grid_plan): e_f = 2^-23 |E| for its float32 dx, e_d = 4 u |rows|
+// for its fp64 image sums, 4 u relative for its fp64 squares.  Then as
+// tri_filter_prepare_frame: the fp32 sum of squares (1.5 2^-24 relative on d), the final
+// add (2^-24), the measured sqrt.approx error, the scale / offset FMA (2^-24 d_max scale),
+// the fixed-point resolution 2^-k.  u = 2^-53, E = (a_x, b_y, c_z).
+TriCellFilter tri_cells_filter_prepare(const float *m9, const FilterPrep &Q,
+                                       double *info = nullptr)
+{
+    const double e24 = 1.0 / 16777216.0, u = 1.0 / 9007199254740992.0;
+    const double ax = m9[0], bx = m9[3], by = m9[4], cx = m9[6], cy = m9[7], cz = m9[8];
+    const double R[3] = {ax + std::fabs(bx) + std::fabs(cx), by + std::fabs(cy), cz};
+    const double E[3] = {ax, by, cz};
+    double A2 = 0.0;
+    for (int k = 0; k < 3; ++k) {
+        const double Qk = R[k] * (1.0 + 1e-9);
+        const double eq = e24 * Qk + 3.0 * u * (1.5 * E[k] + kTriShiftMax * R[k]);
+        const double ev = e24 * (R[k] + Qk) * (1.0 + 2.0 * e24) + 3.0 * u * (R[k] + Qk);
+        const double A = 2.0 * eq + ev;
+        A2 += A * A;
+    }
+    const double A = std::sqrt(A2) * (1.0 + 1e-9);
+    const double rows[3] = {2 * ax + ax + std::fabs(bx) + std::fabs(cx),
+                            2 * by + by + std::fabs(cy), 2 * cz + cz};
+    const double e_f = 2.0 * std::sqrt(ax * ax + by * by + cz * cz) * e24;
+    const double e_d = 4 * u * std::sqrt(rows[0] * rows[0] + rows[1] * rows[1] + rows[2] * rows[2]);
+    const double a = (A + e_f + e_d) * (1.0 + 1e-9);
+    const double two_k = (double)(1u << Q.k);
+    const double mu = Q.scale * (a + Q.d_max * (2.5 * e24 * 1.001 + Q.sqrt_err + 4.0 * u)) +
+                      e24 * Q.scale * Q.d_max * 1.001 + 1.0 / two_k + 1e-9;
+    const double m = std::ceil(1.25 * mu * two_k) + 1.0;
+    const bool ok = m >= 1.0 && 2.0 * m + 1.0 < two_k / 8.0;
+    if (info) { info[0] = A; info[1] = a; info[2] = mu; }
+    TriCellFilter tf;
+    tf.offm = ok ? (float)(Q.offbase + m / two_k) : 0.f;
+    tf.wlim = ok ? 2u * (unsigned)m + 1u : 0u;
+    return tf;
+}
+
 }  // namespace
 
 int rdf_triclinic_grid_impl(const float *cell9, double r_hi, int64_t n_max, int32_t *nc,
@@ -1088,8 +1426,10 @@ namespace {
 //   cell[0] TriBox[F]   cell[5] TriGrid[F]   cell[1] int cnt[2][G][cstride] | far[G]
 //   cell[2] int start[2][G][cstride]   cell[3] int2 keyrank[G][n1]   cell[4] float4 sorted1
 //   cell[6] int kcode[G][n1] | [G][n2]   cell[7] keyrank2   cell[8] sorted2   cell[9] evals
+//   fp32 filter (filt not empty): cell[1] also bad[G] after far[G], cell[10] float4 q1[G][n1],
+//   cell[11] float4 q2[G][n2], R.filt TriCellFilter[F]
 int tri_cells_accumulate(mdh_ctx *c, const std::vector<TriGrid> &grids, int64_t pad1,
-                         int64_t pad2)
+                         int64_t pad2, const std::vector<TriCellFilter> &filt, bool audit)
 {
     RdfState &R = c->rdf;
     const int n_frames = (int)grids.size();
@@ -1101,14 +1441,22 @@ int tri_cells_accumulate(mdh_ctx *c, const std::vector<TriGrid> &grids, int64_t 
     // pageable source: the runtime stages it before returning
     MDH_CUDA(cudaMemcpyAsync(d_grids.p, grids.data(), sizeof(TriGrid) * n_frames,
                              cudaMemcpyHostToDevice, c->stream));
+    const bool use_filter = !filt.empty();
+    if (use_filter) {
+        if (int rc = R.filt.reserve(sizeof(TriCellFilter) * n_frames)) return rc;
+        MDH_CUDA(cudaMemcpyAsync(R.filt.p, filt.data(), sizeof(TriCellFilter) * n_frames,
+                                 cudaMemcpyHostToDevice, c->stream));
+    }
     // frames per group: what one group reads and writes between the passes should stay
     // in L2 (the rule of rdf_cells_accumulate; 44 bytes per particle here)
     const int n_groups = R.same ? 1 : 2;
     const int64_t n1 = R.n1, n2 = R.n2;
-    const double per_frame = 44.0 * (double)(n1 + (R.same ? 0 : n2)) + 8.0 * cstride * n_groups;
+    const double per_frame = (use_filter ? 60.0 : 44.0) * (double)(n1 + (R.same ? 0 : n2)) +
+                             8.0 * cstride * n_groups;
     int G = (int)std::max(1.0, std::min(64.0, floor(R.cells_ws_mb * 1048576.0 / per_frame)));
     G = std::min(G, n_frames);
-    const size_t cnt_words = (size_t)2 * G * cstride, reset_words = cnt_words + G;
+    const size_t cnt_words = (size_t)2 * G * cstride,
+                 reset_words = cnt_words + (use_filter ? 2 : 1) * (size_t)G;
     if (int rc = R.cell[1].reserve(sizeof(int) * reset_words)) return rc;
     if (int rc = R.cell[2].reserve(sizeof(int) * cnt_words)) return rc;
     if (int rc = R.cell[3].reserve(sizeof(int2) * (size_t)n1 * G)) return rc;
@@ -1119,7 +1467,12 @@ int tri_cells_accumulate(mdh_ctx *c, const std::vector<TriGrid> &grids, int64_t 
         if (int rc = R.cell[7].reserve(sizeof(int2) * (size_t)n2 * G)) return rc;
         if (int rc = R.cell[8].reserve(sizeof(float4) * (size_t)n2 * G)) return rc;
     }
-    int *d_cnt = R.cell[1].as<int>(), *d_far = d_cnt + cnt_words;
+    if (use_filter) {
+        if (int rc = R.cell[10].reserve(sizeof(float4) * (size_t)n1 * G)) return rc;
+        if (!R.same)
+            if (int rc = R.cell[11].reserve(sizeof(float4) * (size_t)n2 * G)) return rc;
+    }
+    int *d_cnt = R.cell[1].as<int>(), *d_far = d_cnt + cnt_words, *d_bad = d_far + G;
     int *d_start = R.cell[2].as<int>();
     int *d_k1 = R.cell[6].as<int>(), *d_k2 = R.same ? d_k1 : d_k1 + (size_t)n1 * G;
     const size_t scan_smem = sizeof(int) * (kScanTile + kScanTile / 32);
@@ -1156,6 +1509,13 @@ int tri_cells_accumulate(mdh_ctx *c, const std::vector<TriGrid> &grids, int64_t 
                 grp ? d_k2 : d_k1);
             MDH_CUDA(cudaGetLastError());
             c->launches++;
+            if (use_filter) {
+                tri_cellq_kernel<<<grid, 256, 0, c->stream>>>(
+                    R.cell[grp ? 8 : 4].as<float4>(), grp ? d_k2 : d_k1, n, gg,
+                    R.cell[grp ? 11 : 10].as<float4>(), d_bad);
+                MDH_CUDA(cudaGetLastError());
+                c->launches++;
+            }
         }
         TriCellParams P;
         P.s1 = R.cell[4].as<float4>();
@@ -1174,10 +1534,25 @@ int tri_cells_accumulate(mdh_ctx *c, const std::vector<TriGrid> &grids, int64_t 
         P.half = R.same;
         dim3 grid((unsigned)((n1 + kThreads - 1) / kThreads), (unsigned)ng);
         int rc;
-        if (excl) rc = fast ? launch_tri_cells<true, true>(c, P, grid)
-                            : launch_tri_cells<true, false>(c, P, grid);
-        else rc = fast ? launch_tri_cells<false, true>(c, P, grid)
-                       : launch_tri_cells<false, false>(c, P, grid);
+        if (use_filter) {
+            TriCellFilterParams F;
+            F.c = P;
+            F.q1 = R.cell[10].as<float4>();
+            F.q2 = R.same ? F.q1 : R.cell[11].as<float4>();
+            F.bad = d_bad;
+            F.filt = R.filt.as<TriCellFilter>() + g0;
+            F.fc = R.fc;
+            F.fast_bins = fast ? 1 : 0;
+            F.fstats = R.fstats.as<unsigned long long>();
+            rc = excl ? launch_tri_cells_filter_e<true>(c, F, grid, audit)
+                      : launch_tri_cells_filter_e<false>(c, F, grid, audit);
+        } else if (excl) {
+            rc = fast ? launch_tri_cells<true, true>(c, P, grid)
+                      : launch_tri_cells<true, false>(c, P, grid);
+        } else {
+            rc = fast ? launch_tri_cells<false, true>(c, P, grid)
+                      : launch_tri_cells<false, false>(c, P, grid);
+        }
         if (rc) return rc;
     }
     return MDH_OK;
@@ -1230,6 +1605,45 @@ int rdf_triclinic_filter_window_impl(int n_bins, double r_lo, double r_hi, doubl
         o[5] = (double)tf.offm;
         o[6] = (double)tf.wlim;
         o[7] = (double)Q.k;
+    }
+    return MDH_OK;
+}
+
+// Device-free: the per-frame parameters of the cell-list filter
+// (mdh_rdf_triclinic_cells_filter_window)
+int rdf_triclinic_cells_filter_window_impl(int n_bins, double r_lo, double r_hi, double sqrt_err,
+                                           int n_frames, const float *cell, double *frames)
+{
+    MDH_REQUIRE(n_bins >= 1 && n_bins <= 65536, MDH_EINVAL,
+                "triclinic_cells_filter_window: n_bins must be in [1, 65536]");
+    MDH_REQUIRE(r_hi > r_lo && r_lo >= 0, MDH_EINVAL,
+                "triclinic_cells_filter_window: invalid range");
+    MDH_REQUIRE(n_frames >= 1 && cell != nullptr && frames != nullptr, MDH_EINVAL,
+                "triclinic_cells_filter_window: NULL argument");
+    RdfState R;                    // host fields only: no device buffer is touched
+    R.n_bins = n_bins;
+    R.r_lo = r_lo;
+    R.r_hi = r_hi;
+    R.ipt = 4;
+    std::vector<double> thr(n_bins + 1);
+    for (int i = 0; i <= n_bins; ++i) {
+        const double e = r_lo + i * ((r_hi - r_lo) / n_bins);
+        thr[i] = e * e;
+    }
+    MDH_REQUIRE(rdf_filter_configure(R, thr.data(), sqrt_err), MDH_EINVAL,
+                "triclinic_cells_filter_window: the configuration is not eligible for the fp32 "
+                "filter");
+    const FilterPrep Q = rdf_filter_prep(R, sqrt_err);
+    for (int f = 0; f < n_frames; ++f) {
+        if (int rc = tri_check_matrix(cell + 9 * f, r_hi)) return rc;
+        double info[3];
+        const TriCellFilter tf = tri_cells_filter_prepare(cell + 9 * f, Q, info);
+        double *o = frames + 7 * f;
+        o[0] = tf.wlim != 0u ? 1.0 : 0.0;
+        for (int i = 0; i < 3; ++i) o[1 + i] = info[i];
+        o[4] = (double)tf.offm;
+        o[5] = (double)tf.wlim;
+        o[6] = (double)Q.k;
     }
     return MDH_OK;
 }
@@ -1323,13 +1737,22 @@ int rdf_accumulate_triclinic_impl(mdh_ctx *c, const float *pos1, int64_t s1, con
                              cudaMemcpyHostToDevice, c->stream));
     MDH_CUDA(cudaStreamSynchronize(c->stream));        // hb is a local
 
-    // fp32 filter of the all-pairs path (arith auto / on / audit); the cell list stays fp64
+    // fp32 filter (arith auto / on / audit) of the all-pairs path and of the cell list
     const bool use_filter = mode == MDH_RDF_ALLPAIRS && R.filter_ok &&
                             R.filter_mode != MDH_FILTER_OFF &&
                             tri_filter_smem_bytes(R.n_bins, R.fc.hslots, R.fc.cb) <= kMaxSmem;
+    const bool cells_filter = mode == MDH_RDF_CELLS && R.filter_ok &&
+                              R.filter_mode != MDH_FILTER_OFF;
     double sqrt_err = 0.0;         // measured once per process (rdf_filter.cu)
-    if (use_filter)
+    if (use_filter || cells_filter)
         if (int rc = rdf_filter_sqrt_error(c, &sqrt_err)) return rc;
+    // the cell list's per-frame window depends on the cell matrix only
+    std::vector<TriCellFilter> cfilt;
+    if (cells_filter) {
+        const FilterPrep fq = rdf_filter_prep(R, sqrt_err);
+        cfilt.resize(n_frames);
+        for (int f = 0; f < n_frames; ++f) cfilt[f] = tri_cells_filter_prepare(box9 + 9 * f, fq);
+    }
     const int64_t pq = use_filter ? kTriTile : 256;
     const int64_t pad1 = (R.n1 + pq - 1) / pq * pq, pad2 = (R.n2 + pq - 1) / pq * pq;
     const int n_groups = R.same ? 1 : 2;
@@ -1376,7 +1799,9 @@ int rdf_accumulate_triclinic_impl(mdh_ctx *c, const float *pos1, int64_t s1, con
         }
     }
     if (mode == MDH_RDF_CELLS) {
-        if (int rc = tri_cells_accumulate(c, grids, pad1, pad2)) return rc;
+        if (int rc = tri_cells_accumulate(c, grids, pad1, pad2, cfilt,
+                                          R.filter_mode == MDH_FILTER_AUDIT))
+            return rc;
         return c->t_rdf.end(c->stream);
     }
 
