@@ -348,6 +348,22 @@ int mdh_sq_configure(mdh_ctx *ctx, int64_t n_total, int n_groups,
                      const int32_t *lattice_n, const double *lattice_b, int n_pairs,
                      const int32_t *pairs, int mode);
 
+/*
+ * Wavevectors on the reciprocal lattice of a triclinic cell.  cell: HOST pointer, [9], the
+ * row-major lower-triangular cell matrix H (a_x 0 0 / b_x b_y 0 / c_x c_y c_z) with float32
+ * values, the layout of mdh_rdf_accumulate_triclinic; NULL clears it.  While a cell is set,
+ * the wavevectors of mdh_sq_configure are taken in fractional space, k = q H^T (2 pi n for
+ * q = n B*, B* = 2 pi H^-T: lattice_n = n, lattice_b = (2 pi, 2 pi, 2 pi)), and every
+ * coordinate r that mdh_sq_accumulate(_f64) and mdh_isf_accumulate(_f64) receive is first
+ * mapped to s = r H^-1 in fp64 (forward substitution, relative error a few 2^-53 of the
+ * magnitudes involved; DESIGN.md 4.3c), so that k . s = q . r.  From there the float64
+ * coordinate path is followed (float32 + float32 remainder; the ISF's float64 window holds
+ * s).  Call after mdh_sq_configure, which clears the cell; resets the accumulator and ends
+ * an ISF run (mdh_isf_configure after this call).  MDH_ESTATE before mdh_sq_configure;
+ * MDH_EINVAL for a non-finite or non-lower-triangular matrix or a diagonal element <= 0.
+ */
+int mdh_sq_set_cell(mdh_ctx *ctx, const double *cell /* [9] or NULL */);
+
 /* Adds sum over frames of the per-frame |rho|^2 terms to the fp64 accumulator. */
 int mdh_sq_accumulate(mdh_ctx *ctx, const float *pos, int64_t frame_stride, int location,
                       int n_frames);

@@ -67,6 +67,7 @@ SIGNATURES = {
     "mdh_rdf_filter_cleanx": (_i32, [_p, _p]),
     "mdh_rdf_filter_triclinic": (_i32, [_p, _p]),
     "mdh_sq_configure": (_i32, [_p, _i64, _i32, _p, _i32, _p, _p, _p, _i32, _p, _i32]),
+    "mdh_sq_set_cell": (_i32, [_p, _p]),
     "mdh_sq_accumulate": (_i32, [_p, _p, _i64, _i32, _i32]),
     "mdh_sq_accumulate_f64": (_i32, [_p, _p, _i64, _i32, _i32]),
     "mdh_sq_fetch": (_i32, [_p, _p]),
@@ -463,6 +464,16 @@ class Context:
         self._sq_key = key
         self._sq_shape = (len(pr), len(wv))
         self._sq_nrho = 1 if (pr < 0).any() else len(goff) - 1
+
+    def sq_set_cell(self, cell):
+        """Coordinates enter the Fourier sums as fractional coordinates of ``cell`` (the
+        ``[3, 3]`` lower-triangular cell matrix, or ``None`` to clear it); the configured
+        wavevectors are then ``k = q H^T`` (``mdh_sq_set_cell``)."""
+        h = None if cell is None else np.ascontiguousarray(cell, dtype=np.float64).reshape(9)
+        check(self._lib.mdh_sq_set_cell(self._h, _ptr(h)))
+        if h is not None and getattr(self, "_sq_key", None) is not None:
+            # the reset shortcut of sq_configure must not reuse a context whose cell differs
+            self._sq_key = (self._sq_key, h.tobytes())
 
     def sq_accumulate(self, pos, stride, n_frames, *, device=False, keepalive=None,
                       f64=False):

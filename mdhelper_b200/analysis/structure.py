@@ -515,6 +515,14 @@ class RadialDistributionFunction(GpuAnalysisBase):
                 n_dims=2 + (self._drop_axis is None), formalism=formalism)
 
 
+def _grid_indices(n_points: int) -> np.ndarray:
+    """``[n_points^3, 3]`` indices of the first-octant grid in the reference's
+    ``np.meshgrid`` 'xy' order: row (i, j, k) holds (j, i, k)."""
+    idx = np.arange(n_points)
+    ii, jj, kk = np.meshgrid(idx, idx, idx, indexing="ij")
+    return np.stack((jj, ii, kk), axis=-1).reshape(-1, 3)
+
+
 def _lattice_indices(wavevectors: np.ndarray, dimensions) -> tuple:
     """
     If every wavevector is a non-negative integer multiple of the reciprocal
@@ -560,6 +568,16 @@ class StructureFactor(GpuAnalysisBase):
     dimensions, n_points, n_surfaces, n_surface_points, q_max, wavevectors,
     sort, unique
         As in the reference (``structure.py:1366-1416``).
+    reciprocal : `str`, keyword-only, default: :code:`"edges"`
+        ``"edges"`` builds the grid as the reference does, ``2 pi n_k / L_k`` along
+        the Cartesian axes from the three edge lengths (cell angles ignored).
+        ``"cell"`` builds it on the reciprocal lattice of the full cell,
+        ``q = n B*`` with ``B* = 2 pi H^-T`` (``H`` the lower-triangular cell matrix),
+        so that a tilted cell gets wavevectors whose phases do not change when a
+        particle moves by a cell vector; ``dimensions`` may then have 6 entries
+        (3 mean right angles), explicit ``wavevectors`` are Cartesian, and the cell
+        is the one at construction time.  An orthorhombic cell gives the
+        ``"edges"`` results.  No reference counterpart.
     parallel : `bool`, keyword-only
         Accepted for compatibility (the reference's numba thread switch).
     precision : `str`, keyword-only, default: :code:`"fp64"`
@@ -589,7 +607,7 @@ class StructureFactor(GpuAnalysisBase):
             wavevectors: np.ndarray = None, sort: bool = True,
             unique: bool = True, parallel: bool = False, verbose: bool = True,
             precision: str = "fp64", kernel: str = None, host_com: bool = False,
-            **kwargs) -> None:
+            reciprocal: str = "edges", **kwargs) -> None:
 
         self._host_com = bool(host_com)
         self._groups = ([groups] if hasattr(groups, "universe")
@@ -635,22 +653,56 @@ class StructureFactor(GpuAnalysisBase):
         if precision not in {"fp64", "fp32"}:
             raise ValueError("Invalid precision. Valid values: 'fp64', 'fp32'.")
 
+        if reciprocal not in {"edges", "cell"}:
+            raise ValueError("Invalid reciprocal. Valid values: 'edges', 'cell'.")
+        cell_mode = reciprocal == "cell"
+
         self._dimensions = None
         if dimensions is not None:
-            if len(dimensions) != 3:
-                raise ValueError("'dimensions' must have length 3.")
+            if len(dimensions) != 3 and not (cell_mode and len(dimensions) == 6):
+                raise ValueError("'dimensions' must have length 3"
+                                 + (" or 6." if cell_mode else "."))
             self._dimensions = np.asarray(dimensions)
         elif self.universe.dimensions is not None:
-            self._dimensions = self.universe.dimensions[:3].copy()
-        elif wavevectors is None:
+            self._dimensions = self.universe.dimensions[
+                :6 if cell_mode else 3].copy()
+        elif wavevectors is None or cell_mode:
             raise ValueError("No system dimensions found or provided.")
+
+        # reciprocal="cell": H of a tilted cell; the Fourier sums then run on
+        # fractional coordinates s = r H^-1 (mdh_sq_set_cell) and take the
+        # wavevectors as k = q H^T.  An orthorhombic cell keeps the "edges" path.
+        self._cell = None
+        if cell_mode:
+            full = self._dimensions
+            if len(full) == 3:
+                full = np.concatenate((full, np.full(3, 90, full.dtype)))
+            cell = _cell_matrices(full)[0]
+            self._dimensions = full[:3]
+            if not is_orthorhombic(full)[0]:
+                self._cell = cell
+                if n_surfaces:
+                    raise ValueError("'n_surfaces' requires a cubic box.")
 
         # Wavevectors (reference: structure.py:1375-1416).  The grid spacing
         # uses the box edge as stored (float32 from the universe) promoted to
         # float64, and the np.meshgrid 'xy' ordering: row (i, j, k) of the
         # reshaped grid holds (g[j], g[i], g[k]).
         self._lattice_n = self._lattice_b = None
-        if wavevectors is not None:
+        if self._cell is not None:
+            h = self._cell.astype(np.float64)
+            if wavevectors is not None:
+                self._wavevectors = np.asarray(wavevectors, dtype=np.float64)
+                self._kvectors = self._wavevectors @ h.T
+                self._lattice_n, self._lattice_b = _lattice_indices(
+                    self._kvectors, np.ones(3))
+            else:
+                n = _grid_indices(n_points)
+                self._wavevectors = n @ (2 * np.pi * np.linalg.inv(h).T)
+                self._kvectors = 2 * np.pi * n
+                self._lattice_n = n.astype(np.int32)
+                self._lattice_b = np.full(3, 2 * np.pi)
+        elif wavevectors is not None:
             self._wavevectors = np.asarray(wavevectors, dtype=np.float64)
             self._lattice_n, self._lattice_b = _lattice_indices(
                 self._wavevectors, self._dimensions)
@@ -661,8 +713,7 @@ class StructureFactor(GpuAnalysisBase):
                 grids = 3 * [2 * np.pi * idx / self._dimensions[0]]
             else:
                 grids = [2 * np.pi * idx / L for L in self._dimensions]
-            ii, jj, kk = np.meshgrid(idx, idx, idx, indexing="ij")
-            n = np.stack((jj, ii, kk), axis=-1).reshape(-1, 3)
+            n = _grid_indices(n_points)
             self._wavevectors = np.stack(
                 (grids[0][n[:, 0]], grids[1][n[:, 1]], grids[2][n[:, 2]]), axis=-1
             )
@@ -678,11 +729,14 @@ class StructureFactor(GpuAnalysisBase):
                                           n_surface_points))
                 )
                 self._lattice_n = self._lattice_b = None
+        if self._cell is None:
+            self._kvectors = self._wavevectors      # what sq_configure receives
         self._wavenumbers = np.linalg.norm(self._wavevectors, axis=1)
 
         if q_max is not None:
             keep = self._wavenumbers <= q_max
             self._wavevectors = self._wavevectors[keep]
+            self._kvectors = self._kvectors[keep]
             self._wavenumbers = self._wavenumbers[keep]
             if self._lattice_n is not None:
                 self._lattice_n = self._lattice_n[keep]
@@ -724,9 +778,11 @@ class StructureFactor(GpuAnalysisBase):
             mode = "general_fp64"
         else:
             mode = "lattice_fp32" if self._precision == "fp32" else "auto"
-        ctx.sq_configure(int(self._N), offsets, self._wavevectors, pairs,
+        ctx.sq_configure(int(self._N), offsets, self._kvectors, pairs,
                          lattice_n=self._lattice_n, lattice_b=self._lattice_b,
                          mode=mode)
+        if self._cell is not None:
+            ctx.sq_set_cell(self._cell)
         atoms_only = all(g == "atoms" for g in self._groupings)
         self._com = None
         if atoms_only:
@@ -919,9 +975,11 @@ class IntermediateScatteringFunction(StructureFactor):
         else:
             mode = "lattice_fp32" if self._precision == "fp32" else "auto"
         ctx.sq_configure(
-            int(self._N), offsets, self._wavevectors[cols], pairs,
+            int(self._N), offsets, self._kvectors[cols], pairs,
             lattice_n=None if self._lattice_n is None else self._lattice_n[cols],
             lattice_b=self._lattice_b, mode=mode)
+        if self._cell is not None:
+            ctx.sq_set_cell(self._cell)
         ctx.isf_configure(self._n_lags, self._incoherent, len(frames))
 
         atoms_only = all(g == "atoms" for g in self._groupings)

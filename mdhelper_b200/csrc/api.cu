@@ -523,6 +523,12 @@ int mdh_sq_configure(mdh_ctx *c, int64_t n_total, int n_groups, const int64_t *g
                              lattice_b, n_pairs, pairs, mode);
 }
 
+int mdh_sq_set_cell(mdh_ctx *c, const double *cell)
+{
+    CTX_GUARD(c);
+    return sq_set_cell_impl(c, cell);
+}
+
 int mdh_sq_accumulate(mdh_ctx *c, const float *pos, int64_t frame_stride, int location,
                       int n_frames)
 {

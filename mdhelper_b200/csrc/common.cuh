@@ -142,6 +142,25 @@ struct RdfState {
     DevBuf xform;          // unsigned char[F][i-tiles][j-tiles]: x form of every tile pair
 };
 
+struct TriBox {            // lower-triangular cell matrix (rows a, b, c), float32 values
+    double ax, bx, by, cx, cy, cz;
+};
+
+// Fractional coordinates s = r H^-1 of the lower-triangular cell H by forward substitution:
+// s_c = z / c_z, s_b = (y - s_c c_y) / b_y, s_a = ((x - s_b b_x) - s_c c_x) / a_x, every
+// operation rounded once in fp64 (no contraction).  The triclinic cell list (rdf_tri.cu
+// tri_cell, error bound in tri_grid_plan) and the S(q) cell mapping (sq.cu sq_frac_kernel)
+// both go through it.  C: float or double coordinates, widened where they are used.
+template <typename C>
+__device__ __forceinline__ void tri_frac(C x, C y, C z, const TriBox &h, double &sa,
+                                         double &sb, double &sc)
+{
+    sc = __ddiv_rn((double)z, h.cz);
+    sb = __ddiv_rn(__dsub_rn((double)y, __dmul_rn(sc, h.cy)), h.by);
+    sa = __ddiv_rn(__dsub_rn(__dsub_rn((double)x, __dmul_rn(sb, h.bx)), __dmul_rn(sc, h.cx)),
+                   h.ax);
+}
+
 struct SqWorkItem {        // one thread's tile of the lattice kernels: two (nx, ny)
     int nx[2], ny[2];      // columns x one segment of kSqTN consecutive nz
     int nz0;
@@ -198,6 +217,10 @@ struct SqState {
     // single-chain mode (mdh_sq_configure_chains): chunks are chains, ssf[0][q]
     // accumulates sum over chains of |rho_chain(q)|^2
     int64_t n_chains = 0, n_monomers = 0;
+    // mdh_sq_set_cell: coordinates enter the kernels as fractional coordinates of this
+    // cell (sq_frac_kernel); cleared by mdh_sq_configure
+    bool cell = false;
+    TriBox h = {0, 0, 0, 0, 0, 0};
 };
 
 constexpr int kComSlots = 8;
@@ -213,10 +236,12 @@ struct IsfState {           // intermediate scattering function on top of SqStat
     bool on = false;
     int n_lags = 0;
     bool incoherent = false;
-    bool f64 = false;      // the window holds doubles (mdh_isf_accumulate_f64)
+    bool f64 = false;      // float64 input (mdh_isf_accumulate_f64)
     int64_t max_frames = 0, n_done = 0;
     DevBuf rho_all;        // double2[max_frames][n_rho][n_q]: rho(q, t) of every frame
-    DevBuf window[2];      // float (or double) [kept + batch][n_total][3], ping-pong
+    DevBuf window[2];      // float (or double: float64 input or a cell set)
+                           // [kept + batch][n_total][3], ping-pong
+    DevBuf stage;          // host frames on their way to sq_frac_kernel (cell set)
     int window_frames = 0, which = 0;
     DevBuf vmap;           // int4 per virtual frame: {frame, reference frame, lag, 0}
     DevBuf cisf;           // double[n_lags][n_pairs][n_q]
@@ -333,6 +358,7 @@ int com_reduce_impl(mdh_ctx *c, int slot, const float *pos, int64_t stride, int 
 int com_reduce_f64_impl(mdh_ctx *c, int slot, const float *pos, int64_t stride, int location,
                         int n_frames, double *out_device, int64_t out_stride);
 int sq_configure_chains_impl(mdh_ctx *c, int64_t n_chains, int64_t n_monomers);
+int sq_set_cell_impl(mdh_ctx *c, const double *cell);
 int sq_plan_impl(int n_q, const int32_t *lat_n, int64_t *stats, int32_t *coverage,
                  int32_t *pair_rule_violations);
 int sq_plan_items_impl(int n_q, const int32_t *lat_n, int32_t *mma, int32_t *lattice_r,

@@ -33,10 +33,6 @@ using namespace rdfdev;
 
 namespace {
 
-struct TriBox {            // per frame: lower-triangular cell matrix, float32 values
-    double ax, bx, by, cx, cy, cz;
-};
-
 // in place on the packed float4 array
 __global__ void tri_wrap_kernel(float4 *__restrict__ p, int64_t npad, int n,
                                 const TriBox *__restrict__ boxes)
@@ -596,11 +592,8 @@ struct TriGrid {           // per frame
 // cell; its pairs are NaN and binned nowhere.
 __device__ __forceinline__ int tri_cell(const float4 &p, const TriGrid &g, unsigned &kcode)
 {
-    const TriBox &h = g.h;
-    const double sc = __ddiv_rn((double)p.z, h.cz);
-    const double sb = __ddiv_rn(__dsub_rn((double)p.y, __dmul_rn(sc, h.cy)), h.by);
-    const double sa = __ddiv_rn(
-        __dsub_rn(__dsub_rn((double)p.x, __dmul_rn(sb, h.bx)), __dmul_rn(sc, h.cx)), h.ax);
+    double sa, sb, sc;
+    tri_frac(p.x, p.y, p.z, g.h, sa, sb, sc);
     const double s[3] = {sa, sb, sc};
     int c[3];
     kcode = 0u;

@@ -1217,6 +1217,7 @@ int sq_configure_impl(mdh_ctx *c, int64_t n_total, int n_groups, const int64_t *
     S.pairs.assign(pairs, pairs + 2 * n_pairs);
     S.rho_frames = 0;
     S.n_chains = S.n_monomers = 0;
+    S.cell = false;
 
     // ---- lattice work items (lattice_build_items) ----
     bool lattice = lat_n && lat_b && mode != MDH_SQ_GENERAL_FP64;
@@ -1435,6 +1436,78 @@ __global__ void sq_split_kernel(const double *__restrict__ src, int64_t src_stri
     if (blockIdx.x == 0 && threadIdx.x == 0) vmap[f] = make_int4(f, n_frames + f, 0, 0);
 }
 
+// A cell is set (mdh_sq_set_cell): every coordinate r enters as its fractional coordinates
+// s = r H^-1, formed in fp64 by tri_frac.  With q = n B*, B* = 2 pi H^-T, q . r = 2 pi n . s,
+// so the lattice kernels evaluate the reciprocal-lattice grid of the cell with
+// lattice_b = (2 pi, 2 pi, 2 pi), and the general kernel any q given as k = q H^T.
+// split != NULL: s is written as sq_split_kernel writes float64 coordinates (frame f of
+// split: float32 hi, frame n_frames + f: negated float32 remainder; vmap[f]).  Else s itself
+// goes to win ([n_frames][n][3] doubles: the ISF's float64 window).
+template <typename T>
+__global__ void sq_frac_kernel(const T *__restrict__ src, int64_t src_stride, int64_t n,
+                               const TriBox h, int n_frames, float *__restrict__ split,
+                               int4 *__restrict__ vmap, double *__restrict__ win)
+{
+    const int f = blockIdx.y;
+    const T *r = src + (int64_t)f * src_stride;
+    const int64_t n3 = 3 * n;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n;
+         i += (int64_t)gridDim.x * blockDim.x) {
+        double s[3];
+        tri_frac(r[3 * i], r[3 * i + 1], r[3 * i + 2], h, s[0], s[1], s[2]);
+        if (split) {
+            float *hi = split + (int64_t)f * n3 + 3 * i;
+            float *nlo = split + (int64_t)(n_frames + f) * n3 + 3 * i;
+#pragma unroll
+            for (int k = 0; k < 3; ++k) {
+                const float v = (float)s[k];
+                hi[k] = v;
+                nlo[k] = (float)((double)v - s[k]);
+            }
+        } else {
+            double *w = win + (int64_t)f * n3 + 3 * i;
+#pragma unroll
+            for (int k = 0; k < 3; ++k) w[k] = s[k];
+        }
+    }
+    if (split && blockIdx.x == 0 && threadIdx.x == 0) vmap[f] = make_int4(f, n_frames + f, 0, 0);
+}
+
+template <typename T>
+static int launch_frac(mdh_ctx *c, const T *src, int64_t src_stride, int n_frames,
+                       float *split, int4 *vmap, double *win)
+{
+    const SqState &S = c->sq;
+    dim3 grid((unsigned)std::min<int64_t>((S.n_total + 255) / 256, 1024), n_frames);
+    sq_frac_kernel<T><<<grid, 256, 0, c->stream>>>(src, src_stride, S.n_total, S.h, n_frames,
+                                                   split, vmap, win);
+    MDH_CUDA(cudaGetLastError());
+    c->launches++;
+    return MDH_OK;
+}
+
+int sq_set_cell_impl(mdh_ctx *c, const double *cell)
+{
+    SqState &S = c->sq;
+    MDH_REQUIRE(S.configured, MDH_ESTATE, "sq: set the cell after mdh_sq_configure");
+    if (cell) {
+        for (int k = 0; k < 9; ++k)
+            MDH_REQUIRE(std::isfinite(cell[k]), MDH_EINVAL, "sq: the cell matrix is not finite");
+        MDH_REQUIRE(cell[1] == 0.0 && cell[2] == 0.0 && cell[5] == 0.0, MDH_EINVAL,
+                    "sq: the cell matrix is not lower triangular");
+        MDH_REQUIRE(cell[0] > 0.0 && cell[4] > 0.0 && cell[8] > 0.0, MDH_EINVAL,
+                    "sq: the cell matrix is not a valid cell");
+        S.h = TriBox{cell[0], cell[3], cell[4], cell[6], cell[7], cell[8]};
+    }
+    S.cell = cell != nullptr;
+    // sums over other coordinates do not carry over; the ISF window's layout follows the
+    // cell, so an ISF run is configured after this call
+    S.rho_frames = 0;
+    c->isf.on = false;
+    MDH_CUDA(cudaMemsetAsync(S.ssf.p, 0, sizeof(double) * (size_t)S.n_pairs * S.n_q, c->stream));
+    return MDH_OK;
+}
+
 template <typename T>
 static int sq_accumulate_piece(mdh_ctx *c, const T *pos, int64_t stride, int location,
                                int n_frames, int nominal_frames, bool probe);
@@ -1466,7 +1539,7 @@ static int sq_accumulate_any(mdh_ctx *c, const T *pos, int64_t stride, int locat
         for (int slot = 0; slot < 2 && pieces.size() > 1; ++slot)
             if (int rc = S.raw[slot].reserve(sizeof(T) * 3 * S.n_total * (size_t)longest))
                 return rc;
-        if (sizeof(T) == 8) {
+        if (sizeof(T) == 8 || S.cell) {
             if (int rc = S.split.reserve(sizeof(float) * 6 * S.n_total * (size_t)longest))
                 return rc;
             if (int rc = S.split_vmap.reserve(sizeof(int4) * (size_t)longest)) return rc;
@@ -1526,21 +1599,25 @@ static int sq_accumulate_piece(mdh_ctx *c, const T *pos, int64_t stride, int loc
     const size_t rho_bytes = sizeof(double) * 2 * (size_t)n_frames * S.n_rho * S.n_q;
     if (S.n_chains == 0)
         if (int rc = S.rho.reserve(rho_bytes)) return rc;
-    const float *fsrc;
+    const float *fsrc = nullptr;
     const int4 *vmap = nullptr;
-    if constexpr (kF64) {
+    if (kF64 || S.cell) {
         const int64_t n3 = 3 * S.n_total;
         if (int rc = S.split.reserve(sizeof(float) * 2 * n3 * n_frames)) return rc;
         if (int rc = S.split_vmap.reserve(sizeof(int4) * (size_t)n_frames)) return rc;
         fsrc = S.split.as<float>();
         vmap = S.split_vmap.as<int4>();
-    } else {
+    } else if constexpr (!kF64) {
         fsrc = dsrc;
     }
 
     if (int rc = c->t_sq.begin(c->stream)) return rc;
     if (probe) MDH_CUDA(cudaEventRecord(S.probe.ev[2], c->stream));
-    if constexpr (kF64) {
+    if (S.cell) {
+        if (int rc = launch_frac(c, dsrc, dstride, n_frames, S.split.as<float>(),
+                                 S.split_vmap.as<int4>(), (double *)nullptr)) return rc;
+        dstride = 3 * S.n_total;
+    } else if constexpr (kF64) {
         const int64_t n3 = 3 * S.n_total;
         dim3 grid((unsigned)std::min<int64_t>((n3 + 255) / 256, 1024), n_frames);
         sq_split_kernel<<<grid, 256, 0, c->stream>>>(dsrc, dstride, S.split.as<float>(), n3,
@@ -1699,12 +1776,13 @@ int isf_configure_impl(mdh_ctx *c, int n_lags, int incoherent, int64_t max_frame
 
 // T = float: the window holds the float32 frames the kernels read directly; T = double
 // (centres of mass: the reference's float64 position buffer, structure.py:1927-1957): the
-// window holds doubles and the kernels get float32 + remainder copies
+// window holds doubles and the kernels get float32 + remainder copies.  A cell set: the
+// window holds the fractional coordinates (sq_frac_kernel) as doubles, whatever T, and the
+// float64 path follows (displacements s(t) - s(t - lag) in fp64).
 template <typename T>
 static int isf_accumulate_any(mdh_ctx *c, const T *pos, int64_t stride, int location,
                               int n_frames)
 {
-    constexpr bool kF64 = sizeof(T) == 8;
     SqState &S = c->sq;
     IsfState &I = c->isf;
     MDH_REQUIRE(S.configured && I.on, MDH_ESTATE, "isf: accumulate before configure");
@@ -1719,33 +1797,48 @@ static int isf_accumulate_any(mdh_ctx *c, const T *pos, int64_t stride, int loca
 
     // coordinate window: [frames kept from earlier calls][the frames of this call]
     const int64_t fsz = 3 * S.n_total;                     // coordinates per frame
+    const bool wide = sizeof(T) == 8 || S.cell;           // the window holds doubles
+    const size_t esz = wide ? sizeof(double) : sizeof(float);
     const int keep = I.window_frames;
     DevBuf &win = I.window[I.which];
-    const size_t need = sizeof(T) * fsz * (size_t)(keep + n_frames);
+    const size_t need = esz * fsz * (size_t)(keep + n_frames);
     if (win.cap < need) {
         // grow WITHOUT losing the frames kept from earlier calls (DevBuf::reserve frees)
         DevBuf bigger;
         if (int rc = bigger.reserve(need)) return rc;
         if (keep > 0)
-            MDH_CUDA(cudaMemcpyAsync(bigger.p, win.p, sizeof(T) * fsz * (size_t)keep,
+            MDH_CUDA(cudaMemcpyAsync(bigger.p, win.p, esz * fsz * (size_t)keep,
                                      cudaMemcpyDeviceToDevice, c->stream));
         MDH_CUDA(cudaStreamSynchronize(c->stream));
         win.adopt(bigger);
     }
-    MDH_CUDA(mdh_copy_frames(win.as<T>() + fsz * keep, sizeof(T) * fsz, pos,
-                               sizeof(T) * stride, sizeof(T) * fsz, n_frames,
-                               location == MDH_HOST ? cudaMemcpyHostToDevice
-                                                    : cudaMemcpyDeviceToDevice, c->stream));
+    const T *src = pos;                 // where sq_frac_kernel reads the frames
+    int64_t src_stride = stride;
+    if (!S.cell) {
+        MDH_CUDA(mdh_copy_frames(win.as<T>() + fsz * keep, sizeof(T) * fsz, pos,
+                                 sizeof(T) * stride, sizeof(T) * fsz, n_frames,
+                                 location == MDH_HOST ? cudaMemcpyHostToDevice
+                                                      : cudaMemcpyDeviceToDevice, c->stream));
+    } else if (location == MDH_HOST) {
+        if (int rc = I.stage.reserve(sizeof(T) * fsz * (size_t)n_frames)) return rc;
+        MDH_CUDA(mdh_copy_frames(I.stage.p, sizeof(T) * fsz, pos, sizeof(T) * stride,
+                                 sizeof(T) * fsz, n_frames, cudaMemcpyHostToDevice, c->stream));
+        src = I.stage.as<T>();
+        src_stride = fsz;
+    }
     if (int rc = c->t_sq.begin(c->stream)) return rc;
+    if (S.cell)
+        if (int rc = launch_frac(c, src, src_stride, n_frames, nullptr, nullptr,
+                                 win.as<double>() + fsz * keep)) return rc;
 
     // rho(q, t) of the new frames, straight into the per-frame store
     const size_t row = (size_t)2 * S.n_rho * S.n_q;        // doubles per frame
     const float *fwin = nullptr;
-    if constexpr (kF64) {
+    if (wide) {
         if (int rc = S.split.reserve(sizeof(float) * 2 * fsz * n_frames)) return rc;
         if (int rc = S.split_vmap.reserve(sizeof(int4) * (size_t)n_frames)) return rc;
         dim3 grid((unsigned)std::min<int64_t>((fsz + 255) / 256, 1024), n_frames);
-        sq_split_kernel<<<grid, 256, 0, c->stream>>>(win.as<T>() + fsz * keep, fsz,
+        sq_split_kernel<<<grid, 256, 0, c->stream>>>(win.as<double>() + fsz * keep, fsz,
                                                      S.split.as<float>(), fsz, n_frames,
                                                      S.split_vmap.as<int4>());
         MDH_CUDA(cudaGetLastError());
@@ -1754,7 +1847,7 @@ static int isf_accumulate_any(mdh_ctx *c, const T *pos, int64_t stride, int loca
                                     n_frames, I.rho_all.as<double>() + row * I.n_done,
                                     n_frames)) return rc;
     } else {
-        fwin = win.as<T>();
+        fwin = win.as<float>();
         if (int rc = sq_compute_rho(c, fwin + fsz * keep, fsz, nullptr, n_frames,
                                     I.rho_all.as<double>() + row * I.n_done, n_frames))
             return rc;
@@ -1776,7 +1869,7 @@ static int isf_accumulate_any(mdh_ctx *c, const T *pos, int64_t stride, int loca
         // batches sized to ~256 MB of temporary rho
         int vmax = (int)std::max<size_t>(1, std::min<size_t>(
             8192, ((size_t)256 << 20) / (sizeof(double) * row)));
-        if constexpr (kF64) {
+        if (wide) {
             // ... and to ~256 MB of materialised displacements
             vmax = (int)std::max<size_t>(1, std::min<size_t>(
                 vmax, ((size_t)256 << 20) / (sizeof(float) * 2 * (size_t)fsz)));
@@ -1791,10 +1884,10 @@ static int isf_accumulate_any(mdh_ctx *c, const T *pos, int64_t stride, int loca
             MDH_CUDA(cudaMemcpyAsync(I.vmap.p, vm.data() + v0, sizeof(int4) * nv,
                                      cudaMemcpyHostToDevice, c->stream));
             const int4 *vdev = I.vmap.as<int4>();
-            if constexpr (kF64) {
+            if (wide) {
                 dim3 sgrid((unsigned)std::min<int64_t>((fsz + 255) / 256, 1024), nv);
                 isf_displacement_split_kernel<<<sgrid, 256, 0, c->stream>>>(
-                    win.as<T>(), fsz, I.vmap.as<int4>(), nv, S.split.as<float>(),
+                    win.as<double>(), fsz, I.vmap.as<int4>(), nv, S.split.as<float>(),
                     S.split_vmap.as<int4>());
                 MDH_CUDA(cudaGetLastError());
                 c->launches++;
@@ -1816,9 +1909,9 @@ static int isf_accumulate_any(mdh_ctx *c, const T *pos, int64_t stride, int loca
         const int next_keep = std::min(total, I.n_lags - 1);
         DevBuf &nxt = I.window[I.which ^ 1];
         if (next_keep > 0) {
-            if (int rc = nxt.reserve(sizeof(T) * fsz * (size_t)next_keep)) return rc;
-            MDH_CUDA(cudaMemcpyAsync(nxt.p, win.as<T>() + fsz * (total - next_keep),
-                                     sizeof(T) * fsz * next_keep,
+            if (int rc = nxt.reserve(esz * fsz * (size_t)next_keep)) return rc;
+            MDH_CUDA(cudaMemcpyAsync(nxt.p, win.as<char>() + esz * fsz * (total - next_keep),
+                                     esz * fsz * next_keep,
                                      cudaMemcpyDeviceToDevice, c->stream));
         }
         I.window_frames = next_keep;
